@@ -1,6 +1,6 @@
 """Host logic of bench.py that runs without a GPU: the choice of the reference arm's grid (a measured, unscaled run of the compiled reference at
 the largest S3 grid that fits the time / memory budget -- 256^3, the metric's own configuration, on the GPU box's host) and the per-machine cache
-that lets the N > 1 lines of a scaling run reuse the N = 1 measurement."""
+that lets the N > 1 lines of a scaling run reuse the N = 1 measurement; the --dump-outputs writer."""
 import importlib.util
 import json
 import os
@@ -42,3 +42,23 @@ def test_reference_run_cache_is_per_boot_and_expires(tmp_path, monkeypatch):
     assert b.ref_cache_load() is None
     json.dump(dict(stale, time=time.time() - 13 * 3600), open(b.REF_CACHES[1], "w"))
     assert b.ref_cache_load() is None
+
+
+def test_dump_outputs_writes_fp32_fields_and_a_fixed_sample_of_large_ones(tmp_path, monkeypatch):
+    import numpy as np
+    b = _bench()
+    monkeypatch.setattr(b, "DUMP_MAX_ENTRIES", 1000)
+    rng = np.random.default_rng(1)
+    small = [rng.standard_normal((4, 5, 6)).astype(np.float32) for _ in range(3)]
+    large = [rng.standard_normal((20, 10, 10)).astype(np.float32) for _ in range(3)]
+    for run in ("a", "b"):
+        b.dump_outputs(str(tmp_path / run), small, large)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == [f"{k}{ax}.npy" for k in ("valid", "vel") for ax in range(3)]
+    for ax in range(3):
+        vel = np.load(tmp_path / "a" / f"vel{ax}.npy")
+        assert vel.dtype == np.float32 and np.array_equal(vel, small[ax])               # small enough: the whole field, shape kept
+        valid = np.load(tmp_path / "a" / f"valid{ax}.npy")
+        assert valid.dtype == np.float32 and valid.shape == (1000,)
+        assert np.isin(valid, large[ax]).all()                                             # a sample of the field's own entries ...
+        assert np.array_equal(valid, np.load(tmp_path / "b" / f"valid{ax}.npy"))          # ... at the same positions on every run
