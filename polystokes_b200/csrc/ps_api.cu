@@ -523,6 +523,10 @@ int64_t ps_get_count(ps_handle h, const char* name) {
     if (n == "directHalo") return S.fusedHalo ? 1 : 0;      // boundary entries stored straight into the neighbours' vectors (ps_peer.hpp, VecLink)
     if (n == "result") return S.result; if (n == "usedBiCGStab") return S.usedBiCGStab;
     if (n == "nRowsExt") return C.nRowsExt; if (n == "fixLoops") return S.fixLoops;
+    // the shape of the reduced regions and the kernels their term of an apply takes (ps_pcg.cu, region_path)
+    if (n == "maxRegionRows") return S.RG.maxRegionRows; if (n == "maxRegionAxisRows") return S.RG.maxRegionAxisRows;
+    if (n == "maxRegionCells") return S.RG.maxRegionCells; if (n == "minRegionCells") return S.RG.minRegionCells;
+    if (n == "regionPath") return region_path(S.make_op_args(), S.RG);
     return INT64_MIN;
 }
 double ps_get_real(ps_handle h, const char* name) {

@@ -1140,8 +1140,13 @@ __global__ void __launch_bounds__(HOT_THREADS, 5) pass1_regions_kernel(const __g
         rowsTurn = !rowsTurn;
     }
 }
-bool pass1_regions_applicable(const OpArgs& A, const RegionData& RG) {
+// regions with more coupled rows than this take the chunked kernels (reduced_moments_kernel + reduced_expand_kernel)
+static int region_fuse_limit() {
     static const int fuseLimit = getenv("PS_REGION_FUSE_MAX") ? atoi(getenv("PS_REGION_FUSE_MAX")) : 16384;
+    return fuseLimit;
+}
+bool pass1_regions_applicable(const OpArgs& A, const RegionData& RG) {
+    const int fuseLimit = region_fuse_limit();
     // measured on S3 256^3 (profiles/r02_probe_s3_256_v8*.log): 0.181 ms against 0.141 ms for sweep + region kernel on one GPU -- a CTA
     // sitting in a region's chain keeps 8 warps from streaming rows, and only ~half of the CTAs are in a chain at any time (5 rounds of
     // regions instead of 2 waves).  Off by default; PS_OVERLAP=1 for A/B runs.
@@ -1165,15 +1170,27 @@ static void launch_region(cudaStream_t st, const Geom& g, const RegionData& RG, 
     const int32_t* order = lpt && RG.regionOrder.n >= (size_t)RG.regHi ? RG.regionOrder.p : nullptr;
     launch_chain(reduced_region_kernel<GROUP, ROWS, MINB>, (unsigned)(RG.regHi - RG.regLo), 3 * GROUP, st, g.dx, RG.rowXYZ.p, RG.rowAxisStart.p, RG.com.p, RG.Binv.p, wRows, scale, S, RG.regLo, order);
 }
+// template instance of reduced_region_kernel for these regions.  A/B knob.  Default: 64 lanes per axis, 6 CTAs per SM for many regions
+// (throughput); few regions per GPU (slab decomposition) are latency bound -- 128 lanes per axis with the rows kept in registers put
+// every load of a region in flight at once
+static int region_variant(const RegionData& RG) {
+    static const int forced = getenv("PS_REGION_VARIANT") ? atoi(getenv("PS_REGION_VARIANT")) : -1;
+    return forced >= 0 ? forced : (RG.regHi - RG.regLo <= 900 ? 1 : 0);
+}
+// which kernels carry the reduced term of a forward apply (pass1Apply), knobs included: -1 no owned region, 0 reduced_region_kernel with
+// 64 lanes per axis, 1 with 128 lanes, 2 the chunked kernels, 3 pass1_regions_kernel, 4 reduced_region_kernel with 32 lanes
+int region_path(const OpArgs& A, const RegionData& RG) {
+    if (RG.regHi <= RG.regLo) return -1;
+    if (pass1_regions_applicable(A, RG)) return 3;
+    if (RG.maxRegionRows > region_fuse_limit()) return 2;
+    const int variant = region_variant(RG);
+    return variant == 1 || variant == 4 ? 1 : (variant == 3 ? 4 : 0);
+}
 // w_f <- scale * c_f . B^-1 J w on the coupled reduced rows (the reduced term of one operator apply)
 void reduced_apply(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
-    static const int fuseLimit = getenv("PS_REGION_FUSE_MAX") ? atoi(getenv("PS_REGION_FUSE_MAX")) : 16384;
     if (RG.regHi <= RG.regLo) return;
-    if (RG.maxRegionRows > fuseLimit) { reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S); return; }
-    // A/B knob.  Default: 64 lanes per axis, 6 CTAs per SM for many regions (throughput); few regions per GPU (slab decomposition) are
-    // latency bound -- 128 lanes per axis with the rows kept in registers put every load of a region in flight at once
-    static const int forced = getenv("PS_REGION_VARIANT") ? atoi(getenv("PS_REGION_VARIANT")) : -1;
-    const int variant = forced >= 0 ? forced : (RG.regHi - RG.regLo <= 900 ? 1 : 0);
+    if (RG.maxRegionRows > region_fuse_limit()) { reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S); return; }
+    const int variant = region_variant(RG);
     if (variant == 1) launch_region<128, 8, 2>(st, g, RG, wRows, scale, S);
     else if (variant == 2) launch_region<64, 8, 4>(st, g, RG, wRows, scale, S);
     else if (variant == 3) launch_region<32, 0, 10>(st, g, RG, wRows, scale, S);
@@ -1235,6 +1252,7 @@ void reduced_finish(cudaStream_t, const Geom&, const RegionData& RG, const doubl
 void reduced_apply(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
     reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S);
 }
+int region_path(const OpArgs&, const RegionData& RG) { return RG.regHi > RG.regLo ? 2 : -1; }      // the twin has the chunked form only
 void reduced_expand(cudaStream_t, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
     if (S && S->done) return;
     for (int ch = RG.rowChunkLo; ch < RG.rowChunkHi; ++ch) {

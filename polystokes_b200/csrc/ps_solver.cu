@@ -633,7 +633,7 @@ static void build_chunks(const std::vector<int>& perRegion, int chunk, std::vect
 void Solver::computeReducedRegionMatrices() {
     const int R = RG.count;
     if (!part.local) part.regionCut.assign((size_t)part.nranks + 1, 0);      // slab-local: known since the regions were numbered
-    RG.regLo = RG.regHi = 0; RG.cellChunkLo = RG.cellChunkHi = 0;
+    RG.regLo = RG.regHi = 0; RG.cellChunkLo = RG.cellChunkHi = 0; RG.maxRegionCells = RG.minRegionCells = 0;
     if (R <= 0) return;
     const int64_t nc = g.n[SL_CENTER];
     DBuf<unsigned long long>& sums = scratch().sums;
@@ -669,6 +669,10 @@ void Solver::computeReducedRegionMatrices() {
         while (owner < part.nranks) part.regionCut[++owner] = R;
     }
     RG.regLo = part.regionCut[part.rank]; RG.regHi = part.regionCut[part.rank + 1];
+    if (RG.regHi > RG.regLo) {
+        const auto mm = std::minmax_element(perRegion.begin() + RG.regLo, perRegion.begin() + RG.regHi);
+        RG.minRegionCells = *mm.first; RG.maxRegionCells = *mm.second;
+    }
     std::vector<int32_t> start, table, chunkStart;
     build_chunks(perRegion, 256, start, table, chunkStart);
     RG.nCellChunks = (int32_t)(table.size() / 3);
@@ -699,7 +703,7 @@ void Solver::constructMatrixBlocks() {
         z_range(g, SL_FACE + a, g.wzLo, g.wzHi, lo, hi);
         k_krow_active(st, lo, hi, F.aidx[SL_FACE + a], (int32_t)C.faceOff[a], F.krow[a]);
     }
-    RG.nRows = 0; RG.nRowChunks = 0; RG.rowChunkLo = RG.rowChunkHi = 0; RG.ownRowLo = RG.ownRowHi = 0;
+    RG.nRows = 0; RG.nRowChunks = 0; RG.rowChunkLo = RG.rowChunkHi = 0; RG.ownRowLo = RG.ownRowHi = 0; RG.maxRegionRows = RG.maxRegionAxisRows = 0;
     part.redRowCut.assign((size_t)part.nranks + 1, 0);
     if (R > 0) {
         // the coupled reduced faces of the regions this rank builds rows for: all regions (one GPU, replicated setup) or its own;
@@ -746,8 +750,8 @@ void Solver::constructMatrixBlocks() {
         std::vector<int> perRA = rc.to_host(st, (size_t)3 * R);
         // chunk table: rows are sorted by (region, axis, voxel order); a chunk holds <= 2048 rows of one (region, axis)
         std::vector<int32_t> start((size_t)R + 1, 0), chunkStart((size_t)R + 1, 0), table, axisStart((size_t)3 * R + 1, 0);
-        RG.maxRegionRows = 0;
         for (int r = 0; r < R; ++r) RG.maxRegionRows = std::max(RG.maxRegionRows, (int32_t)(perRA[3 * r] + perRA[3 * r + 1] + perRA[3 * r + 2]));
+        for (int i = 0; i < 3 * R; ++i) RG.maxRegionAxisRows = std::max(RG.maxRegionAxisRows, (int32_t)perRA[i]);
         if (part.local) RG.maxRegionRows = (int32_t)std::llround(hostAllreduceSum((double)RG.maxRegionRows));      // every rank takes the same kernels (an upper bound is enough)
         int32_t pos = 0;
         for (int r = 0; r < R; ++r) {

@@ -80,6 +80,8 @@ struct RegionData {
     DBuf<int32_t> cellChunkStart, rowChunkStart;  // [R+1] first chunk of each region
     DBuf<int32_t> rowAxisStart;  // [3R+1] first coupled reduced row of (region, face axis): the row ranges of reduced_region_kernel
     int32_t maxRegionRows = 0;   // largest number of coupled reduced rows of one region (decides fused vs chunked reduced kernels)
+    int32_t maxRegionAxisRows = 0;                    // largest row count of one (region, face axis) built here (read-only count)
+    int32_t maxRegionCells = 0, minRegionCells = 0;   // REDUCED cells of the largest / smallest owned region (read-only counts)
     DBuf<int32_t> regionOrder;   // [R] launch order of reduced_region_kernel: the owned regions by decreasing row count (longest CTA first)
     DBuf<double> partial;    // per-chunk partial sums
     DBuf<double> t, s;       // [R][26] per-apply moment / B^-1 t
@@ -348,6 +350,7 @@ void reduced_finish(cudaStream_t, const Geom&, const RegionData&, const double* 
 void reduced_expand(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
 // the reduced term of one apply: w_f <- scale * c_f . B^-1 (sum_f c_f w_f); one fused launch for tiled regions, moments + expand otherwise
 void reduced_apply(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
+int region_path(const OpArgs&, const RegionData&);      // the kernels reduced_apply / pass1Apply choose (ps_pcg.cu)
 void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, bool reverse = false, const VecLink& V = VecLink());
 void k_cg_init(cudaStream_t, const RangeSet& own, const double* b, double* x, double* r, double* p, double* dotPartial, PcgScalars* scal, double tol, int maxIter, const PeerCtx& P);
 void k_cg_begin(cudaStream_t, PcgScalars* scal, const PeerCtx& P);

@@ -89,17 +89,7 @@ def test_oracle_bicgstab_fallback_matches_reference_code(built):
     assert abs(err - o.real("solveError")) <= 1e-6 * abs(err)
 
 
-def _scipy_operator(csr, dt):
-    """A = -dt K^T Mc^-1 K - J^T B^-1 J - 1/2 [0, 0; 0, mu^-1] by scipy.sparse from the component matrices `csr(name)`."""
-    import scipy.sparse as sp
-    M = {}
-    for name in ("McInv", "BInv", "uInv", "G", "JG", "Dt", "JDt"):
-        shape, ptr, idx, val = csr(name)
-        M[name] = sp.csr_matrix((val, idx, ptr), shape=shape)
-    K = sp.hstack([M["G"], M["Dt"]]).tocsr(); J = sp.hstack([M["JG"], M["JDt"]]).tocsr()
-    nP = M["G"].shape[1]
-    C22 = sp.block_diag([sp.csr_matrix((nP, nP)), M["uInv"]]).tocsr()
-    return (-dt * (K.T @ M["McInv"] @ K) - J.T @ M["BInv"] @ J - 0.5 * C22).tocsr()
+_scipy_operator = parity.scipy_operator
 
 
 def _product_vs_oracle(lib_path, sc):
