@@ -137,8 +137,11 @@ const char* ps_last_error(void);
  * reads, classifies, numbers and assembles only its slab plus a halo of a few layers, the global numbering follows from an
  * all-gather of per-slab counts (ps_part.hpp); with tilePadding 1 every rank classifies the whole grid redundantly.  Output
  * contract: a rank writes velocity and `valid` on ITS SLAB of the output arrays (cells / faces / edges with z in [zLo, zHi), the
- * last rank also the top layer); the rest of the arrays is not touched.  Reduced regions need doTile with tilePadding >= 1
- * (untiled regions may span slabs).
+ * last rank also the top layer); the rest of the arrays is not touched.  Reduced regions that cross a cut (doTile off, or
+ * tilePadding 0) are solved with a cross-rank reduction: each rank forms the moments of the region's rows in its slab, one
+ * all-reduce per operator apply sums them, and every rank solves the region's small system; the setup stays replicated for
+ * these configurations (ps_get_count "sharedRegions" counts such regions).  ps_set_params may switch doTile between steps: the
+ * cuts follow (multiples of 16 without tiles, of lcm(16, tileSize) with them).
  * cancel_cb must answer identically on all ranks. */
 /* ---- several GPUs behind ONE handle (SURVEY.md section 8b; the caller is one cook thread, exec/HDK_PolyStokes.C:222-345) ----
  * ps_create_multi builds the same slab decomposition inside one process: one rank per device devs[0..ndev) (NULL: devices

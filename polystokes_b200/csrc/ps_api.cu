@@ -520,6 +520,9 @@ int64_t ps_get_count(ps_handle h, const char* name) {
     if (n == "regionCount") return S.RG.count; if (n == "iterations") return S.solveIterations;
     if (n == "peerTransport") return S.peer.on ? 1 : 0;
     if (n == "slabLocal") return S.part.local ? 1 : 0;
+    if (n == "sharedRegions") return S.RG.nShared;
+    if (n == "sharedPeerExchanges") return S.sharedPeerExchanges;      // moment sums of shared regions since the last setup, peer transport
+    if (n == "sharedCommExchanges") return S.sharedCommExchanges;      // ... and by the communicator's all-reduce
     if (n == "directHalo") return S.fusedHalo ? 1 : 0;      // boundary entries stored straight into the neighbours' vectors (ps_peer.hpp, VecLink)
     if (n == "result") return S.result; if (n == "usedBiCGStab") return S.usedBiCGStab;
     if (n == "nRowsExt") return C.nRowsExt; if (n == "fixLoops") return S.fixLoops;

@@ -78,6 +78,11 @@ struct Partition {
     // S_Cls:1073-1172 never fires then).  Otherwise the setup is replicated on every rank as in round 1.
     bool local = false;
     int halo = 0;
+    // Reduced regions that may cross a cut (doTile off, or tiles without padding): the setup is replicated, a region belongs to the
+    // rank of its first cell (regions are numbered in voxel order, so regionCut stays monotone), and a region with reduced faces in
+    // more than one slab is SHARED: its coupled rows follow the slab of the face (the convention of the active rows, slotCut), and
+    // every operator apply sums its moments over the ranks (Solver::sharedApply).
+    bool spanning = false;
 };
 
 }  // namespace ps

@@ -1219,7 +1219,43 @@ void reduced_expand(cudaStream_t st, const Geom& g, const RegionData& RG, double
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
+void shared_moments(cudaStream_t st, const Geom& g, const RegionData& RG, const double* wRows, const PcgScalars* S) {
+    if (RG.nShChunks <= 0) return;
+    launch_chain(reduced_moments_kernel, (unsigned)RG.nShChunks, MOM_THREADS, st, g.dx, RG.rowXYZ.p, RG.shChunk.p, RG.shChunkStart.p, RG.com.p, wRows, RG.shPartial.p, RG.Binv.p, RG.sigma.p,
+                 (unsigned int*)nullptr, S, 0);
+    PS_COUNT_LAUNCH(1);
+    PS_CUDA(cudaGetLastError());
+}
+void shared_expand(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
+    if (RG.shRowHi <= RG.shRowLo) return;
+    const int n = RG.shRowHi - RG.shRowLo;
+    launch_chain(reduced_expand_kernel, (unsigned)std::min((n + RED_THREADS - 1) / RED_THREADS, sm_count() * 8), RED_THREADS, st, g.dx, RG.rowXYZ.p, RG.rowRegion.p, RG.com.p, RG.sigma.p, wRows, scale, S, RG.shRowLo, RG.shRowHi);
+    PS_COUNT_LAUNCH(1);
+    PS_CUDA(cudaGetLastError());
+}
 #else
+void shared_moments(cudaStream_t, const Geom& g, const RegionData& RG, const double* wRows, const PcgScalars* S) {
+    if (S && S->done) return;
+    for (int ch = 0; ch < RG.nShChunks; ++ch) {
+        const int region = RG.shChunk.p[4 * ch], begin = RG.shChunk.p[4 * ch + 1], end = RG.shChunk.p[4 * ch + 2];
+        double acc[10] = {0};
+        for (int row = begin; row < end; ++row) {
+            double m[10]; row_monomials(g.dx, RG.rowXYZ.p[row], RG.com.p + 3 * region, m);
+            for (int k = 0; k < 10; ++k) acc[k] += m[k] * wRows[row];
+        }
+        for (int k = 0; k < 10; ++k) RG.shPartial.p[(size_t)ch * 10 + k] = acc[k];
+    }
+}
+void shared_expand(cudaStream_t, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
+    if (S && S->done) return;
+    for (int row = RG.shRowLo; row < RG.shRowHi; ++row) {
+        const int region = RG.rowRegion.p[row], axis = (int)(RG.rowXYZ.p[row] >> 30);
+        double m[10]; row_monomials(g.dx, RG.rowXYZ.p[row], RG.com.p + 3 * region, m);
+        double v = 0.;
+        for (int k = 0; k < 10; ++k) v += RG.sigma.p[(size_t)region * 30 + axis * 10 + k] * m[k];
+        wRows[row] = scale * v;
+    }
+}
 void reduced_finish(cudaStream_t, const Geom&, const RegionData& RG, const double* extra, double extraScale, double tScale, const PcgScalars* S);
 void reduced_moments(cudaStream_t st, const Geom& g, const RegionData& RG, const double* wRows, const PcgScalars* S, bool solve) {
     if (S && S->done) return;
@@ -1264,6 +1300,90 @@ void reduced_expand(cudaStream_t, const Geom& g, const RegionData& RG, double* w
             wRows[row] = scale * v;
         }
     }
+}
+#endif
+// [nShared][3][10]: this rank's chunk partials of every shared slot, summed in chunk order (0 where it holds no rows); the caller sums
+// the table over the ranks.  Runs after `done` too: the all-reduce that follows is summed every time.
+void shared_pack(cudaStream_t st, const RegionData& RG) {
+    const int32_t* cs = RG.shChunkStart.p; const int32_t* chunk = RG.shChunk.p; const double* partial = RG.shPartial.p; double* mom = RG.shMoments.p;
+    ps_for(st, (int64_t)RG.nShared * 30, PS_LAMBDA(int64_t i) {
+        const int j = (int)(i / 30), axis = (int)(i % 30) / 10, k = (int)(i % 10);
+        double s = 0.;
+        for (int ch = cs[j]; ch < cs[j + 1]; ++ch) if (chunk[4 * ch + 3] == axis) s += partial[(size_t)ch * 10 + k];
+        mom[i] = s;
+    });
+}
+// the small solve of one shared region from its summed moments M: t, s = B^-1 (extraScale extra + tScale t), sigma (both transports)
+PS_D void shared_solve_slot(const double* M, int r, const double* Binv, const double* extra, double extraScale, double tScale, double* sOut, double* sigma) {
+    double t[RDOF], sv[RDOF], sg[30];
+    moments_to_t(M, t);
+    for (int n = 0; n < RDOF; ++n) { double v = tScale * t[n]; if (extra) v += extraScale * extra[(size_t)r * RDOF + n]; t[n] = v; }
+    const double* B = Binv + (size_t)r * RDOF * RDOF;
+    for (int a = 0; a < RDOF; ++a) { double s = 0.; for (int b = 0; b < RDOF; ++b) s += B[a * RDOF + b] * t[b]; sv[a] = s; if (sOut) sOut[(size_t)r * RDOF + a] = s; }
+    s_to_sigma(sv, sg);
+    for (int k = 0; k < 30; ++k) sigma[(size_t)r * 30 + k] = sg[k];
+}
+// the small solve of the slots this rank takes part in, from shMoments (summed over the ranks by the communicator)
+// (every rank that holds rows of the region forms the same s from the same sums)
+void shared_finish(cudaStream_t st, const RegionData& RG, const double* extra, double extraScale, double tScale, double* sOut, const PcgScalars* S) {
+    const int32_t* mine = RG.shMine.p; const int32_t* reg = RG.shRegion.p; const double* mom = RG.shMoments.p; const double* Binv = RG.Binv.p;
+    double* sigma = RG.sigma.p;
+    ps_for(st, RG.nShMine, PS_LAMBDA(int64_t i) {
+        if (S && S->done) return;
+        const int j = mine[i];
+        double M[30];
+        for (int k = 0; k < 30; ++k) M[k] = tScale != 0. ? mom[(size_t)j * 30 + k] : 0.;
+        shared_solve_slot(M, reg[j], Binv, extra, extraScale, tScale, sOut, sigma);
+    });
+}
+#ifndef PS_EMULATE
+// Peer transport.  CTA d packs this rank's [nShared][30] moments (chunk partials summed in chunk order, as shared_pack) straight into
+// row [parity][rank] of rank d's moment area, fences, and raises flag [parity][rank] there.  Runs after `done` too: the finish kernels
+// of every rank wait for every exchange, so the sequence numbers stay in step.
+__global__ void __launch_bounds__(256) shared_push_kernel(const int32_t* __restrict__ cs, const int32_t* __restrict__ chunk, const double* __restrict__ partial, int nShared,
+                                                          const __grid_constant__ SharedPeer P) {    pdl_sync();
+    const int d = blockIdx.x, par = (int)(P.seq & 1ull);
+    double* dst = P.val[d] + ((size_t)par * PEER_MAX_RANKS + P.rank) * P.stride;
+    for (int i = threadIdx.x; i < nShared * 30; i += blockDim.x) {
+        const int j = i / 30, axis = (i % 30) / 10, k = i % 10;
+        double s = 0.;
+        for (int ch = cs[j]; ch < cs[j + 1]; ++ch) if (chunk[4 * ch + 3] == axis) s += partial[(size_t)ch * 10 + k];
+        peer_st_f64(dst + i, s);
+    }
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) peer_st_flag(P.flag[d] + par * PEER_MAX_RANKS + P.rank, P.seq);
+}
+// one warp per slot this rank takes part in: wait for the N ranks' rows of this exchange (time-out -> peerError), sum them in rank
+// order (the same sums on every rank), then the slot's small solve
+__global__ void __launch_bounds__(32) shared_finish_peer_kernel(const int32_t* __restrict__ mine, const int32_t* __restrict__ reg, const double* __restrict__ Binv,
+                                                                const double* __restrict__ extra, double extraScale, double tScale, double* sOut, double* sigma,
+                                                                const PcgScalars* S, PcgScalars* err, const __grid_constant__ SharedPeer P) {    pdl_sync();
+    __shared__ double M[30];
+    const int lane = threadIdx.x, par = (int)(P.seq & 1ull);
+    bool good = true;
+    if (lane < P.nranks) good = peer_wait_flag(P.flag[P.rank] + par * PEER_MAX_RANKS + lane, P.seq);
+    good = __all_sync(0xffffffffu, good);
+    if (!good) { if (lane == 0) err->peerError = 1; return; }
+    if (S && S->done) return;
+    const int j = mine[blockIdx.x];
+    if (lane < 30) {
+        double s = 0.;
+        for (int q = 0; q < P.nranks; ++q) s += peer_ld_f64(P.val[P.rank] + ((size_t)par * PEER_MAX_RANKS + q) * P.stride + (size_t)j * 30 + lane);
+        M[lane] = s;
+    }
+    __syncwarp();
+    if (lane == 0) shared_solve_slot(M, reg[j], Binv, extra, extraScale, tScale, sOut, sigma);
+}
+void shared_exchange_peer(cudaStream_t st, const RegionData& RG, const SharedPeer& P, const double* extra, double extraScale, double tScale, double* sOut,
+                          const PcgScalars* S, PcgScalars* err) {
+    launch_chain(shared_push_kernel, (unsigned)P.nranks, 256, st, RG.shChunkStart.p, RG.shChunk.p, RG.shPartial.p, (int)RG.nShared, P);
+    PS_COUNT_LAUNCH(1);
+    PS_CUDA(cudaGetLastError());
+    if (RG.nShMine <= 0) return;
+    launch_chain(shared_finish_peer_kernel, (unsigned)RG.nShMine, 32, st, RG.shMine.p, RG.shRegion.p, RG.Binv.p, extra, extraScale, tScale, sOut, RG.sigma.p, S, err, P);
+    PS_COUNT_LAUNCH(1);
+    PS_CUDA(cudaGetLastError());
 }
 #endif
 
@@ -1392,6 +1512,10 @@ void k_recover_active(cudaStream_t st, const Geom& g, const RowSet& rows, const 
     ps_for(st, R.total(), PS_LAMBDA(int64_t l) { const int64_t i = R.at(l); velSol[i] = dt * (mcInv[i] * (invDt * rhsU[i])) - wAct[i]; });
 }
 
+PS_HD bool face_is_mine(const FaceOwner& own, int ri, int z) {
+    if (own.shared && own.shared[ri]) return z >= own.zLo && (z < own.zHi || own.zHi >= own.nz);
+    return ri >= own.regLo && ri < own.regHi;
+}
 // W2 applySolutionToVelocity (S.cpp:937-1028) fused with buildValidFaces (S_Cls:4-54).  With several ranks a
 // face carrying a DOF is written by the rank that owns the DOF; faces without one are written by everybody.
 // Visits the faces [lo, hi); `valid` is written on [validLo, validHi) only (the part of the field this rank delivers).
@@ -1411,8 +1535,8 @@ void k_writeback_velocity(cudaStream_t st, const Geom& g, const Fields& F, const
         const int ri = haveReduced ? FR[q] : -1;
         const int ai = FA[q];
         if (ri >= 0) {
-            if (ri < own.regLo || ri >= own.regHi) return;
             const I3 f = delin(g, SL_FACE + axis, q);
+            if (!face_is_mine(own, ri, f.z)) return;
             double ox, oy, oz, c[RDOF];
             face_offset(g, f, axis, com + 3 * ri, ox, oy, oz);
             conversion_coefficients(ox, oy, oz, axis, c);
@@ -1435,7 +1559,7 @@ void k_merge_face_plane(cudaStream_t st, const Geom& g, const Fields& F, int axi
         const int lab = FL[q];
         if (lab == L_UNSOLVED || lab == L_UNASSIGNED) return;
         const int ri = FR[q], ai = FA[q];
-        const bool mine = ri >= 0 ? (ri >= own.regLo && ri < own.regHi) : (ai >= 0 ? (ai >= own.aLo && ai < own.aHi) : true);
+        const bool mine = ri >= 0 ? face_is_mine(own, ri, k) : (ai >= 0 ? (ai >= own.aLo && ai < own.aHi) : true);
         if (!mine) velOut[q] = peerPlane[i];
     });
 }

@@ -22,6 +22,10 @@ namespace ps {
 constexpr int PEER_MAX_RANKS = 8;
 constexpr int PEER_SLOTS = 2;      // reduction slots: 0 (p.Ap, r.Ap, Ap.Ap) of pass 2, 1 (r.r, x.p, p.p) of the x/r/p update (or b.b, 0, b.b from init)
 constexpr int PEER_VALS = 3;       // values per reduction
+// Shared-region moments (Solver::sharedApply): behind the halo buffers every block holds flags [parity][source rank] and values
+// [parity][source rank][PEER_SH_CAP][30]; a step with more shared regions takes the communicator's all-reduce instead
+constexpr int PEER_SH_CAP = 4096;
+constexpr size_t PEER_SH_FLAG_BYTES = 256;
 
 struct PeerSync {                  // head of every rank's symmetric block
     unsigned long long haloFlag[2][2][2];                      // [kind x|w][parity][side: from below | from above]
@@ -56,6 +60,15 @@ struct PeerCtx {                   // passed by value to the CG kernels; nranks 
     PeerSync* sync[PEER_MAX_RANKS] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 };
 
+// the moment exchange of the shared regions, by value to its two kernels: every rank's flags and values, this exchange's sequence number
+struct SharedPeer {
+    int nranks = 1, rank = 0;
+    unsigned long long seq = 0;
+    size_t stride = 0;                            // doubles per [parity][source rank] row (shCap * 30)
+    unsigned long long* flag[PEER_MAX_RANKS] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    double* val[PEER_MAX_RANKS] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+};
+
 // host-side state of the peer transport of one solver
 struct PeerLink {
     bool on = false;
@@ -71,9 +84,14 @@ struct PeerLink {
     void* vecPublished = nullptr;
     size_t vecOffW = 0;                          // offset of w in EVERY rank's arena this step (doubles; from the global system size)
     bool vecReady = false;
+    size_t shCap = 0;                            // shared-region slots of the moment area
+    unsigned long long seqSh = 0;
     PeerSync* sync(int r) const { return (PeerSync*)block[r]; }
     double* recv(int r, int kind, int par, int side) const { return (double*)((char*)block[r] + sizeof(PeerSync)) + ((size_t)((kind * 2 + par) * 2 + side)) * cap; }
-    size_t bytes() const { return sizeof(PeerSync) + 8 * cap * sizeof(double); }
+    size_t shOff() const { return sizeof(PeerSync) + 8 * cap * sizeof(double); }
+    unsigned long long* shFlag(int r) const { return (unsigned long long*)((char*)block[r] + shOff()); }          // [2][PEER_MAX_RANKS]
+    double* shVal(int r) const { return (double*)((char*)block[r] + shOff() + PEER_SH_FLAG_BYTES); }             // [2][PEER_MAX_RANKS][shCap * 30]
+    size_t bytes() const { return shOff() + PEER_SH_FLAG_BYTES + (size_t)2 * PEER_MAX_RANKS * shCap * 30 * sizeof(double); }
     PeerCtx ctx() const { PeerCtx c; if (on) { c.nranks = nranks; c.rank = rank; for (int r = 0; r < nranks; ++r) c.sync[r] = sync(r); } return c; }
 };
 

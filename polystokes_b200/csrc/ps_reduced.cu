@@ -19,8 +19,8 @@ void k_region_com(cudaStream_t st, const Geom& g, const Fields& F, int32_t R, un
     const int8_t* L = F.label[SL_CENTER]; const int32_t* Rg = F.ridx[SL_CENTER];
     dev_memset(sums, 0, (size_t)R * 4 * sizeof(unsigned long long), st);
     int64_t lo, hi;
-    z_range(g, SL_CENTER, g.zLo, g.zHi, lo, hi);          // the rank's own cells: a region never crosses a z cut
-    if (!g.slabLocal) { lo = 0; hi = g.n[SL_CENTER]; }     // one GPU / replicated setup: every region
+    z_range(g, SL_CENTER, g.zLo, g.zHi, lo, hi);          // the rank's own cells: with slab-local setup a region never crosses a z cut
+    if (!g.slabLocal) { lo = 0; hi = g.n[SL_CENTER]; }     // one GPU / replicated setup (regions crossing cuts included): every region
     ps_for_range(st, lo, hi, PS_LAMBDA(int64_t q) {
         if (L[q] != L_REDUCED) return;
         const int r = Rg[q];
@@ -542,8 +542,8 @@ __global__ void __launch_bounds__(32) region_factor_kernel(double invDt, int reg
 // sums the chunk moments of every owned region in chunk order, expands them to M_r, N_r, (JD^T mu DJ^T)_r and the
 // least-squares right-hand side, then factorises
 void region_gram_finish(cudaStream_t st, const Geom& g, RegionData& RG, int nChunks) {
-    // only the regions this rank owns [regLo, regHi) (all of them on one GPU)
-    const int R0 = RG.regLo, R = RG.regHi - RG.regLo;
+    // only the regions this rank builds [bldLo, regHi) (all of them on one GPU)
+    const int R0 = RG.bldLo, R = RG.regHi - RG.bldLo;
     if (R <= 0) return;
     if (RG.tables.n < (size_t)TAB_COUNT) { std::vector<double> T(TAB_COUNT); build_region_tables(T.data()); RG.tables.from_host(st, T.data(), T.size()); }
     RG.moments.alloc((size_t)RG.count * MOM_COUNT);

@@ -42,6 +42,30 @@ static void k_rows_finalize(cudaStream_t st, const Geom& g, int64_t n, const int
 static void k_scale_rows(cudaStream_t st, int64_t n, const double* a, const double* b, double* out) {
     ps_for(st, n, PS_LAMBDA(int64_t i) { out[i] = a[i] * b[i]; });
 }
+// slab of a face plane / cell layer z: rank k holds [zCut[k], zCut[k+1]), the last one also z = nz (the convention of slotCut)
+PS_HD int slab_of(const int32_t* zCut, int nranks, int z) { int k = 0; while (k + 1 < nranks && z >= zCut[k + 1]) ++k; return k; }
+static void k_gather_first(cudaStream_t st, int32_t R, const int32_t* list, const int32_t* start, int32_t* first) {
+    ps_for(st, R, PS_LAMBDA(int64_t r) { first[r] = list[start[r]]; });
+}
+// touch[region * nranks + k] = 1 if the region has a reduced face in slab k
+static void k_region_face_slabs(cudaStream_t st, const Geom& g, int slot, const int32_t* FR, const int32_t* zCut, int nranks, uint8_t* touch) {
+    ps_for(st, g.n[slot], PS_LAMBDA(int64_t q) {
+        const int ri = FR[q];
+        if (ri >= 0) touch[(int64_t)ri * nranks + slab_of(zCut, nranks, delin(g, slot, q).z)] = 1;
+    });
+}
+// sort key of a coupled reduced row: (slab of the face, shared, region) -- a rank's own rows first, those of shared regions last
+static void k_span_row_keys(cudaStream_t st, const Geom& g, int64_t n, const int32_t* rowFace, const uint8_t* shared, const int32_t* zCut, int nranks, int32_t R, int32_t* keys) {
+    ps_for(st, n, PS_LAMBDA(int64_t i) {
+        const int32_t packed = rowFace[i], r = keys[i];
+        const int axis = (packed >> 29) & 3;
+        const int k = slab_of(zCut, nranks, delin(g, SL_FACE + axis, (int64_t)(packed & 0x1fffffff)).z);
+        keys[i] = (2 * k + shared[r]) * R + r;
+    });
+}
+static void k_key_region(cudaStream_t st, int64_t n, const int32_t* keys, int32_t R, int32_t* region) {
+    ps_for(st, n, PS_LAMBDA(int64_t i) { region[i] = keys[i] % R; });
+}
 static void k_copy_reduced_solution(cudaStream_t st, int64_t n, const double* s, double* velSolReduced) {
     ps_for(st, n, PS_LAMBDA(int64_t i) { velSolReduced[i] = s[i]; });
 }
@@ -94,11 +118,9 @@ void Solver::initComm(Comm* c) {
 // the slab decomposition as a function of the grid and the tiling / layer parameters (ps_comm_init, ps_set_params)
 void Solver::computePartition(int rank, int nranks) {
     int unit = 16;
-    if (P.doReducedRegions) {
-        if (nranks > 1 && (!P.doTile || P.tilePadding < 1 || P.tileSize < 1))
-            throw Error("ps_comm_init: reduced regions need doTile with tilePadding >= 1 on more than one GPU (untiled regions may span slabs)");
-        if (P.doTile && P.tileSize >= 1) unit = 16 / gcd_i(16, P.tileSize) * P.tileSize;
-    }
+    if (P.doReducedRegions && P.doTile && P.tileSize >= 1) unit = 16 / gcd_i(16, P.tileSize) * P.tileSize;
+    // untiled regions, or tiles without padding, may reach across a cut: shared regions (ps_part.hpp), replicated setup
+    part.spanning = nranks > 1 && P.doReducedRegions && (!P.doTile || P.tilePadding < 1 || P.tileSize < 1);
     const int nUnits = (g.nz + unit - 1) / unit;
     if (nranks > nUnits) throw Error("ps_comm_init: more ranks than z-slabs of lcm(16, tileSize) cells");
     part.rank = rank; part.nranks = nranks;
@@ -159,6 +181,7 @@ void Solver::setupPeer() {
     if (env && std::string(env) == "nccl") return;
     peer.rank = part.rank; peer.nranks = part.nranks;
     peer.cap = (size_t)12 * (g.nx + 1) * (g.ny + 1);
+    peer.shCap = PEER_SH_CAP;
     double okLocal = 1.;
     void* mine = nullptr;
     if (cudaMalloc(&mine, peer.bytes()) != cudaSuccess) { cudaGetLastError(); okLocal = 0.; mine = nullptr; }
@@ -309,7 +332,9 @@ void Solver::peerResync() {
     if (any < 0.5) return;
     stream_sync(st);
     PS_CUDA(cudaMemsetAsync(peer.block[peer.rank], 0, sizeof(PeerSync), st));
+    PS_CUDA(cudaMemsetAsync(peer.shFlag(peer.rank), 0, PEER_SH_FLAG_BYTES, st));
     dev_memset(&scal.p->peerError, 0, sizeof(int), st);
+    peer.seqSh = 0;
     for (auto& q : peer.seqHalo) q = 0;
     for (auto& q : peer.seqRed) q = 0;
     for (auto& q : peer.seqVec) q = 0;
@@ -655,9 +680,14 @@ void Solver::computeReducedRegionMatrices() {
     std::vector<unsigned long long> hs = sums.to_host(st, (size_t)4 * R);
     std::vector<int> perRegion((size_t)R);
     for (int r = 0; r < R; ++r) perRegion[r] = (int)hs[4 * r + 3];
+    std::vector<int32_t> start, table, chunkStart;
+    build_chunks(perRegion, 256, start, table, chunkStart);
+    RG.cellStart.from_host(st, start.data(), start.size());
     // region -> rank: regions are numbered by their first cell in voxel order (z-slowest tiles) and never span a
-    // z cut, so every rank owns one contiguous id range (slab-local setup: already known from the all-gathered counts)
-    if (!part.local) {
+    // z cut, so every rank owns one contiguous id range (slab-local setup: already known from the all-gathered counts;
+    // regions that may span a cut: classifySharedRegions)
+    if (part.spanning) classifySharedRegions();
+    else if (!part.local) {
         int owner = 0;
         for (int r = 0; r < R; ++r) {
             const int zmean = (int)(hs[4 * r + 2] / std::max<unsigned long long>(hs[4 * r + 3], 1ull));
@@ -669,15 +699,13 @@ void Solver::computeReducedRegionMatrices() {
         while (owner < part.nranks) part.regionCut[++owner] = R;
     }
     RG.regLo = part.regionCut[part.rank]; RG.regHi = part.regionCut[part.rank + 1];
+    if (!part.spanning) RG.bldLo = RG.regLo;
     if (RG.regHi > RG.regLo) {
         const auto mm = std::minmax_element(perRegion.begin() + RG.regLo, perRegion.begin() + RG.regHi);
         RG.minRegionCells = *mm.first; RG.maxRegionCells = *mm.second;
     }
-    std::vector<int32_t> start, table, chunkStart;
-    build_chunks(perRegion, 256, start, table, chunkStart);
     RG.nCellChunks = (int32_t)(table.size() / 3);
-    RG.cellChunkLo = chunkStart[RG.regLo]; RG.cellChunkHi = chunkStart[RG.regHi];
-    RG.cellStart.from_host(st, start.data(), start.size());
+    RG.cellChunkLo = chunkStart[RG.bldLo]; RG.cellChunkHi = chunkStart[RG.regHi];
     RG.cellChunk.from_host(st, table.data(), table.size());
     RG.cellChunkStart.from_host(st, chunkStart.data(), chunkStart.size());
     const size_t NN = (size_t)RDOF * RDOF;
@@ -687,6 +715,48 @@ void Solver::computeReducedRegionMatrices() {
     RG.t.alloc((size_t)R * RDOF); RG.s.alloc((size_t)R * RDOF);
     region_gram_partials(st, g, F, RG, RG.partial.p);
     region_gram_finish(st, g, RG, RG.nCellChunks);
+}
+
+// Partition::spanning.  Owner of a region = slab of its first cell in voxel order (RG.cellList is sorted by (region, voxel order)); a
+// region with reduced faces in more than one slab, or in one slab that is not its owner's, is shared.  Everything follows from the
+// replicated classification: every rank derives the same owners and the same shared list.  This rank builds the region matrices
+// of the contiguous id range from the lowest shared region it takes part in (rows or reduced faces in its slab) to its last own
+// region: the regions of the lower ranks numbered in between are built too.  When region 0 crosses every cut (one untiled body)
+// that is every region up to this rank's last one -- on the top rank the whole Gram build.
+void Solver::classifySharedRegions() {
+    const int R = RG.count, N = part.nranks, me = part.rank;
+    zCutDev.from_host(st, part.zCut.data(), part.zCut.size());
+    DBuf<int32_t>& first = scratch().rc;
+    first.alloc((size_t)R);
+    k_gather_first(st, R, RG.cellList.p, RG.cellStart.p, first.p);
+    DBuf<uint8_t>& touch = scratch().haloFlag;
+    touch.alloc((size_t)R * N); touch.zero(st, (size_t)R * N);
+    for (int a = 0; a < 3; ++a) k_region_face_slabs(st, g, SL_FACE + a, F.ridx[SL_FACE + a], zCutDev.p, N, touch.p);
+    const std::vector<int32_t> fh = first.to_host(st, (size_t)R);
+    const std::vector<uint8_t> th = touch.to_host(st, (size_t)R * N);
+    std::vector<int32_t> shList, mine;
+    std::vector<uint8_t> flag((size_t)R, 0);
+    int owner = 0, lo = INT_MAX;
+    for (int r = 0; r < R; ++r) {
+        const int k = slab_of(part.zCut.data(), N, delin(g, SL_CENTER, fh[r]).z);
+        if (k < owner) throw Error("region numbering is not monotone in z: cannot slab-decompose these reduced regions");
+        while (owner < k) part.regionCut[++owner] = r;
+        int slabs = 0;
+        for (int j = 0; j < N; ++j) slabs += th[(size_t)r * N + j];
+        if (slabs > 1 || (slabs == 1 && !th[(size_t)r * N + k])) {
+            flag[r] = 1;
+            if (th[(size_t)r * N + me] || k == me) { mine.push_back((int32_t)shList.size()); lo = std::min(lo, r); }
+            shList.push_back(r);
+        }
+    }
+    while (owner < N) part.regionCut[++owner] = R;
+    RG.bldLo = std::min(lo, part.regionCut[me]);
+    RG.nShared = (int32_t)shList.size(); RG.nShMine = (int32_t)mine.size();
+    RG.shRegion.from_host(st, shList.data(), shList.size() + 0);
+    RG.shMine.from_host(st, mine.data(), mine.size());
+    RG.shFlag.from_host(st, flag.data(), flag.size());
+    RG.shMoments.alloc((size_t)RG.nShared * 30 + 1);
+    stream_sync(st);      // the host vectors die here
 }
 
 // constructMatrixBlocks (S_CMB:9-868): row numbering of K_ext, then the ELL fills
@@ -737,23 +807,37 @@ void Solver::constructMatrixBlocks() {
             if (part.local) z_range(g, SL_FACE + a, g.zLo, std::min(g.nz, g.zHi + 1), lo, hi);
             k_collect_region_keys(st, g, scratch32[a].p, scratch8[a].p, F.ridx[SL_FACE + a], lo, hi, (int32_t)(a << 29), (int32_t)off[a], lk.p, lv.p);
         }
+        // shared regions (Partition::spanning): the rows go by the slab of the face, the rank's shared rows after its other rows
+        const int KM = part.spanning ? 2 * part.nranks : 1;
+        if ((int64_t)R * KM >= INT32_MAX) throw Error("too many reduced regions x ranks for 32-bit row keys");
+        if (part.spanning) k_span_row_keys(st, g, nLocal, lv.p, RG.shFlag.p, zCutDev.p, part.nranks, R, lk.p);
         DBuf<int32_t>& kt = scratch().kt; DBuf<int32_t>& vt = scratch().vt;
-        sort_pairs_by_key(st, nLocal, key_bits(R), lk, lv, kt, vt);
-        copy_d2d(RG.rowRegion.p + rowOff, lk.p, (size_t)nLocal * sizeof(int32_t), st);
+        sort_pairs_by_key(st, nLocal, key_bits((int64_t)R * KM), lk, lv, kt, vt);
+        if (part.spanning) k_key_region(st, nLocal, lk.p, R, RG.rowRegion.p);
+        else copy_d2d(RG.rowRegion.p + rowOff, lk.p, (size_t)nLocal * sizeof(int32_t), st);
         copy_d2d(RG.rowFace.p + rowOff, lv.p, (size_t)nLocal * sizeof(int32_t), st);
         if (C.nActiveVs + nRows >= INT32_MAX) throw Error("K_ext has too many rows for int32");
         k_krow_reduced(st, nLocal, RG.rowFace.p + rowOff, (int32_t)(C.nActiveVs + rowOff), F.krow[0], F.krow[1], F.krow[2]);
         DBuf<int>& rc = scratch().rc;
-        rc.alloc((size_t)3 * R); rc.zero(st, (size_t)3 * R);
+        rc.alloc((size_t)3 * R * KM); rc.zero(st, (size_t)3 * R * KM);
         RG.rowXYZ.alloc((size_t)nRows + 1);
-        k_rows_finalize(st, g, nLocal, RG.rowRegion.p + rowOff, RG.rowFace.p + rowOff, rc.p, RG.rowXYZ.p + rowOff);
-        std::vector<int> perRA = rc.to_host(st, (size_t)3 * R);
+        k_rows_finalize(st, g, nLocal, part.spanning ? lk.p : RG.rowRegion.p + rowOff, RG.rowFace.p + rowOff, rc.p, RG.rowXYZ.p + rowOff);
+        const std::vector<int> perRAall = rc.to_host(st, (size_t)3 * R * KM);
+        // row counts per (region, axis) of the rows laid out below: all of them, or this rank's rows of its unshared regions
+        const int* perRA = perRAall.data() + (part.spanning ? (size_t)3 * R * (2 * part.rank) : 0);
+        if (part.spanning) {
+            for (int k = 0; k < part.nranks; ++k) {
+                int64_t n = 0;
+                for (size_t i = (size_t)3 * R * (2 * k); i < (size_t)3 * R * (2 * k + 2); ++i) n += perRAall[i];
+                part.redRowCut[k + 1] = part.redRowCut[k] + n;
+            }
+        }
         // chunk table: rows are sorted by (region, axis, voxel order); a chunk holds <= 2048 rows of one (region, axis)
         std::vector<int32_t> start((size_t)R + 1, 0), chunkStart((size_t)R + 1, 0), table, axisStart((size_t)3 * R + 1, 0);
         for (int r = 0; r < R; ++r) RG.maxRegionRows = std::max(RG.maxRegionRows, (int32_t)(perRA[3 * r] + perRA[3 * r + 1] + perRA[3 * r + 2]));
         for (int i = 0; i < 3 * R; ++i) RG.maxRegionAxisRows = std::max(RG.maxRegionAxisRows, (int32_t)perRA[i]);
         if (part.local) RG.maxRegionRows = (int32_t)std::llround(hostAllreduceSum((double)RG.maxRegionRows));      // every rank takes the same kernels (an upper bound is enough)
-        int32_t pos = 0;
+        int32_t pos = part.spanning ? (int32_t)part.redRowCut[part.rank] : 0;
         for (int r = 0; r < R; ++r) {
             if (part.local && r == RG.regLo) pos = (int32_t)rowOff;      // the regions below belong to other ranks (no rows here)
             start[r] = pos; chunkStart[r] = (int32_t)(table.size() / 4);
@@ -769,7 +853,30 @@ void Solver::constructMatrixBlocks() {
         RG.rowChunkLo = chunkStart[RG.regLo]; RG.rowChunkHi = chunkStart[RG.regHi];
         RG.ownRowLo = start[RG.regLo]; RG.ownRowHi = start[RG.regHi];
         RG.regionTicket.alloc((size_t)R + 1); RG.regionTicket.zero(st, (size_t)R + 1);
-        if (!part.local) for (int k = 0; k <= part.nranks; ++k) part.redRowCut[k] = start[part.regionCut[k]];
+        if (!part.local && !part.spanning) for (int k = 0; k <= part.nranks; ++k) part.redRowCut[k] = start[part.regionCut[k]];
+        if (part.spanning) {      // this rank's rows of the shared regions: chunks of <= 2048 rows of one (region, axis), per slot
+            const int* shRA = perRAall.data() + (size_t)3 * R * (2 * part.rank + 1);
+            const std::vector<int32_t> shList = RG.shRegion.to_host(st, (size_t)RG.nShared);
+            std::vector<int32_t> shTable, shStart((size_t)RG.nShared + 1, 0);
+            RG.shRowLo = pos;
+            for (int j = 0; j < RG.nShared; ++j) {
+                const int r = shList[j];
+                shStart[j] = (int32_t)(shTable.size() / 4);
+                for (int a = 0; a < 3; ++a) {
+                    const int32_t e = pos + shRA[3 * r + a];
+                    for (int32_t b = pos; b < e; b += 2048) { shTable.push_back(r); shTable.push_back(b); shTable.push_back(std::min(b + 2048, e)); shTable.push_back(a); }
+                    pos = e;
+                }
+            }
+            shStart[RG.nShared] = (int32_t)(shTable.size() / 4);
+            RG.shRowHi = pos;
+            if (pos != part.redRowCut[part.rank + 1]) throw Error("shared-region row layout does not match the row cut");
+            RG.nShChunks = (int32_t)(shTable.size() / 4);
+            RG.shChunk.from_host(st, shTable.data(), shTable.size() + 0);
+            RG.shChunkStart.from_host(st, shStart.data(), shStart.size());
+            RG.shPartial.alloc((size_t)RG.nShChunks * 10 + 1);
+            stream_sync(st);
+        }
         axisStart[(size_t)3 * R] = pos;
         RG.rowAxisStart.from_host(st, axisStart.data(), axisStart.size());
         {   // one CTA per region: start the long ones first, so that the last wave is made of short CTAs
@@ -1078,12 +1185,49 @@ static OpArgs make_op(const Solver& S) {
 OpArgs Solver::make_op_args() const { return make_op(*this); }
 
 // pass 1 of an operator apply including the reduced term: w = [dt Mc^-1 K x ; c_f . B^-1 J x]
-void Solver::pass1Apply(const OpArgs& A, const double* xin, const PcgScalars* S, bool reverse, const VecLink& V) {
+void Solver::pass1Apply(const OpArgs& A, const double* xin, const PcgScalars* S, bool reverse, const VecLink& V, bool withShared) {
 #ifndef PS_EMULATE
-    if (RG.count > 0 && !reverse && k_pass1_regions(st, A, xin, w.p, g.dt, S, g, RG, 1.0, V)) return;      // active rows and regions in one launch
+    if (RG.count > 0 && !reverse && k_pass1_regions(st, A, xin, w.p, g.dt, S, g, RG, 1.0, V)) {}      // active rows and regions in one launch
+    else
 #endif
-    k_pass1(st, A, xin, w.p, g.dt, S, reverse, 0, V);       // V: wait for the neighbours' entries of x at the head (direct halo stores)
-    if (RG.count > 0) reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, S);          // moments -> B^-1 -> expand, one CTA per region
+    {
+        k_pass1(st, A, xin, w.p, g.dt, S, reverse, 0, V);       // V: wait for the neighbours' entries of x at the head (direct halo stores)
+        if (RG.count > 0) reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, S);          // moments -> B^-1 -> expand, one CTA per region
+    }
+    if (withShared) sharedApply(w.p + C.nActiveVs, nullptr, 0.0, 1.0, 1.0, nullptr, S);
+}
+
+// Shared regions: every rank forms the 3 x 10 moments of its own rows of them, the packed table [nShared][30] is summed over the
+// ranks, then every rank solves the regions it takes part in and expands s_r onto its own rows.  The sum travels
+//   * with the peer transport: straight into every rank's moment area of the symmetric blocks, summed in rank order by the waiting
+//     finish kernel (time-outs set peerError like every other peer wait) -- two launches, no collective;
+//   * otherwise, and in a step with more shared regions than that area holds (PEER_SH_CAP): ONE all-reduce of the communicator
+//     (NCCL, or the host callbacks of the emulation twin), which hands every rank the same sums.
+// Either way every rank forms the same s_r.  One more synchronisation point per apply, in every step with nShared > 0 (the same on
+// all ranks); none otherwise.
+void Solver::sharedApply(double* wRows, const double* extra, double extraScale, double tScale, double scale, double* sOut, const PcgScalars* S) {
+    if (RG.nShared <= 0) return;
+    bool solved = false;
+    if (tScale != 0.) {
+        shared_moments(st, g, RG, wRows, S);
+#ifndef PS_EMULATE
+        if (peer.on && (size_t)RG.nShared <= peer.shCap) {
+            SharedPeer sp;
+            sp.nranks = peer.nranks; sp.rank = peer.rank; sp.seq = ++peer.seqSh; sp.stride = peer.shCap * 30;
+            for (int r = 0; r < peer.nranks; ++r) { sp.flag[r] = peer.shFlag(r); sp.val[r] = peer.shVal(r); }
+            shared_exchange_peer(st, RG, sp, extra, extraScale, tScale, sOut, S, scal.p);
+            ++sharedPeerExchanges;
+            solved = true;
+        }
+#endif
+        if (!solved) {
+            shared_pack(st, RG);
+            if (part.multi() && comm) comm->allreduce_sum(RG.shMoments.p, 30 * RG.nShared, st);
+            ++sharedCommExchanges;
+        }
+    }
+    if (!solved) shared_finish(st, RG, extra, extraScale, tScale, sOut, S);
+    if (scale != 0.) shared_expand(st, g, RG, wRows, scale, S);
 }
 
 // assembleSystemPressureStressFactored (S_AS:432-470):
@@ -1101,6 +1245,7 @@ void Solver::assemble() {
     if (RG.count > 0) {
         reduced_finish(st, g, RG, RG.rhsR.p, 1.0, 0.0, nullptr);                     // s = B^-1 rhs_r
         reduced_expand(st, g, RG, w.p + C.nActiveVs, g.invDt, nullptr);
+        sharedApply(w.p + C.nActiveVs, RG.rhsR.p, 1.0, 0.0, g.invDt, nullptr, nullptr);     // rhs_r is replicated: no reduction
     }
     exchange(haloW, w.p, nullptr);            // the neighbours' coupled reduced rows (active rows are replicated above)
     k_pass2(st, A, w.p, nullptr, b.p, 0.0, rhsPT.p, nullptr, PeerCtx(), nullptr, 0);
@@ -1120,7 +1265,7 @@ void Solver::timedOperator(int which) {
     if (which == 0) { applyOperator(b.p, Ap.p, nullptr); return; }
     if (which == 1) pass1Apply(A, b.p, nullptr);                       // includes the reduced term (fused region epilogue)
     else if (which == 3) k_pass1(st, A, b.p, w.p, g.dt, nullptr);            // the sweep alone (raw products on the coupled reduced rows)
-    else if (which == 6 && RG.count > 0) reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, nullptr);
+    else if (which == 6 && RG.count > 0) { reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, nullptr); sharedApply(w.p + C.nActiveVs, nullptr, 0.0, 1.0, 1.0, nullptr, nullptr); }
     else if (which == 5) k_cg_update(st, ownSys, x.p, r.p, p.p, Ap.p, dotPartial.p, scal.p, PeerCtx());   // rank-local (timing only)
     else k_pass2(st, A, w.p, b.p, Ap.p, 0.5, nullptr, dotPartial.p, PeerCtx(), scal.p, which == 4 ? 3 : 0, r.p);      // 4: with the three fused dot products of the CG loop
 }
@@ -1195,7 +1340,8 @@ int Solver::solve() {
                 else xchg(haloX, p.p);
             } else xchg(haloX, p.p);
             mark(tr, "halo p");
-            pass1Apply(A, p.p, scal.p, rev, l1);                mark(tr, "pass1 + regions");          // w = [dt Mc^-1 K p ; c_f . B^-1 J p]
+            pass1Apply(A, p.p, scal.p, rev, l1, false);         mark(tr, "pass1 + regions");          // w = [dt Mc^-1 K p ; c_f . B^-1 J p]
+            if (RG.nShared > 0) { sharedApply(w.p + C.nActiveVs, nullptr, 0.0, 1.0, 1.0, nullptr, scal.p); mark(tr, "shared regions"); }
             if (fused) { l2 = pushDirect(haloW, 1, nullptr); l2.wait[0] = myFlag(1, 0); l2.wait[1] = myFlag(1, 1); l2.waitSeq = peer.seqVec[1]; }
             else xchg(haloW, w.p);
             mark(tr, "halo w");
@@ -1375,6 +1521,7 @@ void Solver::recoverVelocityFromPressureStress() {
         reduced_finish(st, g, RG, RG.rhsR.p, g.invDt, -1.0, nullptr);                            // B^-1 (rhs_r/dt - J x)
         k_copy_reduced_solution(st, (int64_t)(RG.regHi - RG.regLo) * RDOF, RG.s.p + (size_t)RG.regLo * RDOF, velSol.p + C.nActiveVs + (size_t)RG.regLo * RDOF);
     }
+    sharedApply(w.p + C.nActiveVs, RG.rhsR.p, g.invDt, -1.0, 0.0, velSol.p + C.nActiveVs, nullptr);   // after the copy: it overwrites the shared regions
     checkPeer("the velocity recovery");
 }
 
@@ -1407,7 +1554,8 @@ void Solver::applySolutionToVelocity(const ps_fields_out& out) {
         if (out.valid[a] && !(validSent && !dev)) {
             if (dev) validDev = out.valid[a]; else { outStage[3 + a].alloc(nf); validDev = outStage[3 + a].p; }
         }
-        const FaceOwner own = {(int32_t)part.slotCut[SL_FACE + a][part.rank], (int32_t)part.slotCut[SL_FACE + a][part.rank + 1], RG.regLo, RG.regHi};
+        FaceOwner own = {(int32_t)part.slotCut[SL_FACE + a][part.rank], (int32_t)part.slotCut[SL_FACE + a][part.rank + 1], RG.regLo, RG.regHi};
+        if (RG.nShared > 0) { own.shared = RG.shFlag.p; own.zLo = g.zLo; own.zHi = g.zHi; own.nz = g.nz; }
         k_writeback_velocity(st, g, F, C, RG, velSol.p, a, velDev, validDev != nullptr, validDev, own, kLo, kHi, oLo, oHi);
         if (a == 2 && part.multi() && comm && velDev) {
             // the z-face plane on a slab cut carries DOFs of both neighbours (active: upper rank, reduced: lower rank's regions)
@@ -1463,7 +1611,9 @@ void Solver::setup() {
         classifyFaces();
         classifyEdges();
     }
-    RG.count = 0; RG.regLo = RG.regHi = 0; RG.cellChunkLo = RG.cellChunkHi = 0; RG.rowChunkLo = RG.rowChunkHi = 0;
+    RG.count = 0; RG.regLo = RG.regHi = 0; RG.cellChunkLo = RG.cellChunkHi = 0; RG.rowChunkLo = RG.rowChunkHi = 0; RG.bldLo = 0;
+    RG.nShared = RG.nShChunks = RG.nShMine = 0; RG.shRowLo = RG.shRowHi = 0;
+    sharedPeerExchanges = sharedCommExchanges = 0;
     part.regionCut.assign((size_t)part.nranks + 1, 0);
     {
         StageTimer T(st, &stageMs[PS_STAGE_REDUCED]);

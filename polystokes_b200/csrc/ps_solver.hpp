@@ -89,6 +89,18 @@ struct RegionData {
     int32_t ownRowLo = 0, ownRowHi = 0;   // coupled reduced rows of the owned regions
     // owned pieces of this rank (everything on one GPU): regions [regLo, regHi) and their chunk ranges
     int32_t regLo = 0, regHi = 0, cellChunkLo = 0, cellChunkHi = 0, rowChunkLo = 0, rowChunkHi = 0;
+    int32_t bldLo = 0;       // region matrices are built for [bldLo, regHi): the owned regions, the shared ones this rank takes part in, and
+                             // (one contiguous range) every region of lower ranks numbered between them
+    // Shared regions (ps_part.hpp, Partition::spanning): reduced faces in more than one slab.  Their coupled rows follow the slab of
+    // the face and sit after the rank's other coupled rows, [shRowLo, shRowHi); every apply sums their 3 x 10 moments over the ranks.
+    int32_t nShared = 0;                 // global count (the same on every rank)
+    int32_t nShChunks = 0, shRowLo = 0, shRowHi = 0, nShMine = 0;
+    DBuf<int32_t> shRegion;              // [nShared] region id of every shared slot, ascending
+    DBuf<int32_t> shChunk;               // [nShChunks][4] = region, begin, end, axis: this rank's rows of the shared regions
+    DBuf<int32_t> shChunkStart;          // [nShared+1] first chunk of every slot
+    DBuf<int32_t> shMine;                // [nShMine] slots this rank solves: it holds rows or reduced faces of the region, or owns it
+    DBuf<uint8_t> shFlag;                // [R] 1 for a shared region (velocity write-back: faces are written by the slab that holds them)
+    DBuf<double> shPartial, shMoments;   // per-chunk moments; [nShared][30] moments summed over the ranks
 };
 
 // halo of one distributed vector: entries this rank must send to / receive from its z-neighbours
@@ -191,6 +203,7 @@ public:
 
     // ---- multi-GPU (one process per GPU; ps_part.hpp) ----
     Partition part;
+    DBuf<int32_t> zCutDev;              // part.zCut on the device (Partition::spanning: slab of a face)
     Comm* comm = nullptr;
     void initComm(Comm* c);             // takes ownership; computes the z cuts
     void computePartition(int rank, int nranks);
@@ -239,7 +252,12 @@ public:
 
     // operator y = A x on device vectors (Apply.h:102-179)
     void applyOperator(const double* x, double* y, double* pApPartial);
-    void pass1Apply(const OpArgs& A, const double* x, const PcgScalars* S, bool reverse = false, const VecLink& V = VecLink());   // pass 1 + the reduced term
+    void pass1Apply(const OpArgs& A, const double* x, const PcgScalars* S, bool reverse = false, const VecLink& V = VecLink(), bool withShared = true);   // pass 1 + the reduced term
+    // the reduced term of the shared regions: s_r = B_r^-1 (extraScale extra_r + tScale t_r), t_r summed over the ranks (collective
+    // when tScale != 0), then w_f = scale c_f . s_r on this rank's shared rows (scale 0: no expansion); sOut (region-indexed) receives s_r
+    void sharedApply(double* wRows, const double* extra, double extraScale, double tScale, double scale, double* sOut, const PcgScalars* S);
+    void classifySharedRegions();
+    int64_t sharedPeerExchanges = 0, sharedCommExchanges = 0;      // moment sums of shared regions since the last setup, by transport      // Partition::spanning: region owners, shared list, build range (replicated classification, no communication)
     void timedOperator(int which);     // 0 = whole apply, 1 = pass 1 only, 2 = pass 2 only (on b -> Ap)
 
     // ---- device state ----
@@ -351,6 +369,17 @@ void reduced_expand(cudaStream_t, const Geom&, const RegionData&, double* wRows,
 // the reduced term of one apply: w_f <- scale * c_f . B^-1 (sum_f c_f w_f); one fused launch for tiled regions, moments + expand otherwise
 void reduced_apply(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
 int region_path(const OpArgs&, const RegionData&);      // the kernels reduced_apply / pass1Apply choose (ps_pcg.cu)
+// shared regions (RegionData::nShared): moments of this rank's shared rows per chunk, their sum per slot in chunk order (shMoments,
+// then summed over the ranks by the caller), the small solve of the slots this rank takes part in, the expansion onto its shared rows
+void shared_moments(cudaStream_t, const Geom&, const RegionData&, const double* wRows, const PcgScalars* scal);
+void shared_pack(cudaStream_t, const RegionData&);
+void shared_finish(cudaStream_t, const RegionData&, const double* extra, double extraScale, double tScale, double* sOut, const PcgScalars* scal);
+void shared_expand(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
+#ifndef PS_EMULATE
+// peer transport: push this rank's packed moments into every rank's moment area, then wait, sum in rank order and solve (ps_pcg.cu)
+void shared_exchange_peer(cudaStream_t, const RegionData&, const SharedPeer& P, const double* extra, double extraScale, double tScale, double* sOut,
+                          const PcgScalars* scal, PcgScalars* err);
+#endif
 void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, bool reverse = false, const VecLink& V = VecLink());
 void k_cg_init(cudaStream_t, const RangeSet& own, const double* b, double* x, double* r, double* p, double* dotPartial, PcgScalars* scal, double tol, int maxIter, const PeerCtx& P);
 void k_cg_begin(cudaStream_t, PcgScalars* scal, const PeerCtx& P);
@@ -385,8 +414,10 @@ void k_halo_unpack_peer(cudaStream_t, int64_t n0, int64_t n1, const int32_t* idx
                         unsigned long long seq, double* v, PcgScalars* S, bool respectDone);
 #endif
 void k_recover_active(cudaStream_t, const Geom&, const RowSet& rows, const double* wAct, const double* mcInv, const double* rhsU, double* velSol);
-// faces this rank writes: active faces with index in [aLo, aHi), reduced faces of regions [regLo, regHi), every face without a DOF
-struct FaceOwner { int32_t aLo, aHi, regLo, regHi; };
+// faces this rank writes: active faces with index in [aLo, aHi), reduced faces of regions [regLo, regHi), every face without a DOF;
+// with `shared` (Partition::spanning) a reduced face of a shared region is written by the slab that holds it: z in [zLo, zHi)
+// (the last slab also takes the top plane)
+struct FaceOwner { int32_t aLo, aHi, regLo, regHi; const uint8_t* shared = nullptr; int32_t zLo = 0, zHi = 0, nz = 0; };
 void k_writeback_velocity(cudaStream_t, const Geom&, const Fields&, const Counts&, const RegionData&, const double* velSol, int axis, float* velOut, bool writeValid, float* validOut, FaceOwner own,
                           int64_t lo, int64_t hi, int64_t validLo, int64_t validHi);
 void k_merge_face_plane(cudaStream_t, const Geom&, const Fields&, int axis, int k, const float* peerPlane, float* velOut, FaceOwner own);
