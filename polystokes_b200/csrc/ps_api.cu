@@ -523,6 +523,7 @@ int64_t ps_get_count(ps_handle h, const char* name) {
     if (n == "sharedRegions") return S.RG.nShared;
     if (n == "sharedPeerExchanges") return S.sharedPeerExchanges;      // moment sums of shared regions since the last setup, peer transport
     if (n == "sharedCommExchanges") return S.sharedCommExchanges;      // ... and by the communicator's all-reduce
+    if (n == "peerSharedCap") return PEER_SH_CAP;      // shared regions the peer moment area holds; a step with more takes the communicator
     if (n == "directHalo") return S.fusedHalo ? 1 : 0;      // boundary entries stored straight into the neighbours' vectors (ps_peer.hpp, VecLink)
     if (n == "result") return S.result; if (n == "usedBiCGStab") return S.usedBiCGStab;
     if (n == "nRowsExt") return C.nRowsExt; if (n == "fixLoops") return S.fixLoops;

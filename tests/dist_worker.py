@@ -59,6 +59,48 @@ def attach_gloo(solver):
     assert rc == 1, solver.last_error()
 
 
+REGION_VECTORS = ("b", "reducedRHS", "BinvDense", "MrDense", "ViscDense", "bestFit")
+
+
+def applies_before_step(s, out, outdir):
+    """apply(x1), apply(x2), apply(x1) again after one apply, then after two (parity.apply_inputs), then the single-region inputs of
+    <outdir>/probes.npz if the parent wrote one (parity.write_region_probes).  Returns what applies_after_step needs."""
+    import parity
+    n = s.count("nSystemSize")
+    if n == 0:
+        out.update(apply=np.zeros(0), apply_x2=np.zeros(0))
+        return None
+    x1, x2 = parity.apply_inputs(n)
+    out["apply"] = s.apply(x1)
+    out["apply_x2"] = s.apply(x2)
+    again = [s.apply(x1)]
+    again += [s.apply(x2), s.apply(x2)]
+    again.append(s.apply(x1))
+    path = os.path.join(outdir, "probes.npz")
+    if os.path.exists(path):
+        P = np.load(path)
+        for i in range(len(P["regions"])):
+            x = np.zeros(n)
+            x[P[f"cols{i}"]] = P[f"vals{i}"]
+            y = s.apply(x)
+            rows = P[f"rows{i}"]
+            out[f"probe{i}"] = y[rows]
+            y[rows] = 0.0
+            out[f"probe{i}_outside"] = np.count_nonzero(y)
+    return x1, again
+
+
+def applies_after_step(s, out, state):
+    """apply(x1) once more after the step; every apply(x1) and apply(x2) of this rank must be bit-identical to its first."""
+    if state is None:
+        out["apply_stable"] = True
+        return
+    x1, again = state
+    y1, y2 = out["apply"], out["apply_x2"]
+    out["apply_stable"] = bool(np.array_equal(again[0], y1) and np.array_equal(again[1], y2) and np.array_equal(again[2], y2)
+                               and np.array_equal(again[3], y1) and np.array_equal(s.apply(x1), y1))
+
+
 def main():
     case, outdir = sys.argv[1], sys.argv[2]
     gpu = len(sys.argv) > 3 and sys.argv[3] == "gpu"
@@ -84,11 +126,9 @@ def main():
         out[f"labels{slot}"] = s.index_field(0, slot)
         out[f"active{slot}"] = s.index_field(1, slot)
         out[f"reduced{slot}"] = s.index_field(2, slot)
-    for v in ("b", "reducedRHS", "BinvDense", "MrDense"):
+    for v in REGION_VECTORS:
         out["vec_" + v] = s.vector(v)
-    nsys = s.count("nSystemSize")
-    x = np.random.default_rng(0).standard_normal(nsys)
-    out["apply"] = s.apply(x) if nsys else np.zeros(0)
+    state = applies_before_step(s, out, outdir)
     rc, vel, valid = s.step_scene(sc)
     out["rc"] = rc
     out["iterations"] = s.count("iterations")
@@ -96,6 +136,7 @@ def main():
     for a in range(3):
         out[f"vel{a}"] = vel[a]
         out[f"valid{a}"] = valid[a]
+    applies_after_step(s, out, state)
     # a second step on the same handle must reproduce the first bit for bit
     rc2, vel2, _ = s.step_scene(sc)
     out["repeat_ok"] = bool(rc2 == rc and all(np.array_equal(vel[a], vel2[a]) for a in range(3)))

@@ -145,6 +145,11 @@ def check_region_blocks(o, s):
     return err
 
 
+# Componentwise gate of an apply against the factored scipy evaluation, in units of the factored bound.  Measured on the emulation
+# twin: <= 2.0e-15 (the one-region scene), 5e-16 on the tiled ones; an error of one lost row is O(1).
+OPERATOR_GATE = 1e-13
+
+
 def operator_error(y, Ax, bound):
     """Componentwise error of an apply: max |y_i - (Ax)_i| / (|A||x|)_i, where a row with bound 0 must be exactly 0."""
     return float(_ratio(np.abs(y - Ax), bound).max()) if y.size else 0.0
@@ -345,10 +350,61 @@ def run_case(name, lib_path=None, solve=True):
     return o
 
 
+_DIST_REF = {}
+
+
+def dist_reference(case):
+    """The oracle set up on a distributed case and its factored scipy apply (the last case asked for is kept, so that the probes written
+    before a run and the comparison after it share one setup)."""
+    if case not in _DIST_REF:
+        _DIST_REF.clear()
+        sc, ov = DIST_CASES[case]()
+        o = Oracle(sc, **ov).setup()
+        _DIST_REF[case] = dict(sc=sc, ov=ov, o=o, apply=scipy_factored(o.csr, sc.dt), probes=None)
+    return _DIST_REF[case]
+
+
+def apply_inputs(n):
+    """x1, x2 of the applies of the distributed workers (tests/dist_worker.py)."""
+    return np.random.default_rng(0).standard_normal(n), np.random.default_rng(1).standard_normal(n)
+
+
+PROBE_REGIONS = 8
+
+
+def write_region_probes(case, outdir):
+    """Inputs that isolate single regions: x_r is non-zero only on the DOFs region r couples (the columns of its rows of J), for up to
+    PROBE_REGIONS regions spread over the id range (every region of a small scene).  With a random x over many regions, an error in one
+    region's sum hides behind the rounding scale of a looser row; A x_r is checked componentwise on its own.  Written to
+    <outdir>/probes.npz with the rows where the factored bound of A x_r is non-zero; the workers apply each input and report those rows
+    (and how many entries elsewhere are non-zero)."""
+    import scipy.sparse as sp
+    ref = dist_reference(case)
+    o = ref["o"]
+    R, n = o.count("regionCount"), o.count("nSystemSize")
+    if R == 0:
+        return
+    J = sp.hstack([o.scipy_csr("JG"), o.scipy_csr("JDt")]).tocsr()
+    regions = np.unique(np.linspace(0, R - 1, min(R, PROBE_REGIONS)).round().astype(np.int64))
+    rng = np.random.default_rng(2)
+    out, probes = {"regions": regions}, []
+    for i, r in enumerate(regions):
+        cols = np.unique(J[26 * r:26 * (r + 1)].indices)
+        x = np.zeros(n)
+        x[cols] = rng.standard_normal(cols.size)
+        Ax, bound = ref["apply"](x)
+        rows = np.nonzero(bound)[0]
+        probes.append((int(r), Ax[rows], bound[rows]))
+        out.update({f"cols{i}": cols, f"vals{i}": x[cols], f"rows{i}": rows})
+    ref["probes"] = probes
+    np.savez(os.path.join(str(outdir), "probes.npz"), **out)
+
+
 def check_distributed(case, ranks):
     """`ranks`: per-rank result dicts written by tests/dist_worker.py (or the GPU twin); merged and compared with the oracle."""
-    sc, ov = DIST_CASES[case]()
-    o = Oracle(sc, **ov).setup()
+    ref = dist_reference(case)
+    _DIST_REF.pop(case)           # the solve below changes the oracle's state
+    sc, ov, o = ref["sc"], ref["ov"], ref["o"]
     world = len(ranks)
     cuts = list(ranks[0]["cuts"])
     assert cuts[0] == 0 and cuts[-1] == sc.nz and all(b > a and a % 16 == 0 for a, b in zip(cuts[:-1], cuts[1:]))
@@ -367,12 +423,32 @@ def check_distributed(case, ranks):
     # every global vector is the sum of the ranks' shares
     tot = lambda key: sum(r[key] for r in ranks)
     assert rel(o.vector("b"), tot("vec_b")) <= 1e-10, f"b rel {rel(o.vector('b'), tot('vec_b')):.2e}"
-    for v in ("reducedRHS", "BinvDense", "MrDense"):
-        assert rel(o.vector(v), tot("vec_" + v)) <= 1e-8, f"{v} rel {rel(o.vector(v), tot('vec_' + v)):.2e}"
+    assert rel(o.vector("reducedRHS"), tot("vec_reducedRHS")) <= 1e-8, f"reducedRHS rel {rel(o.vector('reducedRHS'), tot('vec_reducedRHS')):.2e}"
+    # the region blocks, region by region and entry by entry (each region is reported by its owner only)
+    R = o.count("regionCount")
+    blk = region_block_errors(o.vector, lambda v: tot("vec_" + v), R)
+    for v, gate in REGION_GATES.items():
+        assert blk[v] <= gate, f"{v}: worst per-region error {blk[v]:.2e} > {gate:.0e} on {world} ranks"
+    # the operator, componentwise against the factored scipy evaluation; and bit for bit the same apply(x1) on every rank after other
+    # applies (an odd and an even number of them, so either parity of the peer moment area) and after the step
     n = o.count("nSystemSize")
+    op = probe = 0.0
     if n:
-        x = np.random.default_rng(0).standard_normal(n)
-        assert rel(o.apply(x), tot("apply")) <= 1e-12, f"apply rel {rel(o.apply(x), tot('apply')):.2e}"
+        for key, x in zip(("apply", "apply_x2"), apply_inputs(n)):
+            Ax, bound = ref["apply"](x)
+            e = operator_error(tot(key), Ax, bound)
+            assert e <= OPERATOR_GATE, f"{key}: componentwise error {e:.2e} > {OPERATOR_GATE:.0e} on {world} ranks"
+            op = max(op, e)
+        for r in ranks:
+            assert bool(r["apply_stable"]), f"rank {int(r['rank'])}: apply(x1) is not bit-identical after other applies and after the step"
+    if ref["probes"] is not None:
+        for i, (region, Ax, bound) in enumerate(ref["probes"]):
+            assert int(tot(f"probe{i}_outside")) == 0, f"A x of region {region}'s DOFs is non-zero where the factored bound is 0"
+            e = operator_error(tot(f"probe{i}"), Ax, bound)
+            assert e <= OPERATOR_GATE, f"A x of region {region}'s DOFs: componentwise error {e:.2e} > {OPERATOR_GATE:.0e} on {world} ranks"
+            probe = max(probe, e)
+    print(f"{case} on {world} ranks: {R} regions, componentwise apply error {op:.1e}, single-region inputs {probe:.1e}; worst per-region "
+          + ", ".join(f"{v} {blk[v]:.1e}" for v in REGION_GATES), flush=True)
     ro = o.solve()
     ovel, ovalid = o.writeback()
     its = [int(r["iterations"]) for r in ranks]

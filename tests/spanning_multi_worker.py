@@ -10,7 +10,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import multi_worker  # noqa: E402
 import spanning_cases  # noqa: E402
 
-for name in ("span_blob64_notile", "span_blob64_tile8_pad0", "span_s3_128_notile"):
+for name in ("span_blob64_notile", "span_blob64_tile8_pad0", "span_s3_128_notile", "span_bodies_notile"):
     multi_worker.CASES[name] = (lambda n: lambda: spanning_cases.CASES[n]()[0])(name)
 
 if __name__ == "__main__":

@@ -1,6 +1,7 @@
 """Worker of tests/test_distributed_spanning_emul.py and tests/test_gpu_spanning_regions.py: one rank of a slab-decomposed
 step on a scene whose reduced regions cross the cuts (tests/spanning_cases.py).  Writes <outdir>/rank<k>.npz with what
-tests/dist_worker.py writes (parity.check_distributed merges it) plus the shared-region count.  For a SWITCH case the handle
+tests/dist_worker.py writes (parity.check_distributed merges it) plus the shared-region count, how the shared moments were summed
+and which kernels carried the reduced term (regionPath).  For a SWITCH case the handle
 first steps the scene with other tiling parameters, then ps_set_params switches it to the case's own.
 Usage: python spanning_worker.py <case> <outdir> [gpu]   (RANK / WORLD_SIZE / MASTER_* in the env)
 """
@@ -17,7 +18,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import parity  # noqa: E402
 import spanning_cases  # noqa: E402
-from dist_worker import attach_gloo  # noqa: E402
+from dist_worker import REGION_VECTORS, applies_after_step, applies_before_step, attach_gloo  # noqa: E402
 
 
 def set_params(s, **kw):
@@ -55,17 +56,15 @@ def main():
     s.setup_scene(sc)
     out.update(rank=rank, nranks=n, zlo=zlo, zhi=zhi, cuts=np.array(cuts), peer=s.count("peerTransport") if gpu else 0, local=s.count("slabLocal"),
                shared=s.count("sharedRegions"))
-    for k in parity.COUNTS:
+    for k in parity.COUNTS + ["maxRegionRows", "regionPath", "peerSharedCap"]:
         out["count_" + k] = s.count(k)
     for slot in range(7):
         out[f"labels{slot}"] = s.index_field(0, slot)
         out[f"active{slot}"] = s.index_field(1, slot)
         out[f"reduced{slot}"] = s.index_field(2, slot)
-    for v in ("b", "reducedRHS", "BinvDense", "MrDense"):
+    for v in REGION_VECTORS:
         out["vec_" + v] = s.vector(v)
-    nsys = s.count("nSystemSize")
-    x = np.random.default_rng(0).standard_normal(nsys)
-    out["apply"] = s.apply(x) if nsys else np.zeros(0)
+    state = applies_before_step(s, out, outdir)
     rc, vel, valid = s.step_scene(sc)
     out["rc"] = rc
     out["peerExchanges"] = s.count("sharedPeerExchanges")      # how the shared-region moments of this step were summed
@@ -77,6 +76,7 @@ def main():
     for a in range(3):
         out[f"vel{a}"] = vel[a]
         out[f"valid{a}"] = valid[a]
+    applies_after_step(s, out, state)
     rc2, vel2, _ = s.step_scene(sc)
     out["repeat_ok"] = bool(rc2 == rc and all(np.array_equal(vel[a], vel2[a]) for a in range(3)))
     if first:

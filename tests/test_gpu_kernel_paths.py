@@ -76,9 +76,7 @@ BIT_IDENTICAL_SOLVE = [("default", "lpt"), ("default", "pdl0")]
 # A solve that is wrong in earnest shows up in x (gated at 10 x tol) and in the stop rule recomputed with the oracle's apply.
 VEL_GATE = {"blob64_tile32": 0.1, "blob64_notile": 0.1, "box96_tile8": 0.1}
 
-# Componentwise gate of an apply against the factored scipy evaluation, in units of the factored bound.  Measured on the emulation
-# twin: <= 2.0e-15 (the one-region scene), 5e-16 on the tiled ones; an error of one lost row is O(1).
-OPERATOR_GATE = 1e-13
+OPERATOR_GATE = parity.OPERATOR_GATE
 
 _results = {}
 _refs = {}
