@@ -122,7 +122,10 @@ int ps_solve(ps_handle h, ps_fields_out* out, ps_stats* stats);
 /* exportMatrices / exportComponentMatrices / exportStats (S.cpp:533-606): MatrixMarket files written with
  * Eigen's saveMarket format.  `what` is a bit mask: 1 = Mat_A + Vec_b + Vec_guess + solutionVector (Mat_A is the explicit
  * matrix with solverType 1 and the empty nSystemSize x nSystemSize matrix of the factored path otherwise, as in the
- * reference), 2 = component matrices, 4 = stats. */
+ * reference), 2 = component matrices, 4 = stats.  On a decomposed handle (one process per GPU, or ps_create_multi) ps_export is a
+ * collective call: every rank calls it, rank 0 writes the whole file set under ITS prefix (the files of one GPU; dimData's "thread
+ * count" is the SMs of all ranks, the solveData times are the slowest rank's) and the other ranks write nothing; every rank returns the
+ * same code (PS_FAILED, naming the prefix, when a write failed).  ps_step's export through the ps_params toggles does the same. */
 int ps_export(ps_handle h, const char* prefix, int what);
 /* thread-local description of the last PS_FAILED / PS_INVALID */
 const char* ps_last_error(void);
@@ -148,7 +151,9 @@ const char* ps_last_error(void);
  * 0..ndev-1), one host thread per rank, NCCL + NVLink peer memory between them.  The handle is used exactly like a single-GPU
  * one: ps_step / ps_setup / ps_solve take the full-grid HOST fields of the caller, every rank uploads only its slab (+ halo) and
  * writes only its slab of velocity / valid, so after the call the caller's arrays are complete.  ps_get_count / ps_get_real /
- * ps_get_partition answer for the whole job; ps_export / ps_apply and the per-voxel introspection need a single-GPU handle. */
+ * ps_get_partition answer for the whole job; ps_export writes the file set of one GPU, and ps_get_vector / ps_get_csr / ps_apply
+ * return the global vectors, matrices and A x, assembled from the ranks that own them.  The per-voxel introspection, diagA and the
+ * explicit A need a single-GPU handle. */
 int ps_create_multi(const ps_params* params, int ndev, const int* devs, ps_handle* out);
 int ps_comm_unique_id(void* id128);
 int ps_comm_init(ps_handle h, int rank, int nranks, const void* id128);
@@ -171,8 +176,9 @@ int64_t ps_get_weight_field(ps_handle h, int liquid, int slot, float* out);
  * blocks are dense, so it only fits for small / medium grids -- PS_FAILED beyond 2^31-1 entries or device memory). */
 int ps_get_csr(ps_handle h, const char* name, int64_t* rows, int64_t* cols, int64_t* nnz, int64_t* rowptr, int32_t* colidx, double* vals);
 /* dense vectors by name (activeRHS reducedRHS pressureRHS stressRHS b guess diagA solution velSolution com bestFit
- * MrDense ViscDense BinvDense); returns the length.  diagA = diag(A) formed from the factors (one GPU).  With several ranks b / solution / region data are zero
- * outside the calling rank's share, so the sum over ranks is the global vector. */
+ * MrDense ViscDense BinvDense); returns the length.  diagA = diag(A) formed from the factors (one GPU).  On a rank of a job with one
+ * process per GPU, b / solution / guess / region data are zero outside the calling rank's share, so the sum over ranks is the global
+ * vector; a ps_create_multi handle returns the global vector. */
 int64_t ps_get_vector(ps_handle h, const char* name, double* out);
 /* y = A x with host vectors of length nSystemSize (ApplyPressureStressMatrix::apply, Apply.h:182-184) */
 int ps_apply(ps_handle h, const double* x, double* y);

@@ -174,34 +174,150 @@ HostCsr blockdiag_csr(const std::vector<double>& blocks, int R) {
     return m;
 }
 
-// G / D^T (active rows) and JG / JD^T (26 rows per region) rebuilt from the device ELL of K_ext
-// with the reference's CSR conventions (sorted columns, duplicates summed in traversal order,
-// explicit zeros kept: S_CMB:454-455, 524-525, 612-613; SURVEY.md section 8c)
-HostCsr k_block(Solver& S, const std::string& name) {
-    const Counts& C = S.C;
-    const int64_t nRows = C.nRowsExt, nP = C.nPressures, nT = C.nStresses;
-    // expand the compact operator (CompactOp, ps_solver.hpp) into 8 (value, column) slots per row
-    std::vector<double> kv((size_t)8 * nRows); std::vector<int32_t> kc((size_t)8 * nRows);
-    {
-        std::vector<uint64_t> code = S.Op.kcode.to_host(S.st, (size_t)nRows);
-        std::vector<int32_t> col = S.Op.kcol.to_host(S.st, (size_t)6 * nRows);
-        const double sc = S.g.invDx / 64.;
-        for (int64_t r = 0; r < nRows; ++r) {
-            const int32_t c0w = col[r];
-            const int64_t cOff = nP + (int64_t)((uint32_t)c0w >> 30) * C.nCenter;
-            const int64_t c0 = c0w & OP_COL_MASK, c1 = col[(size_t)nRows + r];
-            const int64_t cc[8] = {c0, c1, cOff + c0, cOff + c1, col[(size_t)2 * nRows + r], col[(size_t)3 * nRows + r], col[(size_t)4 * nRows + r], col[(size_t)5 * nRows + r]};
-            for (int k = 0; k < 8; ++k) { kv[(size_t)k * nRows + r] = (double)op_code(code[r], k) * sc; kc[(size_t)k * nRows + r] = (int32_t)cc[k]; }
-        }
+// ---- several ranks: the global objects, assembled on rank 0 from the pieces their owners hold ----
+// Every entry is copied from the one rank that owns it, never summed over the ranks: a sum would turn an owner's -0.0 into +0.0,
+// and the exported files print the two differently.
+
+// index ranges [lo, hi) of a table that one rank owns, ascending
+typedef std::vector<std::pair<int64_t, int64_t>> Spans;
+template <int N>
+Spans spans_in(const RangeSetN<N>& s, int64_t lo, int64_t hi) {      // the ranges of s inside [lo, hi), relative to lo
+    Spans o;
+    for (int i = 0; i < s.n; ++i) { const int64_t a = std::max(s.lo[i], lo), b = std::min(s.lo[i] + s.count(i), hi); if (b > a) o.push_back({a - lo, b - lo}); }
+    return o;
+}
+Spans region_spans(const Solver& S, int64_t per, int64_t off = 0) { return {{off + S.RG.regLo * per, off + S.RG.regHi * per}}; }
+
+template <class T> void put(std::vector<uint8_t>& b, const T* p, size_t n) { const size_t o = b.size(); b.resize(o + n * sizeof(T)); if (n) memcpy(b.data() + o, p, n * sizeof(T)); }
+template <class T> const uint8_t* take(const uint8_t* q, T* p, size_t n) { if (n) memcpy(p, q, n * sizeof(T)); return q + n * sizeof(T); }
+
+// Collective: rank 0 receives every rank's bytes in rank order, the other ranks an empty list.  The sizes travel in one all-reduce
+// (Solver::hostAllgather), the payload in one grouped send / receive towards rank 0 through a staging buffer of the solver's device.
+std::vector<std::vector<uint8_t>> gather_bytes(Solver& S, const std::vector<uint8_t>& mine) {
+    PS_WHERE("export / view: gather");
+    const int N = S.part.nranks;
+    const std::vector<double> sz = S.hostAllgather({(double)mine.size()});
+    DBuf<uint8_t>& buf = scratch().gather;
+    std::vector<std::vector<uint8_t>> all;
+    if (S.part.rank == 0) {
+        std::vector<size_t> off((size_t)N + 1, 0);
+        for (int k = 0; k < N; ++k) off[k + 1] = off[k] + (k ? (size_t)std::llround(sz[k]) : 0);
+        buf.alloc(off[N] + 1);
+        std::vector<int> peers; std::vector<const void*> sb; std::vector<void*> rb; std::vector<size_t> sby, rby;
+        for (int k = 1; k < N; ++k) { peers.push_back(k); sb.push_back(nullptr); sby.push_back(0); rb.push_back(buf.p + off[k]); rby.push_back(off[k + 1] - off[k]); }
+        S.comm->sendrecv(N - 1, peers.data(), sb.data(), sby.data(), rb.data(), rby.data(), S.st);
+        all.resize((size_t)N);
+        all[0] = mine;
+        for (int k = 1; k < N; ++k) { all[k].resize(off[k + 1] - off[k]); copy_d2h(all[k].data(), buf.p + off[k], all[k].size(), S.st); }
+        stream_sync(S.st);
+    } else {
+        buf.alloc(mine.size() + 1);
+        copy_h2d(buf.p, mine.data(), mine.size(), S.st);
+        const int root = 0; const void* sb = buf.p; void* rb = nullptr; const size_t sby = mine.size(), rby = 0;
+        S.comm->sendrecv(1, &root, &sb, &sby, &rb, &rby, S.st);
+        stream_sync(S.st);      // the staging buffer is reused by the next gather
     }
+    return all;
+}
+
+// Collective: a table of n items of `stride` values on rank 0, every item copied from the rank that owns it (`own`: the items of
+// this rank's copy `local` that it owns); the other ranks get an empty table
+template <class T>
+std::vector<T> gather_owned(Solver& S, const std::vector<T>& local, const Spans& own, int64_t n, int stride = 1) {
+    std::vector<uint8_t> mine;
+    const int64_t ns = (int64_t)own.size();
+    put(mine, &ns, 1);
+    for (const auto& s : own) { put(mine, &s.first, 1); put(mine, &s.second, 1); put(mine, local.data() + s.first * stride, (size_t)(s.second - s.first) * stride); }
+    const std::vector<std::vector<uint8_t>> all = gather_bytes(S, mine);
+    std::vector<T> out;
+    if (S.part.rank != 0) return out;
+    out.assign((size_t)n * stride, T());
+    for (const auto& piece : all) {
+        const uint8_t* q = piece.data();
+        int64_t m; q = take(q, &m, 1);
+        for (int64_t i = 0; i < m; ++i) { int64_t a, b; q = take(q, &a, 1); q = take(q, &b, 1); q = take(q, out.data() + a * stride, (size_t)(b - a) * stride); }
+    }
+    return out;
+}
+
+// Rows of K_ext in the compact form of CompactOp (code word, then the 6 stored columns of each row): the active rows (G / D^T), or
+// the coupled reduced rows (JG / JD^T) with their packed faces, the rows of region r at [regStart[r], regStart[r+1]), and the
+// regions' centres of mass.  This rank's rows, or (`global`, several ranks, collective) every row from its owner, on rank 0.
+struct KRows { std::vector<uint64_t> code; std::vector<int32_t> col; std::vector<int32_t> face; std::vector<int64_t> regStart; std::vector<double> com; };
+
+KRows k_rows(Solver& S, bool reduced, bool global) {
+    const Counts& C = S.C;
+    const int R = S.RG.count;
+    const int64_t nRows = C.nRowsExt, lo = reduced ? C.nActiveVs : 0, n = reduced ? nRows - C.nActiveVs : C.nActiveVs;
+    KRows K;
+    const std::vector<uint64_t> code = S.Op.kcode.to_host(S.st, (size_t)nRows);
+    const std::vector<int32_t> col = S.Op.kcol.to_host(S.st, (size_t)6 * nRows);      // [6][nRows]
+    K.code.assign(code.begin() + lo, code.begin() + lo + n);
+    K.col.resize((size_t)6 * n);
+    for (int64_t i = 0; i < n; ++i) for (int k = 0; k < 6; ++k) K.col[(size_t)6 * i + k] = col[(size_t)k * nRows + lo + i];
+    if (reduced && R > 0) {
+        K.face = S.RG.rowFace.to_host(S.st, (size_t)n);
+        K.com = S.RG.com.to_host(S.st, (size_t)3 * R);
+        const std::vector<int32_t> start = S.RG.rowStart.to_host(S.st, (size_t)R + 1);
+        K.regStart.assign(start.begin(), start.end());
+    }
+    if (!global || !S.part.multi()) return K;
+    const Spans own = spans_in(S.ownK, lo, lo + n);
+    K.code = gather_owned(S, K.code, own, n);
+    K.col = gather_owned(S, K.col, own, n, 6);
+    if (!reduced || R == 0) return K;
+    std::vector<int32_t> region = S.RG.rowRegion.to_host(S.st, (size_t)n);
+    region = gather_owned(S, region, own, n);
+    K.face = gather_owned(S, K.face, own, n);
+    K.com = gather_owned(S, K.com, region_spans(S, 3), (int64_t)3 * R);
+    if (S.part.rank != 0) return K;
+    // The rows come in the ranks' order: by region, face axis and voxel order within each rank.  A shared region (ps_part.hpp) has rows
+    // on several ranks; the cuts are whole tile layers and the tiles are numbered z-slowest, so its rows of one axis are in voxel
+    // order when taken rank after rank.  A stable sort by (region, axis) thus restores the row order of one GPU, and the duplicate
+    // columns of k_block are summed in the same order.
+    std::vector<int64_t> ord((size_t)n);
+    for (int64_t i = 0; i < n; ++i) ord[i] = i;
+    auto key = [&](int64_t i) { return (int64_t)region[i] * 4 + ((K.face[i] >> 29) & 3); };
+    std::stable_sort(ord.begin(), ord.end(), [&](int64_t a, int64_t b) { return key(a) < key(b); });
+    KRows G;
+    G.code.resize((size_t)n); G.col.resize((size_t)6 * n); G.face.resize((size_t)n); G.com = std::move(K.com);
+    G.regStart.assign((size_t)R + 1, 0);
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t j = ord[i];
+        G.code[i] = K.code[j]; G.face[i] = K.face[j];
+        std::copy(K.col.begin() + 6 * j, K.col.begin() + 6 * j + 6, G.col.begin() + 6 * i);
+        ++G.regStart[region[j] + 1];
+    }
+    for (int r = 0; r < R; ++r) G.regStart[r + 1] += G.regStart[r];
+    return G;
+}
+
+// G / D^T (active rows) and JG / JD^T (26 rows per region) rebuilt from the compact rows of K_ext with the reference's CSR
+// conventions (sorted columns, duplicates summed in traversal order, explicit zeros kept: S_CMB:454-455, 524-525, 612-613;
+// SURVEY.md section 8c)
+HostCsr k_block(const Solver& S, const KRows& K, const std::string& name) {
+    const Counts& C = S.C;
+    const int64_t nP = C.nPressures, nT = C.nStresses;
+    const double sc = S.g.invDx / 64.;
+    // the 8 (value, column) slots of row i: the compact form expanded as the operator kernels read it
+    auto slots = [&](size_t i, double* v, int32_t* c) {
+        const int32_t* col = K.col.data() + 6 * i;
+        const int32_t c0w = col[0];
+        const int64_t cOff = nP + (int64_t)((uint32_t)c0w >> 30) * C.nCenter;
+        const int64_t c0 = c0w & OP_COL_MASK, c1 = col[1];
+        const int64_t cc[8] = {c0, c1, cOff + c0, cOff + c1, col[2], col[3], col[4], col[5]};
+        for (int k = 0; k < 8; ++k) { v[k] = (double)op_code(K.code[i], k) * sc; c[k] = (int32_t)cc[k]; }
+    };
     const bool pressure = (name == "G" || name == "JG");
     const int64_t colLo = pressure ? 0 : nP, colHi = pressure ? nP : nP + nT;
     HostCsr m; m.cols = colHi - colLo;
+    double v[8]; int32_t c[8];
     if (name == "G" || name == "Dt") {
         m.rows = C.nActiveVs; m.ptr.assign(m.rows + 1, 0);
         for (int64_t r = 0; r < m.rows; ++r) {
             std::vector<std::pair<int32_t, double>> e;
-            for (int k = 0; k < 8; ++k) { const double v = kv[(size_t)k * nRows + r]; const int32_t c = kc[(size_t)k * nRows + r]; if (v != 0. && c >= colLo && c < colHi) e.push_back({(int32_t)(c - colLo), v}); }
+            slots((size_t)r, v, c);
+            for (int k = 0; k < 8; ++k) if (v[k] != 0. && c[k] >= colLo && c[k] < colHi) e.push_back({(int32_t)(c[k] - colLo), v[k]});
             std::sort(e.begin(), e.end(), [](auto& a, auto& b) { return a.first < b.first; });
             for (auto& x : e) { m.idx.push_back(x.first); m.val.push_back(x.second); }
             m.ptr[r + 1] = (int64_t)m.idx.size();
@@ -211,26 +327,22 @@ HostCsr k_block(Solver& S, const std::string& name) {
     const int R = S.RG.count;
     m.rows = (int64_t)R * RDOF; m.ptr.assign(m.rows + 1, 0);
     if (R == 0) return m;
-    std::vector<int32_t> rowFace = S.RG.rowFace.to_host(S.st, (size_t)S.RG.nRows);
-    std::vector<int32_t> rowStart = S.RG.rowStart.to_host(S.st, (size_t)R + 1);
-    std::vector<double> com = S.RG.com.to_host(S.st, (size_t)3 * R);
     for (int r = 0; r < R; ++r) {
         std::map<int32_t, std::array<double, RDOF>> cols;
-        for (int32_t row = rowStart[r]; row < rowStart[r + 1]; ++row) {
-            const int32_t packed = rowFace[row];
+        for (int64_t row = K.regStart[r]; row < K.regStart[r + 1]; ++row) {
+            const int32_t packed = K.face[row];
             const int axis = (packed >> 29) & 3;
             const I3 f = delin(S.g, SL_FACE + axis, (int64_t)(packed & 0x1fffffff));
             double p[3] = {(double)f.x, (double)f.y, (double)f.z};
             p[axis] -= 0.5;
-            double c[RDOF];
-            conversion_coefficients(p[0] * S.g.dx - com[3 * r], p[1] * S.g.dx - com[3 * r + 1], p[2] * S.g.dx - com[3 * r + 2], axis, c);
-            const int64_t kr = C.nActiveVs + row;
+            double cf[RDOF];
+            conversion_coefficients(p[0] * S.g.dx - K.com[3 * r], p[1] * S.g.dx - K.com[3 * r + 1], p[2] * S.g.dx - K.com[3 * r + 2], axis, cf);
+            slots((size_t)row, v, c);
             for (int k = 0; k < 8; ++k) {
-                const double v = kv[(size_t)k * nRows + kr]; const int32_t cc = kc[(size_t)k * nRows + kr];
-                if (v == 0. || cc < colLo || cc >= colHi) continue;
-                auto it = cols.find((int32_t)(cc - colLo));
-                if (it == cols.end()) { std::array<double, RDOF> a; for (int n = 0; n < RDOF; ++n) a[n] = v * c[n]; cols.emplace((int32_t)(cc - colLo), a); }
-                else for (int n = 0; n < RDOF; ++n) it->second[n] += v * c[n];
+                if (v[k] == 0. || c[k] < colLo || c[k] >= colHi) continue;
+                auto it = cols.find((int32_t)(c[k] - colLo));
+                if (it == cols.end()) { std::array<double, RDOF> a; for (int n = 0; n < RDOF; ++n) a[n] = v[k] * cf[n]; cols.emplace((int32_t)(c[k] - colLo), a); }
+                else for (int n = 0; n < RDOF; ++n) it->second[n] += v[k] * cf[n];
             }
         }
         for (int n = 0; n < RDOF; ++n) {
@@ -241,71 +353,99 @@ HostCsr k_block(Solver& S, const std::string& name) {
     return m;
 }
 
-bool get_matrix(Solver& S, const std::string& name, HostCsr& out) {
+// A vector as this rank holds it, and the entries of it this rank owns.  `share`: distributed data whose per-rank view keeps only the
+// owned entries (zero elsewhere, so the sum over the ranks is the global vector); the other vectors are returned as held.
+struct Piece { std::vector<double> v; Spans own; bool share = false; };
+
+bool vector_piece(Solver& S, const std::string& n, Piece& p) {
+    const Counts& C = S.C; const int R = S.RG.count; const size_t NN = (size_t)RDOF * RDOF;
+    const int64_t nA = C.nActiveVs, nP = C.nPressures, nSys = C.nSystemSize;
+    auto reg = [&](const DBuf<double>& d, size_t per, bool share) { p.v = R ? d.to_host(S.st, (size_t)R * per) : std::vector<double>(); p.own = region_spans(S, (int64_t)per); p.share = share; };
+    auto sys = [&](std::vector<double>&& v) { p.v = std::move(v); p.own = spans_in(S.ownSys, 0, nSys); p.share = true; };
+    if (n == "activeRHS") { p.v = S.rhsU.to_host(S.st, (size_t)nA); p.own = spans_in(S.ownK, 0, nA); }
+    else if (n == "oldActiveVs") { p.v = S.oldVs.to_host(S.st, (size_t)nA); p.own = spans_in(S.ownK, 0, nA); }
+    else if (n == "reducedRHS") reg(S.RG.rhsR, RDOF, true);
+    else if (n == "pressureRHS") { p.v = S.rhsPT.to_host(S.st, (size_t)nP); p.own = spans_in(S.ownSys, 0, nP); }
+    else if (n == "stressRHS") { auto v = S.rhsPT.to_host(S.st, (size_t)nSys); p.v.assign(v.begin() + nP, v.end()); p.own = spans_in(S.ownSys, nP, nSys); }
+    else if (n == "b") sys(S.b.to_host(S.st, (size_t)nSys));
+    else if (n == "solution") sys(S.x.to_host(S.st, (size_t)nSys));
+    else if (n == "guess") sys(S.haveGuess ? S.guess.to_host(S.st, (size_t)nSys) : std::vector<double>((size_t)nSys, 0.));
+    else if (n == "velSolution") {
+        p.v = S.velSol.to_host(S.st, (size_t)(nA + C.nReducedVs));
+        p.own = spans_in(S.ownK, 0, nA); p.own.push_back(region_spans(S, RDOF, nA)[0]); p.share = true;
+    }
+    else if (n == "com") reg(S.RG.com, 3, false);
+    else if (n == "bestFit") reg(S.RG.bestFit, RDOF, true);
+    else if (n == "MrDense") reg(S.RG.Mr, NN, true);
+    else if (n == "ViscDense") reg(S.RG.Visc, NN, true);
+    else if (n == "BinvDense") reg(S.RG.Binv, NN, true);
+    else return false;
+    return true;
+}
+// the vector as the caller sees it: this rank's view, or with `global` on a decomposed handle the whole vector on rank 0 (collective;
+// the other ranks get an empty vector)
+std::vector<double> view(Solver& S, Piece&& p, bool global) {
+    if (!S.part.multi()) return std::move(p.v);
+    if (global) return gather_owned(S, p.v, p.own, (int64_t)p.v.size());
+    if (!p.share) return std::move(p.v);
+    std::vector<double> m(p.v.size(), 0.);
+    for (const auto& s : p.own) std::copy(p.v.begin() + s.first, p.v.begin() + s.second, m.begin() + s.first);
+    return m;
+}
+
+bool get_vector(Solver& S, const std::string& n, std::vector<double>& out, bool global) {
+    if (n == "diagA") { if (S.part.multi()) return false; S.computeDiagonal(); out = S.diagA.to_host(S.st, (size_t)S.C.nSystemSize); return true; }
+    if (n == "guess" && global && S.part.multi()) S.constructGuessVectors();      // several ranks: formed where it is read (collective)
+    Piece p;
+    if (!vector_piece(S, n, p)) return false;
+    out = view(S, std::move(p), global);
+    return true;
+}
+
+bool is_matrix(const std::string& n) {
+    for (const char* m : {"G", "Dt", "JG", "JDt", "A", "Mc", "McInv", "uInv", "u", "Mr", "B", "BInv"}) if (n == m) return true;
+    return false;
+}
+// a matrix by name: this rank's view (on a rank of a decomposed handle the region blocks of its own regions only), or with `global`
+// the whole matrix on rank 0 (collective; the other ranks leave `out` empty).  The explicit A is built on one GPU only.
+void get_matrix(Solver& S, const std::string& name, HostCsr& out, bool global) {
     const Counts& C = S.C;
     const int R = S.RG.count;
-    if (name == "G" || name == "Dt" || name == "JG" || name == "JDt") { out = k_block(S, name); return true; }
+    const bool here = !global || !S.part.multi() || S.part.rank == 0;
+    if (name == "G" || name == "Dt" || name == "JG" || name == "JDt") {
+        const KRows K = k_rows(S, name == "JG" || name == "JDt", global);
+        if (here) out = k_block(S, K, name);
+        return;
+    }
     if (name == "A") {     // explicit system matrix, built on the device (ps_explicit.cu)
+        if (global && S.part.multi()) throw Error("the explicit A is built on one GPU");
         S.buildExplicitA();
         out.rows = out.cols = S.Aexp.n;
         out.ptr = S.Aexp.ptr.to_host(S.st, (size_t)S.Aexp.n + 1);
         out.idx = S.Aexp.nnz ? S.Aexp.idx.to_host(S.st, (size_t)S.Aexp.nnz) : std::vector<int32_t>();
         out.val = S.Aexp.nnz ? S.Aexp.val.to_host(S.st, (size_t)S.Aexp.nnz) : std::vector<double>();
-        return true;
+        return;
     }
-    if (name == "Mc") { out = diag_csr(S.mc.to_host(S.st, (size_t)C.nActiveVs)); return true; }
-    if (name == "McInv") { out = diag_csr(S.mcInv.to_host(S.st, (size_t)C.nActiveVs)); return true; }
-    if (name == "uInv") { out = diag_csr(S.uInv.to_host(S.st, (size_t)C.nStresses)); return true; }
-    if (name == "u") { out = diag_csr(S.uDiag.to_host(S.st, (size_t)C.nStresses)); return true; }
-    const size_t NN = (size_t)RDOF * RDOF;
-    if (name == "Mr") { out = blockdiag_csr(R ? S.RG.Mr.to_host(S.st, R * NN) : std::vector<double>(), R); return true; }
-    if (name == "BInv") { out = blockdiag_csr(R ? S.RG.Binv.to_host(S.st, R * NN) : std::vector<double>(), R); return true; }
-    if (name == "B") {
-        std::vector<double> b(R * NN);
-        if (R) { auto m = S.RG.Mr.to_host(S.st, R * NN); auto v = S.RG.Visc.to_host(S.st, R * NN); for (size_t i = 0; i < b.size(); ++i) b[i] = S.g.invDt * m[i] + 2. * v[i]; }
-        out = blockdiag_csr(b, R); return true;
-    }
-    return false;
-}
-// several ranks: region blocks exist only on their owner
-void mask_region_blocks(const Solver& S, const std::string& name, HostCsr& m) {
-    if (!S.part.multi() || !(name == "Mr" || name == "B" || name == "BInv")) return;
-    const size_t NN = (size_t)RDOF * RDOF;
-    for (size_t i = 0; i < m.val.size(); ++i) { const int r = (int)(i / NN); if (r < S.RG.regLo || r >= S.RG.regHi) m.val[i] = 0.; }
-}
-
-bool get_vector(Solver& S, const std::string& n, std::vector<double>& out) {
-    const Counts& C = S.C; const int R = S.RG.count; const size_t NN = (size_t)RDOF * RDOF;
-    if (n == "activeRHS") out = S.rhsU.to_host(S.st, (size_t)C.nActiveVs);
-    else if (n == "oldActiveVs") out = S.oldVs.to_host(S.st, (size_t)C.nActiveVs);
-    else if (n == "reducedRHS") out = R ? S.RG.rhsR.to_host(S.st, (size_t)R * RDOF) : std::vector<double>();
-    else if (n == "pressureRHS") out = S.rhsPT.to_host(S.st, (size_t)C.nPressures);
-    else if (n == "stressRHS") { auto v = S.rhsPT.to_host(S.st, (size_t)C.nSystemSize); out.assign(v.begin() + C.nPressures, v.end()); }
-    else if (n == "b") out = S.b.to_host(S.st, (size_t)C.nSystemSize);
-    else if (n == "solution") out = S.x.to_host(S.st, (size_t)C.nSystemSize);
-    else if (n == "velSolution") out = S.velSol.to_host(S.st, (size_t)(C.nActiveVs + C.nReducedVs));
-    else if (n == "com") out = R ? S.RG.com.to_host(S.st, (size_t)3 * R) : std::vector<double>();
-    else if (n == "bestFit") out = R ? S.RG.bestFit.to_host(S.st, (size_t)R * RDOF) : std::vector<double>();
-    else if (n == "MrDense") out = R ? S.RG.Mr.to_host(S.st, R * NN) : std::vector<double>();
-    else if (n == "ViscDense") out = R ? S.RG.Visc.to_host(S.st, R * NN) : std::vector<double>();
-    else if (n == "BinvDense") out = R ? S.RG.Binv.to_host(S.st, R * NN) : std::vector<double>();
-    else if (n == "guess") { if (S.guess.n < (size_t)C.nSystemSize) out.assign((size_t)C.nSystemSize, 0.); else out = S.guess.to_host(S.st, (size_t)C.nSystemSize); }
-    else if (n == "diagA") { if (S.part.multi()) return false; S.computeDiagonal(); out = S.diagA.to_host(S.st, (size_t)C.nSystemSize); }
-    else return false;
-    // several ranks: keep only this rank's share (the sum over ranks is the global vector)
-    if (S.part.multi()) {
-        if (n == "b" || n == "solution") { for (size_t i = 0; i < out.size(); ++i) if (!S.ownSys.has((int64_t)i)) out[i] = 0.; }
-        else if (n == "velSolution") {
-            for (size_t i = 0; i < out.size(); ++i) {
-                const bool mine = (int64_t)i < C.nActiveVs ? S.ownK.has((int64_t)i) : ((int64_t)(i - C.nActiveVs) / RDOF >= S.RG.regLo && (int64_t)(i - C.nActiveVs) / RDOF < S.RG.regHi);
-                if (!mine) out[i] = 0.;
-            }
-        } else if (n == "reducedRHS" || n == "bestFit" || n == "MrDense" || n == "ViscDense" || n == "BinvDense") {
-            const size_t per = (n == "reducedRHS" || n == "bestFit") ? (size_t)RDOF : NN;
-            for (size_t i = 0; i < out.size(); ++i) { const int r = (int)(i / per); if (r < S.RG.regLo || r >= S.RG.regHi) out[i] = 0.; }
+    auto diag = [&](const DBuf<double>& d, int64_t n, const Spans& own) {
+        Piece p; p.v = d.to_host(S.st, (size_t)n); p.own = own;
+        const std::vector<double> v = view(S, std::move(p), global);
+        if (here) out = diag_csr(v);
+    };
+    const Spans active = spans_in(S.ownK, 0, C.nActiveVs), stress = spans_in(S.ownSys, C.nPressures, C.nSystemSize);
+    if (name == "Mc") diag(S.mc, C.nActiveVs, active);
+    else if (name == "McInv") diag(S.mcInv, C.nActiveVs, active);
+    else if (name == "uInv") diag(S.uInv, C.nStresses, stress);
+    else if (name == "u") diag(S.uDiag, C.nStresses, stress);
+    else {
+        // the region blocks; a rank's own view holds those of its own regions only (the blocks of the other regions are zero)
+        std::vector<double> a, v;
+        get_vector(S, name == "BInv" ? "BinvDense" : "MrDense", a, global);
+        if (name == "B") {
+            get_vector(S, "ViscDense", v, global);
+            for (size_t i = 0; i < a.size(); ++i) a[i] = S.g.invDt * a[i] + 2. * v[i];
         }
+        if (here) out = blockdiag_csr(a, R);
     }
-    return true;
 }
 
 // Eigen::saveMarket / saveMarketVector format (extern/eigen/unsupported/Eigen/src/SparseExtra/MarketIO.h:311-372)
@@ -325,6 +465,15 @@ bool save_market_vector(const std::vector<double>& v, const std::string& path) {
     out << "%%MatrixMarket matrix array real general\n" << v.size() << " " << 1 << "\n";
     for (double x : v) out << x << "\n";
     return true;
+}
+
+// The views of a ps_create_multi handle are the global objects: fn(S, global = true, answer) runs on every rank (collective) and
+// rank 0 answers the caller.  A single-GPU handle, or one rank of a job with one process per GPU, answers with its own view.
+template <class Fn>
+int views(ps_handle h, Fn&& fn) {
+    if (!h->multi) return guarded(h, [&] { return fn(*h->S, false, true); });
+    MultiGroup* G = h->multi;
+    return G->run([&](int k) { ps_solver* kid = G->kids[(size_t)k]; return guarded(kid, [&] { return fn(*kid->S, true, k == 0); }); });
 }
 
 }  // namespace
@@ -566,12 +715,15 @@ int64_t ps_get_weight_field(ps_handle h, int liquid, int slot, float* out) {
 
 int ps_get_csr(ps_handle h, const char* name, int64_t* rows, int64_t* cols, int64_t* nnz, int64_t* rowptr, int32_t* colidx, double* vals) {
     if (!h || !name) return PS_INVALID;
-    if (h->multi) { g_lastError = "ps_get_csr: the matrices of a ps_create_multi handle live on several GPUs; use a single-GPU handle"; return PS_INVALID; }
-    return guarded(h, [&] {
+    const std::string nm(name);
+    if (!is_matrix(nm)) { g_lastError = "ps_get_csr: unknown matrix " + nm; return PS_INVALID; }
+    return views(h, [&](Solver& S, bool global, bool answer) {
         HostCsr m;
-        if (!get_matrix(*h->S, name, m)) { g_lastError = std::string("ps_get_csr: unknown matrix ") + name; return (int)PS_INVALID; }
-        mask_region_blocks(*h->S, name, m);
-        if (rows) *rows = m.rows; if (cols) *cols = m.cols; if (nnz) *nnz = (int64_t)m.idx.size();
+        get_matrix(S, nm, m, global);
+        if (!answer) return (int)PS_SUCCESS;
+        if (rows) *rows = m.rows;
+        if (cols) *cols = m.cols;
+        if (nnz) *nnz = (int64_t)m.idx.size();
         if (rowptr) std::copy(m.ptr.begin(), m.ptr.end(), rowptr);
         if (colidx) std::copy(m.idx.begin(), m.idx.end(), colidx);
         if (vals) std::copy(m.val.begin(), m.val.end(), vals);
@@ -580,17 +732,19 @@ int ps_get_csr(ps_handle h, const char* name, int64_t* rows, int64_t* cols, int6
 }
 int64_t ps_get_vector(ps_handle h, const char* name, double* out) {
     if (!h || !name) return -1;
-    if (h->multi) { g_lastError = "ps_get_vector: the vectors of a ps_create_multi handle live on several GPUs; use a single-GPU handle"; return -1; }
     int64_t n = -1;
-    guarded(h, [&] { std::vector<double> v; if (get_vector(*h->S, name, v)) { n = (int64_t)v.size(); if (out) std::copy(v.begin(), v.end(), out); } return 0; });
-    return n;
+    const int rc = views(h, [&](Solver& S, bool global, bool answer) {
+        std::vector<double> v;
+        if (!get_vector(S, name, v, global)) { g_lastError = std::string("ps_get_vector: no vector ") + name + " on this handle"; return (int)PS_INVALID; }
+        if (answer) { n = (int64_t)v.size(); if (out) std::copy(v.begin(), v.end(), out); }
+        return (int)PS_SUCCESS;
+    });
+    return rc == PS_SUCCESS ? n : -1;
 }
 
 int ps_apply(ps_handle h, const double* x, double* y) {
     if (!h || !x || !y) return PS_INVALID;
-    if (h->multi) { g_lastError = "ps_apply: not available on a ps_create_multi handle (use one handle per rank)"; return PS_INVALID; }
-    return guarded(h, [&] {
-        Solver& S = *h->S;
+    return views(h, [&](Solver& S, bool global, bool answer) {
         if (!S.haveSetup) throw Error("ps_apply: call ps_setup first");
         const size_t n = (size_t)S.C.nSystemSize;
         DBuf<double>& dx = scratch().applyX; DBuf<double>& dy = scratch().applyY;
@@ -598,7 +752,9 @@ int ps_apply(ps_handle h, const double* x, double* y) {
         copy_h2d(dx.p, x, n * sizeof(double), S.st);
         dy.zero(S.st, n);                       // several ranks: rows of other ranks stay 0 (sum over ranks = A x)
         S.applyOperator(dx.p, dy.p, nullptr);
-        copy_d2h(y, dy.p, n * sizeof(double), S.st);
+        if (!global || !S.part.multi()) { copy_d2h(y, dy.p, n * sizeof(double), S.st); return (int)PS_SUCCESS; }
+        const std::vector<double> all = gather_owned(S, dy.to_host(S.st, n), spans_in(S.ownSys, 0, (int64_t)n), (int64_t)n);
+        if (answer) std::copy(all.begin(), all.end(), y);
         return (int)PS_SUCCESS;
     });
 }
@@ -710,38 +866,53 @@ double ps_timer(ps_handle h, int stop) {
     return ms;
 }
 
+// On a decomposed handle (several ranks, either front end) ps_export is collective: the objects are assembled on rank 0 from their
+// owners (gather_owned), rank 0 alone writes, and one all-reduce of a status word gives every rank the same return code.
 int ps_export(ps_handle h, const char* prefix, int what) {
     if (!h || !prefix) return PS_INVALID;
-    if (h->multi) { g_lastError = "ps_export: the matrices of a slab-decomposed step live on several GPUs; export from a single-GPU handle"; return PS_INVALID; }
+    if (h->multi) { MultiGroup* G = h->multi; return G->run([&](int k) { return ps_export(G->kids[(size_t)k], prefix, what); }); }
     return guarded(h, [&] {
         Solver& S = *h->S; const std::string pre(prefix);
+        const bool multi = S.part.multi(), writer = S.part.rank == 0;
         bool ok = true;
         std::vector<double> v;
+        auto vec = [&](const char* name, const char* file) { if (get_vector(S, name, v, true) && writer) ok &= save_market_vector(v, pre + file); };
         if (what & 1) {   // exportMatrices / exportMatricesPostSolve (S.cpp:533-541, 568-572); A is implicit on this path
-            if (get_vector(S, "b", v)) ok &= save_market_vector(v, pre + "Vec_b.mtx");
-            if (get_vector(S, "guess", v)) ok &= save_market_vector(v, pre + "Vec_guess.mtx");
+            vec("b", "Vec_b.mtx");
+            vec("guess", "Vec_guess.mtx");
             // Mat_A.mtx: the explicit matrix exists only for solverType EIGEN (S_AS:7-27); the factored path leaves A an
             // empty nSystemSize x nSystemSize matrix (A.resize only, S_AS:446) and that is what the reference writes
             HostCsr Am;
-            if (S.P.solverType == 1 && !S.part.multi()) get_matrix(S, "A", Am);
+            if (S.P.solverType == 1 && !multi) get_matrix(S, "A", Am, true);
             else { Am.rows = Am.cols = S.C.nSystemSize; Am.ptr.assign((size_t)Am.rows + 1, 0); }
-            ok &= save_market(Am, pre + "Mat_A.mtx");
-            if (get_vector(S, "solution", v)) ok &= save_market_vector(v, pre + "solutionVector.mtx");
+            if (writer) ok &= save_market(Am, pre + "Mat_A.mtx");
+            vec("solution", "solutionVector.mtx");
         }
         if (what & 2) {   // exportComponentMatrices (S.cpp:543-566)
             const char* mats[] = {"Mc", "McInv", "Mr", "B", "BInv", "u", "uInv", "G", "Dt", "JG", "JDt"};
             const char* files[] = {"Mat_Mc.mtx", "Mat_McInv.mtx", "Mat_Mr.mtx", "Mat_Mr_plus_2JDtuDJ.mtx", "Mat_Inv_Mr_plus_2JDtuDJ.mtx", "Mat_u.mtx", "Mat_uInv.mtx",
                                    "Mat_G.mtx", "Mat_Dt.mtx", "Mat_JG.mtx", "Mat_JDt.mtx"};
-            for (int i = 0; i < 11; ++i) { HostCsr m; if (get_matrix(S, mats[i], m)) ok &= save_market(m, pre + files[i]); }
+            for (int i = 0; i < 11; ++i) { HostCsr m; get_matrix(S, mats[i], m, true); if (writer) ok &= save_market(m, pre + files[i]); }
             const char* vecs[] = {"activeRHS", "reducedRHS", "pressureRHS", "stressRHS"};
             const char* vfiles[] = {"Vec_activeRHS.mtx", "Vec_reducedRHS.mtx", "Vec_pressureRHS.mtx", "Vec_stressRHS.mtx"};
-            for (int i = 0; i < 4; ++i) if (get_vector(S, vecs[i], v)) ok &= save_market_vector(v, pre + vfiles[i]);
+            for (int i = 0; i < 4; ++i) vec(vecs[i], vfiles[i]);
         }
         if (what & 4) {   // exportStats (S.cpp:574-606)
             ps_stats st; S.fillStats(&st);
-            ok &= save_market_vector(std::vector<double>(st.dimData, st.dimData + 27), pre + "dimData.mtx");
-            ok &= save_market_vector(std::vector<double>(st.solveData, st.solveData + 6), pre + "solveData.mtx");
+            if (multi) {  // the counts are global already; the "thread count" is the SMs of all ranks, the times are the slowest rank's
+                const std::vector<double> all = S.hostAllgather({st.dimData[22], st.solveData[2], st.solveData[3], st.solveData[4], st.solveData[5]});
+                st.dimData[22] = 0.;
+                for (int k = 0; k < S.part.nranks; ++k) {
+                    st.dimData[22] += all[(size_t)5 * k];
+                    for (int j = 1; j < 5; ++j) st.solveData[1 + j] = std::max(st.solveData[1 + j], all[(size_t)5 * k + j]);
+                }
+            }
+            if (writer) {
+                ok &= save_market_vector(std::vector<double>(st.dimData, st.dimData + 27), pre + "dimData.mtx");
+                ok &= save_market_vector(std::vector<double>(st.solveData, st.solveData + 6), pre + "solveData.mtx");
+            }
         }
+        if (multi) ok = S.hostAllreduceSum(ok ? 0. : 1.) < 0.5;
         if (!ok) { g_lastError = "ps_export: could not write under prefix " + pre; return (int)PS_FAILED; }
         return (int)PS_SUCCESS;
     });

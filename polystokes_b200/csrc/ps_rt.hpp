@@ -180,6 +180,7 @@ struct Scratch {
     DBuf<unsigned long long> sums;
     DBuf<float> planes;
     DBuf<double> applyX, applyY;
+    DBuf<uint8_t> gather;                // staging of the pieces sent to rank 0 (ps_api.cu, gather_bytes)
 };
 extern thread_local Scratch* g_scratch;
 inline Scratch& scratch() { static thread_local Scratch fallback; return g_scratch ? *g_scratch : fallback; }

@@ -1382,22 +1382,32 @@ int Solver::solve() {
 
 // useWarmStart (PS.C:465-467): constructGuessVectors (S.cpp:521-531) + the copy into guessVector (S_AS:413-419)
 //   pressureGuess = -G^T u_old - JG^T v*  = (-K_ext^T w)_p,   stressGuess = -2 mu^-1 (-D u_old - DJ^T v*) = -2 mu^-1 (-K_ext^T w)_tau
-//   with w_active = u_old, w_f = c_f . v*_r on the coupled reduced rows.  Single GPU only (the live solver never reads it).
+//   with w_active = u_old, w_f = c_f . v*_r on the coupled reduced rows.  The live solver never reads it: one GPU forms it in the
+//   setup, several ranks only where it is read (ps_export, the global views of ps_api.cu), as a collective call.  Every rank forms
+//   its own rows; v*_r (bestFit) exists for every region whose rows the rank holds (built for [bldLo, regHi)), and neither the
+//   solve nor the write-back changes u_old or v*, so the guess formed after a step is the one of its setup.
 void Solver::constructGuessVectors() {
     haveGuess = false;
     const int64_t n = C.nSystemSize;
     guess.alloc((size_t)std::max<int64_t>(n, 1));
     guess.zero(st, (size_t)n);
-    if (!P.useWarmStart || part.multi() || n == 0) return;
+    if (!P.useWarmStart || n == 0) return;
+    PS_WHERE("constructGuessVectors");
     const OpArgs A = make_op(*this);
     w.zero(st, (size_t)C.nRowsExt);
-    copy_d2d(w.p, oldVs.p, (size_t)C.nActiveVs * sizeof(double), st);
+    for (int i = 0; i < ownK.n; ++i) {      // the owned active rows
+        const int64_t lo = ownK.lo[i], hi = std::min(ownK.lo[i] + ownK.count(i), C.nActiveVs);
+        if (hi > lo) copy_d2d(w.p + lo, oldVs.p + lo, (size_t)(hi - lo) * sizeof(double), st);
+    }
     if (RG.count > 0) {
         k_sigma_from_s(st, RG.count, RG.bestFit.p, RG.sigma.p);
         reduced_expand(st, g, RG, w.p + C.nActiveVs, 1.0, nullptr);
+        if (RG.nShared > 0) shared_expand(st, g, RG, w.p + C.nActiveVs, 1.0, nullptr);
     }
+    exchange(haloW, w.p, nullptr);
     k_pass2(st, A, w.p, nullptr, guess.p, 0.0, nullptr, nullptr, PeerCtx(), nullptr, 0);
     k_guess_finish(st, A, guess.p);
+    checkPeer("constructGuessVectors");
     haveGuess = true;
 }
 
@@ -1630,7 +1640,12 @@ void Solver::setup() {
     { StageTimer T(st, &stageMs[PS_STAGE_MATRIX_BLOCKS]); constructMatrixBlocks(); }
     PS_WHERE("setup: assemble");
     haveDiag = false; haveA = false;
-    { StageTimer T(st, &stageMs[PS_STAGE_ASSEMBLE]); constructGuessVectors(); assemble(); }
+    {
+        StageTimer T(st, &stageMs[PS_STAGE_ASSEMBLE]);
+        if (part.multi()) haveGuess = false;      // formed on demand (collective), a plain step pays nothing for it
+        else constructGuessVectors();
+        assemble();
+    }
     haveSetup = true;
     result = R_INCOMPLETE;
 }
