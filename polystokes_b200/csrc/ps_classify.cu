@@ -28,7 +28,8 @@ void k_build_weights(cudaStream_t st, const Geom& g, const Fields& F, uint8_t* s
     // Every slot's sub-sample stencil at index c lies inside that block (base cells c-1..c per axis, +1 for the upper
     // trilinear corner; an index one past the centre range clamps into the block of the last cell), so where the block
     // has one sign the eighth-counts are 0 or 8 without touching the SDFs again; the exact per-slot test below only
-    // runs near the interfaces.
+    // runs near the interfaces.  A NaN sets both bits of its field: a sub-sample whose interpolation meets a NaN is
+    // NaN, and counts as neither liquid nor fluid, which only the exact test gets right.
     {
         const float* surf = F.surface; const float* coll = F.collision;
         for_window(st, g, SL_CENTER, PS_LAMBDA(int64_t q) {
@@ -37,7 +38,8 @@ void k_build_weights(cudaStream_t st, const Geom& g, const Fields& F, uint8_t* s
             for (int d = -1; d <= 1; ++d) {
                 const int64_t l = lin(g, SL_CENTER, clamped(g, SL_CENTER, I3{c.x + d, c.y, c.z}));
                 const float sv = surf[l], cv = coll[l];
-                code |= (sv < 0.f ? 1 : 0) | (sv >= 0.f ? 2 : 0) | (cv < 0.f ? 4 : 0) | (cv >= 0.f ? 8 : 0);
+                code |= (sv < 0.f ? 1 : 0) | (sv >= 0.f ? 2 : 0) | (cv < 0.f ? 4 : 0) | (cv >= 0.f ? 8 : 0)
+                      | (sv != sv ? 3 : 0) | (cv != cv ? 12 : 0);
             }
             signX[q] = (uint8_t)code;
         }, 1);
@@ -60,7 +62,7 @@ void k_build_weights(cudaStream_t st, const Geom& g, const Fields& F, uint8_t* s
             const I3 c = delin(g, slot, q);
             {
                 const int box = signBox[lin(g, SL_CENTER, clamped(g, SL_CENTER, c))];
-                if ((box & 3) != 3 && (box & 12) != 12) {      // one sign each (a NaN-only block has neither bit: 8 / 8 as below)
+                if ((box & 3) != 3 && (box & 12) != 12) {      // one sign each, no NaN
                     lw[q] = (uint8_t)((box & 3) != 2 ? 8 : 0); fw[q] = (uint8_t)((box & 12) != 4 ? 8 : 0);
                     return;
                 }
@@ -77,8 +79,10 @@ void k_build_weights(cudaStream_t st, const Geom& g, const Fields& F, uint8_t* s
                 }
             // Every sub-sample is a convex combination (all 8 trilinear weights are positive: fractions are 1/4 or 3/4)
             // of the SDF values in the <= 3x3x3 cell block below, so away from the interfaces the count is decided
-            // by the signs alone -- exactly, rounding included -- and the fp64 interpolation is skipped.
+            // by the signs alone -- exactly, rounding included -- and the fp64 interpolation is skipped.  fminf / fmaxf
+            // skip a NaN, so a NaN in the block forces the exact test.
             float minS = 3.4e38f, maxS = -3.4e38f, minC = 3.4e38f, maxC = -3.4e38f;
+            bool nanS = false, nanC = false;
             {
                 int lo[3], hi[3];
                 for (int a = 0; a < 3; ++a) { lo[a] = min(base[a][0], base[a][1]); hi[a] = max(base[a][0], base[a][1]) + 1; }
@@ -86,9 +90,10 @@ void k_build_weights(cudaStream_t st, const Geom& g, const Fields& F, uint8_t* s
                     const int64_t l = lin(g, SL_CENTER, clamped(g, SL_CENTER, I3{x, y, z}));
                     const float sv = surf[l], cv = coll[l];
                     minS = fminf(minS, sv); maxS = fmaxf(maxS, sv); minC = fminf(minC, cv); maxC = fmaxf(maxC, cv);
+                    nanS |= sv != sv; nanC |= cv != cv;
                 }
             }
-            const bool needL = !(minS >= 0.f || maxS < 0.f), needF = !(minC >= 0.f || maxC < 0.f);
+            const bool needL = nanS || !(minS >= 0.f || maxS < 0.f), needF = nanC || !(minC >= 0.f || maxC < 0.f);
             int nl = (maxS < 0.f) ? 8 : 0, nf = (minC >= 0.f) ? 8 : 0;
             if (needL || needF) {
                 int cl = 0, cf = 0;

@@ -119,7 +119,8 @@ def main():
         attach_gloo(s)
     rank, n, zlo, zhi, cuts = s.partition()
     s.setup_scene(sc)
-    out = dict(rank=rank, nranks=n, zlo=zlo, zhi=zhi, cuts=np.array(cuts), peer=s.count("peerTransport") if gpu else 0, local=s.count("slabLocal"))
+    out = dict(rank=rank, nranks=n, zlo=zlo, zhi=zhi, cuts=np.array(cuts), peer=s.count("peerTransport") if gpu else 0, local=s.count("slabLocal"),
+               shared=s.count("sharedRegions"))
     for k in parity.COUNTS:
         out["count_" + k] = s.count(k)
     for slot in range(7):

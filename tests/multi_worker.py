@@ -10,6 +10,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import edge_cases  # noqa: E402
 import parity  # noqa: E402
 from polystokes_b200 import PolyStokesSolver, scenes  # noqa: E402
 
@@ -18,6 +19,8 @@ CASES = {
     "blob48_tile8_pad1": lambda: scenes.blob_scene(48, seed=21, tile=8, pad=1),                         # replicated setup (boundary fix-up)
     "box64_uniform": lambda: scenes.box_scene(64, doReduced=0, tolerance=1e-6),
     "s3_128": lambda: scenes.scene_s3(128),
+    # liquid on the domain faces (tests/test_input_edges.py)
+    **{name: (lambda c: lambda: c()[0])(case) for name, case in edge_cases.DIST.items()},
 }
 
 

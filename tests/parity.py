@@ -8,6 +8,7 @@ import os
 
 import numpy as np
 
+import edge_cases
 from polystokes_b200 import PolyStokesSolver, scenes
 from oracle.oracle import Oracle
 
@@ -45,6 +46,8 @@ DIST_CASES = {
     "blob_40x36x96_tile32_pad3": lambda: (scenes.blob_scene((40, 36, 96), seed=11, tile=32, pad=3, liquidLayers=3, solidLayers=3, tolerance=1e-6), {}),
     # CG runs out of iterations -> BiCGSTAB fallback, itself stopped after 6 iterations (results kept): checks the arithmetic
     "blob48_bicgstab6": lambda: (scenes.blob_scene(48, seed=21, tile=8, pad=1, maxIterations=6, tolerance=1e-12, keepNonConvergedResults=1), {}),
+    # liquid on the domain faces, in the first and the last slab (tests/test_input_edges.py)
+    **edge_cases.DIST,
 }
 
 
