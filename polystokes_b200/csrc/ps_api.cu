@@ -679,7 +679,7 @@ int64_t ps_get_count(ps_handle h, const char* name) {
     // the shape of the reduced regions and the kernels their term of an apply takes (ps_pcg.cu, region_path)
     if (n == "maxRegionRows") return S.RG.maxRegionRows; if (n == "maxRegionAxisRows") return S.RG.maxRegionAxisRows;
     if (n == "maxRegionCells") return S.RG.maxRegionCells; if (n == "minRegionCells") return S.RG.minRegionCells;
-    if (n == "regionPath") return region_path(S.make_op_args(), S.RG);
+    if (n == "regionPath") return region_path(S.RG);
     return INT64_MIN;
 }
 double ps_get_real(ps_handle h, const char* name) {

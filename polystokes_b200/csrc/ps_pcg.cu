@@ -113,9 +113,7 @@ static_assert(HOT_THREADS == SCHED_BLOCK, "one schedule block per CTA iteration"
 // starts with pdl_sync(): "launch_dependents" lets the NEXT kernel's CTAs take SM slots as soon as this kernel's CTAs
 // drain (their launch latency and prologue hide under this kernel's tail), "wait" blocks until the PREVIOUS kernel has
 // completed and flushed -- so nothing that reads or writes global memory may precede it (kernel parameters are fine).
-// PS_PDL=0 launches the same kernels with plain stream order (the instructions are no-ops then).
 __device__ __forceinline__ void pdl_sync() { asm volatile("griddepcontrol.launch_dependents;\n\tgriddepcontrol.wait;" ::: "memory"); }
-static inline bool pdl_enabled() { static const bool on = !(getenv("PS_PDL") && atoi(getenv("PS_PDL")) == 0); return on; }
 template <class... KA, class... AA>
 static inline void launch_chain(void (*kernel)(KA...), unsigned grid, unsigned block, cudaStream_t st, AA&&... args) {
     cudaLaunchConfig_t cfg;
@@ -123,7 +121,7 @@ static inline void launch_chain(void (*kernel)(KA...), unsigned grid, unsigned b
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = 0; cfg.stream = st;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.attrs = at; cfg.numAttrs = 1;
     PS_CUDA(cudaLaunchKernelEx(&cfg, kernel, std::forward<AA>(args)...));
 }
 
@@ -189,7 +187,7 @@ __device__ __forceinline__ void pass1_block(const OpArgs& A, const double* __res
     for (int k2 = 0; k2 < 8; ++k2) s += ((double)op_code(word, k2) * sc) * xv[k2];
     w[r] = r < A.nActiveVs ? activeScale * lut[__ldcs(A.kmc + r)] * s : s;     // coupled reduced rows keep the raw (K_red x)_f
 }
-__global__ void __launch_bounds__(HOT_THREADS, 6) pass1_kernel(const __grid_constant__ OpArgs A, const double* __restrict__ x, double* __restrict__ w, double activeScale, const PcgScalars* S, int reverse,
+__global__ void __launch_bounds__(HOT_THREADS, 6) pass1_kernel(const __grid_constant__ OpArgs A, const double* __restrict__ x, double* __restrict__ w, double activeScale, const PcgScalars* S,
                                                              const int32_t* __restrict__ sched, int nSched, const __grid_constant__ VecLink V) {    pdl_sync();
 
     __shared__ double lut[65];
@@ -199,7 +197,7 @@ __global__ void __launch_bounds__(HOT_THREADS, 6) pass1_kernel(const __grid_cons
     if (!vec_wait(V)) { if (threadIdx.x == 0) const_cast<PcgScalars*>(S)->peerError = 1; return; }      // the neighbours' entries of x (direct halo stores)
     // owned rows in the merged block order of the ranges (SchedRanges, ps_solver.hpp)
 #pragma unroll 2
-    for (int g = blockIdx.x; g < nSched; g += gridDim.x) pass1_block(A, x, w, activeScale, lut, __ldg(sched + (reverse ? nSched - 1 - g : g)));
+    for (int g = blockIdx.x; g < nSched; g += gridDim.x) pass1_block(A, x, w, activeScale, lut, __ldg(sched + g));
 }
 // last CTA of a producer: v0..v2 are valid in thread 0; every rank's block receives this rank's partial sums
 __device__ __forceinline__ void publish_partials(const PeerCtx& P, int slot, double v0, double v1, double v2) {
@@ -213,10 +211,11 @@ __device__ __forceinline__ void publish_partials(const PeerCtx& P, int slot, dou
 // dot(r2, y) and dot(y, y) (r.Ap, Ap.Ap) -> red[1], red[2] while y is in registers (the update kernel's beta, see above).
 // Cell sweep: one thread computes the pressure row and the xx / yy / zz stress rows of its cell from ONE set of 6
 // columns, codes and w gathers (32 B of matrix per cell); edge sweep: 4 columns + 4 codes (20 B per edge).
-template <int OCC>
-__global__ void __launch_bounds__(HOT_THREADS, OCC) pass2_kernel(const __grid_constant__ OpArgs A, const double* __restrict__ w, const double* __restrict__ x, double* __restrict__ y,
-                                                              double muScale, const double* __restrict__ add, double* dotPartial, PcgScalars* S, int mode, const __grid_constant__ PeerCtx P,
-                                                              const double* __restrict__ r2, int reverse, const __grid_constant__ VecLink V) {    pdl_sync();
+// 6 resident CTAs per SM.  Measured on S3 256^3 (profiles/r01_sweep_occupancy.log): 4 -> 0.148 ms, 5 -> 0.137 ms, 6 -> 0.132 ms,
+// 7 / 8 spill and fall back to 0.137 ms
+__global__ void __launch_bounds__(HOT_THREADS, 6) pass2_kernel(const __grid_constant__ OpArgs A, const double* __restrict__ w, const double* __restrict__ x, double* __restrict__ y,
+                                                            double muScale, const double* __restrict__ add, double* dotPartial, PcgScalars* S, int mode, const __grid_constant__ PeerCtx P,
+                                                            const double* __restrict__ r2, const __grid_constant__ VecLink V) {    pdl_sync();
 
     if (S && S->done) return;
     if (blockIdx.x == 0 && threadIdx.x == 0) vec_raise(V);                     // this rank's rows of w are in the neighbours' vectors (the push launch before this one)
@@ -228,7 +227,7 @@ __global__ void __launch_bounds__(HOT_THREADS, OCC) pass2_kernel(const __grid_co
     // owned rows in the merged block order: range 0 = cells, 1..3 = yz / xz / xy edges (SchedRanges, ps_solver.hpp)
 #pragma unroll 1
     for (int g = blockIdx.x; g < A.nSched2; g += gridDim.x) {
-        const int32_t se = __ldg(A.sched2 + (reverse ? A.nSched2 - 1 - g : g));
+        const int32_t se = __ldg(A.sched2 + g);
         const int k = (int)((uint32_t)se >> 28);
         const int64_t row = A.s2.lo[k] + (int64_t)(se & 0x0fffffff) * SCHED_BLOCK + threadIdx.x;
         if (row >= A.s2.hi[k]) continue;
@@ -304,8 +303,9 @@ __global__ void __launch_bounds__(HOT_THREADS, OCC) pass2_kernel(const __grid_co
 // pass 2 and the global r.r of the previous update, beta from |r - alpha Ap|^2 = r.r - 2 alpha r.Ap + alpha^2 Ap.Ap.
 // x += alpha p always (pcg.h:314 runs before the stop test); r and p are only advanced if the stop test did not fire.
 // The last CTA then advances the CG state (every CTA has read the scalars by then).
-__global__ void __launch_bounds__(HOT_THREADS) cg_update_kernel(RangeSet own, double* __restrict__ x, double* __restrict__ r, double* __restrict__ p, const double* __restrict__ Ap,
-                                                               double* dotPartial, PcgScalars* S, const __grid_constant__ PeerCtx P, int reverse, const __grid_constant__ VecLink V) {    pdl_sync();
+// (3 resident CTAs per SM at 80 registers: without the bound ptxas takes 64 and spills)
+__global__ void __launch_bounds__(HOT_THREADS, 3) cg_update_kernel(RangeSet own, double* __restrict__ x, double* __restrict__ r, double* __restrict__ p, const double* __restrict__ Ap,
+                                                               double* dotPartial, PcgScalars* S, const __grid_constant__ PeerCtx P, const __grid_constant__ VecLink V) {    pdl_sync();
 
     if (S->done) return;
     double a[3] = {S->red[0], S->red[1], S->red[2]}, b[3] = {S->red[3], S->red[4], S->red[5]};
@@ -320,19 +320,7 @@ __global__ void __launch_bounds__(HOT_THREADS) cg_update_kernel(RangeSet own, do
     const double beta = rrNew / rsold;
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
     double rr = 0., xp = 0., pp = 0.;
-    if (!converged && reverse) {
-        // the same sweep from the far end (local item total - 1 - l): starts on the part of Ap that pass 2 wrote last
-        const int64_t total = own.total();
-#pragma unroll 4
-        for (int64_t l = tid; l < total; l += stride) {
-            const int64_t i = own.at(total - 1 - l);
-            const double pi = p[i];
-            const double xi = x[i] + alpha * pi, ri = cg_r_new(r[i], alpha, Ap[i]);
-            const double pn = cg_p_new(ri, beta, pi);
-            x[i] = xi; r[i] = ri; p[i] = pn;
-            rr += ri * ri; xp += xi * pn; pp += pn * pn;
-        }
-    } else if (!converged && own.n == 1 && !(own.lo[0] & 1)) {
+    if (!converged && own.n == 1 && !(own.lo[0] & 1)) {
         // one owned range (a single GPU): two consecutive elements per thread and step as 16-byte accesses -- half the memory
         // instructions of the scalar walk below
         const int64_t base = own.lo[0], total = own.total(), pairs = total >> 1;
@@ -409,33 +397,7 @@ __global__ void cg_begin_kernel(PcgScalars* S, const __grid_constant__ PeerCtx P
     if (P.nranks > 1 && !peer_reduce_wait(P, 1, P.seqIn, bb, 3)) { if (threadIdx.x == 0) { S->peerError = 1; S->done = 1; } return; }
     if (threadIdx.x == 0) { S->red[6] = bb[0]; S->rsold = bb[0]; S->done = (bb[0] == 0.) ? 1 : 0; }
 }
-// halo exchange over peer memory, sender side: gather the boundary entries and store them straight into the
-// neighbours' receive buffers (NVLink), then raise their sequence flags once every CTA's stores are fenced
-__global__ void __launch_bounds__(256) halo_push_kernel(int64_t n0, int64_t n1, const int32_t* __restrict__ idx, const double* __restrict__ v,
-                                                       double* __restrict__ dst0, double* __restrict__ dst1, unsigned long long* flag0, unsigned long long* flag1,
-                                                       unsigned long long seq, PcgScalars* S, int respectDone, unsigned int* ticket) {    pdl_sync();
-
-    if (respectDone && S->done) return;
-    const int64_t n = n0 + n1;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const double val = v[idx[i]];
-        if (i < n0) dst0[i] = val; else dst1[i - n0] = val;
-    }
-    // One system fence per CTA, not per thread (membar.sys by every warp costs ~20 us here): the CTA barrier orders
-    // all threads' stores before thread 0's fence, the fence makes them visible system-wide before the ticket,
-    // and the last CTA's release store publishes the flag after every CTA's fence (cumulative).
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        const unsigned t = atomicInc(ticket, gridDim.x - 1);
-        if (t == gridDim.x - 1) {
-            __threadfence_system();
-            if (flag0) peer_st_flag(flag0, seq);
-            if (flag1) peer_st_flag(flag1, seq);
-        }
-    }
-}
-// The same push with the entries stored at their FINAL place: the neighbours map this rank's vector arena (PeerLink::vecBase), entry j
+// Halo push over peer memory with the entries stored at their FINAL place: the neighbours map this rank's vector arena (PeerLink::vecBase), entry j
 // of my vector goes to entry j of theirs (vectors are global-length everywhere).  Nothing is unpacked on the other side: the kernel
 // that consumes the vector there waits for the flag at its head (VecLink).  This launch never waits, so it cannot stall behind a
 // slower neighbour; its tail (two system fences + the flag's NVLink trip) hides under the consumer's launch.
@@ -473,25 +435,6 @@ __global__ void __launch_bounds__(256) halo_push_p_kernel(int64_t n0, int64_t n1
         if (i < n0) dst0[j] = val; else dst1[j] = val;
     }
 }
-// receiver side: wait for the neighbours' flags, then scatter the received entries into the global-length vector
-__global__ void __launch_bounds__(256) halo_wait_unpack_kernel(int64_t n0, int64_t n1, const int32_t* __restrict__ idx, const double* src0, const double* src1,
-                                                              const unsigned long long* flag0, const unsigned long long* flag1, unsigned long long seq,
-                                                              double* __restrict__ v, PcgScalars* S, int respectDone) {    pdl_sync();
-
-    if (respectDone && S->done) return;
-    __shared__ int ok;
-    if (threadIdx.x == 0) {
-        bool good = true;
-        if (flag0) good = peer_wait_flag(flag0, seq) && good;
-        if (flag1) good = peer_wait_flag(flag1, seq) && good;
-        ok = good ? 1 : 0;
-    }
-    __syncthreads();
-    if (!ok) { if (threadIdx.x == 0) S->peerError = 1; return; }
-    const int64_t n = n0 + n1;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        v[idx[i]] = __ldcg(i < n0 ? src0 + i : src1 + (i - n0));
-}
 // Both sides in ONE launch (<= one CTA per SM, so every CTA is resident): each CTA first pushes its share of my boundary
 // entries, the last CTA to finish raises the neighbours' flags, then every CTA waits for MY flags and scatters its share of
 // what the neighbours stored here.  No CTA waits before it has pushed, so two ranks can never wait on each other.
@@ -507,6 +450,9 @@ __global__ void __launch_bounds__(256) halo_exchange_kernel(int64_t ns0, int64_t
         const double val = v[sendIdx[i]];
         if (i < ns0) dst0[i] = val; else dst1[i - ns0] = val;
     }
+    // One system fence per CTA, not per thread (membar.sys by every warp costs ~20 us here): the CTA barrier orders
+    // all threads' stores before thread 0's fence, the fence makes them visible system-wide before the ticket,
+    // and the last CTA's release store publishes the flag after every CTA's fence (cumulative).
     __shared__ int ok;
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -556,29 +502,22 @@ static inline int hot_blocks(K kernel, int64_t n) {
     return (int)b;
 }
 
-void k_pass1(cudaStream_t st, const OpArgs& A, const double* x, double* w, double activeScale, const PcgScalars* S, bool reverse, int part, const VecLink& V) {
-    // part 0: every owned row; 1: the coupled reduced rows only (schedule 1a); the active rows alone go with the regions (k_pass1_regions)
-    const int32_t* sched = part == 1 ? A.sched1a : A.sched1; const int n = part == 1 ? A.nSched1a : A.nSched1;
+void k_pass1(cudaStream_t st, const OpArgs& A, const double* x, double* w, double activeScale, const PcgScalars* S, const VecLink& V) {
+    const int n = A.nSched1;
     if (n <= 0 && !V.waitSeq) return;
-    launch_chain(pass1_kernel, hot_blocks(pass1_kernel, (int64_t)std::max(n, 1) * HOT_THREADS), HOT_THREADS, st, A, x, w, activeScale, S, reverse ? 1 : 0, sched, n, V);
+    launch_chain(pass1_kernel, hot_blocks(pass1_kernel, (int64_t)std::max(n, 1) * HOT_THREADS), HOT_THREADS, st, A, x, w, activeScale, S, A.sched1, n, V);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
-void k_pass2(cudaStream_t st, const OpArgs& A, const double* w, const double* x, double* y, double muScale, const double* add, double* dotPartial, const PeerCtx& P, PcgScalars* scal, int mode, const double* r2, bool reverse, const VecLink& V) {
-    // resident CTAs per SM the kernel is compiled for.  Measured on S3 256^3 (profiles/r01_sweep_occupancy.log): 4 -> 0.148 ms, 5 -> 0.137 ms,
-    // 6 -> 0.132 ms, 7 / 8 spill and fall back to 0.137 ms
-    static const int occ = getenv("PS_PASS2_OCC") ? atoi(getenv("PS_PASS2_OCC")) : 6;
+void k_pass2(cudaStream_t st, const OpArgs& A, const double* w, const double* x, double* y, double muScale, const double* add, double* dotPartial, const PeerCtx& P, PcgScalars* scal, int mode, const double* r2, const VecLink& V) {
     const int64_t rows = A.rowsP.total() + A.rowsE.total();
     if (rows <= 0 && !(mode & 1)) return;
-    const int rev = reverse ? 1 : 0;
-    if (occ >= 6) launch_chain(pass2_kernel<6>, hot_blocks(pass2_kernel<6>, rows), HOT_THREADS, st, A, w, x, y, muScale, add, dotPartial, scal, mode, P, r2, rev, V);
-    else if (occ == 5) launch_chain(pass2_kernel<5>, hot_blocks(pass2_kernel<5>, rows), HOT_THREADS, st, A, w, x, y, muScale, add, dotPartial, scal, mode, P, r2, rev, V);
-    else launch_chain(pass2_kernel<4>, hot_blocks(pass2_kernel<4>, rows), HOT_THREADS, st, A, w, x, y, muScale, add, dotPartial, scal, mode, P, r2, rev, V);
+    launch_chain(pass2_kernel, hot_blocks(pass2_kernel, rows), HOT_THREADS, st, A, w, x, y, muScale, add, dotPartial, scal, mode, P, r2, V);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
-void k_cg_update(cudaStream_t st, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, bool reverse, const VecLink& V) {
-    launch_chain(cg_update_kernel, hot_blocks(cg_update_kernel, own.total()), HOT_THREADS, st, own, x, r, p, Ap, dotPartial, scal, P, reverse ? 1 : 0, V);
+void k_cg_update(cudaStream_t st, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, const VecLink& V) {
+    launch_chain(cg_update_kernel, hot_blocks(cg_update_kernel, own.total()), HOT_THREADS, st, own, x, r, p, Ap, dotPartial, scal, P, V);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
@@ -595,13 +534,6 @@ void k_cg_begin(cudaStream_t st, PcgScalars* scal, const PeerCtx& P) {
 void k_halo_pack(cudaStream_t st, int64_t n, const int32_t* idx, const double* v, double* buf, const PcgScalars* S) {
     if (n <= 0) return;
     launch_chain(halo_pack_kernel, (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 4), 256, st, n, idx, v, buf, S);
-    PS_COUNT_LAUNCH(1);
-    PS_CUDA(cudaGetLastError());
-}
-void k_halo_push_peer(cudaStream_t st, int64_t n0, int64_t n1, const int32_t* idx, const double* v, double* dst0, double* dst1, unsigned long long* flag0, unsigned long long* flag1,
-                      unsigned long long seq, PcgScalars* S, bool respectDone, unsigned int* ticket) {
-    const int64_t n = n0 + n1;
-    launch_chain(halo_push_kernel, (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sm_count())), 256, st, n0, n1, idx, v, dst0, dst1, flag0, flag1, seq, S, respectDone ? 1 : 0, ticket);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
@@ -628,13 +560,6 @@ void k_halo_exchange_peer(cudaStream_t st, int64_t ns0, int64_t ns1, const int32
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
-void k_halo_unpack_peer(cudaStream_t st, int64_t n0, int64_t n1, const int32_t* idx, const double* src0, const double* src1, const unsigned long long* flag0, const unsigned long long* flag1,
-                        unsigned long long seq, double* v, PcgScalars* S, bool respectDone) {
-    const int64_t n = n0 + n1;
-    launch_chain(halo_wait_unpack_kernel, (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 2)), 256, st, n0, n1, idx, src0, src1, flag0, flag1, seq, v, S, respectDone ? 1 : 0);
-    PS_COUNT_LAUNCH(1);
-    PS_CUDA(cudaGetLastError());
-}
 void k_halo_unpack(cudaStream_t st, int64_t n, const int32_t* idx, const double* buf, double* v, const PcgScalars* S) {
     if (n <= 0) return;
     launch_chain(halo_unpack_kernel, (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 4), 256, st, n, idx, buf, v, S);
@@ -642,11 +567,11 @@ void k_halo_unpack(cudaStream_t st, int64_t n, const int32_t* idx, const double*
     PS_CUDA(cudaGetLastError());
 }
 #else  // ---- serial twins ----
-void k_pass1(cudaStream_t, const OpArgs& A, const double* x, double* w, double activeScale, const PcgScalars* S, bool, int, const VecLink&) {
+void k_pass1(cudaStream_t, const OpArgs& A, const double* x, double* w, double activeScale, const PcgScalars* S, const VecLink&) {
     if (S && S->done) return;
     for (int64_t l = 0; l < A.rowsK.total(); ++l) { const int64_t r = A.rowsK.at(l); const double s = k_row(A, r, x); w[r] = r < A.nActiveVs ? activeScale * A.mcInvLut[A.kmc[r]] * s : s; }
 }
-void k_pass2(cudaStream_t, const OpArgs& A, const double* w, const double* x, double* y, double muScale, const double* add, double*, const PeerCtx&, PcgScalars* S, int mode, const double* r2, bool, const VecLink&) {
+void k_pass2(cudaStream_t, const OpArgs& A, const double* w, const double* x, double* y, double muScale, const double* add, double*, const PeerCtx&, PcgScalars* S, int mode, const double* r2, const VecLink&) {
     if (S && S->done) return;
     double acc = 0., accR = 0., accY = 0.;
     auto finish = [&](int64_t j, double ktw) {
@@ -667,7 +592,7 @@ void k_pass2(cudaStream_t, const OpArgs& A, const double* w, const double* x, do
     for (int64_t l = 0; l < A.rowsE.total(); ++l) { const int64_t e = A.rowsE.at(l); finish(A.nP + 3 * A.nC + e, kt_edge_row(A, e, w)); }
     if (mode & 1) { S->red[0] = acc; S->red[1] = accR; S->red[2] = accY; }
 }
-void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double*, PcgScalars* S, const PeerCtx&, bool, const VecLink&) {
+void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double*, PcgScalars* S, const PeerCtx&, const VecLink&) {
     if (S->done) return;
     const double rsold = S->red[3], alpha = rsold / S->red[0];
     const double rrNew = cg_next_rr(rsold, alpha, S->red[1], S->red[2]);
@@ -942,13 +867,12 @@ __global__ void __launch_bounds__(RED_THREADS) reduced_expand_kernel(double dx, 
 // GROUP threads per axis, ROWS rows per thread kept in registers between the two phases (0: re-read rowXYZ through L1/L2)
 template <int GROUP, int ROWS, int MINB>
 __global__ void __launch_bounds__(3 * GROUP, MINB) reduced_region_kernel(double dx, const uint32_t* __restrict__ rowXYZ, const int32_t* __restrict__ rowAxisStart, const double* __restrict__ com,
-                                                                       const double* __restrict__ Binv, double* __restrict__ wRows, double scale, const PcgScalars* S, int region0,
-                                                                       const int32_t* __restrict__ order) {
+                                                                       const double* __restrict__ Binv, double* __restrict__ wRows, double scale, const PcgScalars* S, int region0) {
     constexpr int NW = GROUP / 32, KEEP = ROWS > 0 ? ROWS : 1;
     __shared__ double Bs[RDOF * RDOF];
     __shared__ double red[3][NW][10];
     __shared__ double M[30], t[RDOF], sv[RDOF], sg[30];
-    const int r = order ? __ldg(order + region0 + blockIdx.x) : region0 + blockIdx.x;      // order: longest region first (setup data)
+    const int r = region0 + blockIdx.x;
     // B^-1, the row table and the centres of mass are setup data: they may be fetched before the previous kernel has finished
     for (int i = threadIdx.x; i < RDOF * RDOF; i += 3 * GROUP) Bs[i] = __ldg(Binv + (size_t)r * RDOF * RDOF + i);
     const int axis = threadIdx.x / GROUP, lane = threadIdx.x % GROUP;
@@ -1037,164 +961,29 @@ __global__ void __launch_bounds__(3 * GROUP, MINB) reduced_region_kernel(double 
         wRows[row] = scale * v;
     }
 }
-// (A/B variant, off by default -- see pass1_regions_applicable.)
-// Pass 1 over the ACTIVE rows and the reduced term of the same apply in ONE launch (the coupled reduced rows were swept by the
-// launch before: schedule 1a).  The region work is a latency chain (row round trip -> 30 moments -> 26x26 product -> expand) that
-// leaves the memory system idle, the sweep is bandwidth bound: run back to back they cost 0.10 + 0.05 ms, here every CTA
-// alternates between the two -- a region, a run of row blocks, a region, ... -- and odd CTAs start with rows, so at any moment
-// about half of the resident CTAs stream rows while the others sit in a region's chain.  No hand-off between CTAs: a region is
-// still summed by one CTA in the fixed order of reduced_region_kernel<64, 0, .> (bit-identical results), the rows are untouched.
-constexpr int PR_GROUP = 64, PR_NW = PR_GROUP / 32;
-struct RegionArgs { double dx; const uint32_t* rowXYZ; const int32_t* rowAxisStart; const double* com; const double* Binv; double* wRows; double scale; int regLo, regHi; };
-__global__ void __launch_bounds__(HOT_THREADS, 5) pass1_regions_kernel(const __grid_constant__ OpArgs A, const double* __restrict__ x, double* __restrict__ w, double activeScale, const PcgScalars* S,
-                                                                     const int32_t* __restrict__ sched, int nSched, const __grid_constant__ RegionArgs R) {
-    __shared__ double lut[65];
-    __shared__ double Bs[RDOF * RDOF];
-    __shared__ double red[3][PR_NW][10];
-    __shared__ double M[30], t[RDOF], sv[RDOF], sg[30];
-    pdl_sync();
-    if (S && S->done) return;
-    if (threadIdx.x < 65) lut[threadIdx.x] = A.mcInvLut[threadIdx.x];
-    __syncthreads();
-    const int nReg = R.regHi - R.regLo;
-    const int myRegs = (int)blockIdx.x < nReg ? (nReg - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-    const int myBlocks = (int)blockIdx.x < nSched ? (nSched - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-    bool rowsTurn = (blockIdx.x & 1) || myRegs == 0;
-    const int nRuns = myRegs + ((blockIdx.x & 1) ? 1 : 0);
-    const int run = nRuns > 0 ? (myBlocks + nRuns - 1) / nRuns : myBlocks;
-    const int axis = threadIdx.x / PR_GROUP, lane = threadIdx.x % PR_GROUP;      // axis 3: the last 64 threads only keep the barriers
-    int kb = 0, kr = 0;
-    for (;;) {
-        const bool haveB = kb < myBlocks, haveR = kr < myRegs;
-        if (!haveB && !haveR) break;
-        if ((rowsTurn && haveB) || !haveR) {
-            const int end = min(kb + run, myBlocks);
-#pragma unroll 2
-            for (int j = kb; j < end; ++j) pass1_block(A, x, w, activeScale, lut, __ldg(sched + blockIdx.x + (int64_t)j * gridDim.x));
-            kb = end;
-        } else {
-            const int r = R.regLo + (int)blockIdx.x + kr * (int)gridDim.x;
-            ++kr;
-            for (int i = threadIdx.x; i < RDOF * RDOF; i += HOT_THREADS) Bs[i] = __ldg(R.Binv + (size_t)r * RDOF * RDOF + i);
-            int begin = 0, end = 0;
-            double cm[3] = {0., 0., 0.};
-            if (axis < 3) {
-                begin = __ldg(R.rowAxisStart + 3 * r + axis); end = __ldg(R.rowAxisStart + 3 * r + axis + 1);
-                cm[0] = __ldg(R.com + 3 * r); cm[1] = __ldg(R.com + 3 * r + 1); cm[2] = __ldg(R.com + 3 * r + 2);
-            }
-            double acc[10];
-#pragma unroll
-            for (int k = 0; k < 10; ++k) acc[k] = 0.;
-#pragma unroll 4
-            for (int row = begin + lane; row < end; row += PR_GROUP) {
-                double m[10];
-                row_monomials(R.dx, __ldg(R.rowXYZ + row), cm, m);
-                const double g1 = __ldcs(R.wRows + row);
-#pragma unroll
-                for (int k = 0; k < 10; ++k) acc[k] += m[k] * g1;
-            }
-            if (axis < 3) {
-#pragma unroll
-                for (int k = 0; k < 10; ++k) {
-                    const double v = warp_sum(acc[k]);
-                    if ((lane & 31) == 0) red[axis][lane >> 5][k] = v;
-                }
-            }
-            __syncthreads();
-            if (threadIdx.x < 30) {
-                const int a = threadIdx.x / 10, k = threadIdx.x % 10;
-                double s = 0.;
-#pragma unroll
-                for (int wI = 0; wI < PR_NW; ++wI) s += red[a][wI][k];
-                M[threadIdx.x] = s;
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) moments_to_t(M, t);
-            __syncthreads();
-            if (threadIdx.x < RDOF) {
-                const double* B = Bs + threadIdx.x * RDOF;
-                double s = 0.;
-#pragma unroll
-                for (int j = 0; j < RDOF; ++j) s += B[j] * t[j];
-                sv[threadIdx.x] = s;
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) s_to_sigma(sv, sg);
-            __syncthreads();
-            if (axis < 3) {
-                double sgl[10];
-#pragma unroll
-                for (int k = 0; k < 10; ++k) sgl[k] = sg[axis * 10 + k];
-#pragma unroll 4
-                for (int row = begin + lane; row < end; row += PR_GROUP) {
-                    double m[10];
-                    row_monomials(R.dx, __ldg(R.rowXYZ + row), cm, m);
-                    double v = 0.;
-#pragma unroll
-                    for (int k = 0; k < 10; ++k) v += sgl[k] * m[k];
-                    R.wRows[row] = R.scale * v;
-                }
-            }
-            __syncthreads();      // Bs / red / sg are rewritten by the CTA's next region
-        }
-        rowsTurn = !rowsTurn;
-    }
-}
 // regions with more coupled rows than this take the chunked kernels (reduced_moments_kernel + reduced_expand_kernel)
 static int region_fuse_limit() {
     static const int fuseLimit = getenv("PS_REGION_FUSE_MAX") ? atoi(getenv("PS_REGION_FUSE_MAX")) : 16384;
     return fuseLimit;
 }
-bool pass1_regions_applicable(const OpArgs& A, const RegionData& RG) {
-    const int fuseLimit = region_fuse_limit();
-    // measured on S3 256^3 (profiles/r02_probe_s3_256_v8*.log): 0.181 ms against 0.141 ms for sweep + region kernel on one GPU -- a CTA
-    // sitting in a region's chain keeps 8 warps from streaming rows, and only ~half of the CTAs are in a chain at any time (5 rounds of
-    // regions instead of 2 waves).  Off by default; PS_OVERLAP=1 for A/B runs.
-    static const bool on = getenv("PS_OVERLAP") && atoi(getenv("PS_OVERLAP")) != 0;
-    return on && RG.regHi > RG.regLo && RG.maxRegionRows <= fuseLimit && A.nSched1a > 0;
-}
-bool k_pass1_regions(cudaStream_t st, const OpArgs& A, const double* x, double* w, double activeScale, const PcgScalars* S, const Geom& g, const RegionData& RG, double scale, const VecLink& V) {
-    if (!pass1_regions_applicable(A, RG)) return false;
-    k_pass1(st, A, x, w, activeScale, S, false, 1, V);        // the coupled reduced rows first: the regions read them (this launch waits for the neighbours' x)
-    const RegionArgs R = {g.dx, RG.rowXYZ.p, RG.rowAxisStart.p, RG.com.p, RG.Binv.p, w + A.nActiveVs, scale, RG.regLo, RG.regHi};
-    const int64_t items = std::max<int64_t>((int64_t)A.nSched1b, (int64_t)(RG.regHi - RG.regLo));
-    launch_chain(pass1_regions_kernel, hot_blocks(pass1_regions_kernel, items * HOT_THREADS), HOT_THREADS, st, A, x, w, activeScale, S, A.sched1b, A.nSched1b, R);
-    PS_COUNT_LAUNCH(1);
-    PS_CUDA(cudaGetLastError());
-    return true;
-}
 template <int GROUP, int ROWS, int MINB>
 static void launch_region(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
-    // PS_REGION_LPT=1: regions in the order of decreasing row count (A/B knob)
-    static const bool lpt = getenv("PS_REGION_LPT") && atoi(getenv("PS_REGION_LPT")) != 0;
-    const int32_t* order = lpt && RG.regionOrder.n >= (size_t)RG.regHi ? RG.regionOrder.p : nullptr;
-    launch_chain(reduced_region_kernel<GROUP, ROWS, MINB>, (unsigned)(RG.regHi - RG.regLo), 3 * GROUP, st, g.dx, RG.rowXYZ.p, RG.rowAxisStart.p, RG.com.p, RG.Binv.p, wRows, scale, S, RG.regLo, order);
+    launch_chain(reduced_region_kernel<GROUP, ROWS, MINB>, (unsigned)(RG.regHi - RG.regLo), 3 * GROUP, st, g.dx, RG.rowXYZ.p, RG.rowAxisStart.p, RG.com.p, RG.Binv.p, wRows, scale, S, RG.regLo);
 }
-// template instance of reduced_region_kernel for these regions.  A/B knob.  Default: 64 lanes per axis, 6 CTAs per SM for many regions
-// (throughput); few regions per GPU (slab decomposition) are latency bound -- 128 lanes per axis with the rows kept in registers put
-// every load of a region in flight at once
-static int region_variant(const RegionData& RG) {
-    static const int forced = getenv("PS_REGION_VARIANT") ? atoi(getenv("PS_REGION_VARIANT")) : -1;
-    return forced >= 0 ? forced : (RG.regHi - RG.regLo <= 900 ? 1 : 0);
-}
-// which kernels carry the reduced term of a forward apply (pass1Apply), knobs included: -1 no owned region, 0 reduced_region_kernel with
-// 64 lanes per axis, 1 with 128 lanes, 2 the chunked kernels, 3 pass1_regions_kernel, 4 reduced_region_kernel with 32 lanes
-int region_path(const OpArgs& A, const RegionData& RG) {
+// which kernels carry the reduced term of a forward apply (reduced_apply): -1 no owned region, 0 reduced_region_kernel with 64 lanes per
+// axis, 1 with 128 lanes, 2 the chunked kernels.  64 lanes per axis and 6 CTAs per SM for many regions (throughput); few regions per GPU
+// (slab decomposition) are latency bound -- 128 lanes per axis with the rows kept in registers put every load of a region in flight at once
+int region_path(const RegionData& RG) {
     if (RG.regHi <= RG.regLo) return -1;
-    if (pass1_regions_applicable(A, RG)) return 3;
     if (RG.maxRegionRows > region_fuse_limit()) return 2;
-    const int variant = region_variant(RG);
-    return variant == 1 || variant == 4 ? 1 : (variant == 3 ? 4 : 0);
+    return RG.regHi - RG.regLo <= 900 ? 1 : 0;
 }
 // w_f <- scale * c_f . B^-1 J w on the coupled reduced rows (the reduced term of one operator apply)
 void reduced_apply(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
     if (RG.regHi <= RG.regLo) return;
-    if (RG.maxRegionRows > region_fuse_limit()) { reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S); return; }
-    const int variant = region_variant(RG);
-    if (variant == 1) launch_region<128, 8, 2>(st, g, RG, wRows, scale, S);
-    else if (variant == 2) launch_region<64, 8, 4>(st, g, RG, wRows, scale, S);
-    else if (variant == 3) launch_region<32, 0, 10>(st, g, RG, wRows, scale, S);
-    else if (variant == 4) launch_region<128, 0, 3>(st, g, RG, wRows, scale, S);
+    const int path = region_path(RG);
+    if (path == 2) { reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S); return; }
+    if (path == 1) launch_region<128, 8, 2>(st, g, RG, wRows, scale, S);
     else launch_region<64, 0, 6>(st, g, RG, wRows, scale, S);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
@@ -1288,7 +1077,7 @@ void reduced_finish(cudaStream_t, const Geom&, const RegionData& RG, const doubl
 void reduced_apply(cudaStream_t st, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
     reduced_moments(st, g, RG, wRows, S, true); reduced_expand(st, g, RG, wRows, scale, S);
 }
-int region_path(const OpArgs&, const RegionData& RG) { return RG.regHi > RG.regLo ? 2 : -1; }      // the twin has the chunked form only
+int region_path(const RegionData& RG) { return RG.regHi > RG.regLo ? 2 : -1; }      // the twin has the chunked form only
 void reduced_expand(cudaStream_t, const Geom& g, const RegionData& RG, double* wRows, double scale, const PcgScalars* S) {
     if (S && S->done) return;
     for (int ch = RG.rowChunkLo; ch < RG.rowChunkHi; ++ch) {

@@ -879,13 +879,6 @@ void Solver::constructMatrixBlocks() {
         }
         axisStart[(size_t)3 * R] = pos;
         RG.rowAxisStart.from_host(st, axisStart.data(), axisStart.size());
-        {   // one CTA per region: start the long ones first, so that the last wave is made of short CTAs
-            std::vector<int32_t> order((size_t)R);
-            for (int r = 0; r < R; ++r) order[r] = r;
-            auto rowsOf = [&](int32_t r) { return perRA[3 * r] + perRA[3 * r + 1] + perRA[3 * r + 2]; };
-            std::stable_sort(order.begin() + RG.regLo, order.begin() + RG.regHi, [&](int32_t a, int32_t b) { return rowsOf(a) > rowsOf(b); });
-            RG.regionOrder.from_host(st, order.data(), order.size());
-        }
         RG.rowStart.from_host(st, start.data(), start.size());
         RG.rowChunk.from_host(st, table.data(), table.size());
         RG.rowChunkStart.from_host(st, chunkStart.data(), chunkStart.size());
@@ -948,17 +941,14 @@ void Solver::closeVectorMaps() {
 #endif
 }
 // Collective (every setup with the peer transport on): one host all-reduce tells whether any rank's arena moved (first step, or a
-// larger system) and whether every rank can run the fused form; only then the arenas are published and mapped again.
+// larger system); only then the arenas are published and mapped again.
 void Solver::exchangeVectorPointers() {
     fusedHalo = false;
 #ifndef PS_EMULATE
     if (!peer.on || !comm || !part.multi()) return;
     PS_WHERE("exchangeVectorPointers");
-    static const bool env = !(getenv("PS_HALO_FUSED") && atoi(getenv("PS_HALO_FUSED")) == 0);
-    const bool okHere = env;
     const bool moved = (void*)vecArena.p != peer.vecPublished;
-    const double code = hostAllreduceSum((moved ? 1. : 0.) + (okHere ? 0. : 1024.));
-    const bool anyMoved = std::fmod(code, 1024.) > 0.5, allOk = code < 1023.5;
+    const bool anyMoved = hostAllreduceSum(moved ? 1. : 0.) > 0.5;
     if (anyMoved) {
         stream_sync(st);
         closeVectorMaps();
@@ -987,7 +977,7 @@ void Solver::exchangeVectorPointers() {
         peer.vecReady = hostAllreduceSum(ok ? 0. : 1.) < 0.5;        // also the barrier: every neighbour has closed its mapping of the previous arena
         if (arenaGraveyard) { dev_free(arenaGraveyard); arenaGraveyard = nullptr; }
     }
-    fusedHalo = peer.vecReady && allOk;
+    fusedHalo = peer.vecReady;
 #endif
 }
 
@@ -1046,11 +1036,6 @@ void Solver::buildSchedules() {
     const std::vector<int32_t> a = merge_schedule(sr1), b = merge_schedule(sr2);
     nSched1 = (int)a.size(); nSched2 = (int)b.size();
     sched1.from_host(st, a.data(), a.size()); sched2.from_host(st, b.data(), b.size());
-    // the same order split into the coupled reduced rows (range 3) and the active rows: the reduced term only needs the former
-    std::vector<int32_t> a1, b1;
-    for (int32_t e : a) (((uint32_t)e >> 28) == 3u ? a1 : b1).push_back(e);
-    nSched1a = (int)a1.size(); nSched1b = (int)b1.size();
-    sched1a.from_host(st, a1.data(), a1.size() + 0); sched1b.from_host(st, b1.data(), b1.size() + 0);
     stream_sync(st);    // the vectors die here
 }
 void Solver::computeOwnership() {
@@ -1128,13 +1113,8 @@ void Solver::exchange(Halo& H, double* v, const PcgScalars* S) {
             dst[i] = peer.recv(pr, kind, par, 1 - i); dflag[i] = &peer.sync(pr)->haloFlag[kind][par][1 - i];
             src[i] = peer.recv(part.rank, kind, par, i); sflag[i] = &peer.sync(part.rank)->haloFlag[kind][par][i];
         }
-        static const bool split = getenv("PS_HALO_SPLIT") && atoi(getenv("PS_HALO_SPLIT"));      // the two-launch form, kept for A/B timing
-        if (split) {
-            k_halo_push_peer(st, H.nSend[0], H.nSend[1], H.sendIdx.p, v, dst[0], dst[1], dflag[0], dflag[1], seq, scal.p, S != nullptr, &scal.p->ticket[4 + kind]);
-            k_halo_unpack_peer(st, H.nRecv[0], H.nRecv[1], H.recvIdx.p, src[0], src[1], sflag[0], sflag[1], seq, v, scal.p, S != nullptr);
-        } else
-            k_halo_exchange_peer(st, H.nSend[0], H.nSend[1], H.sendIdx.p, dst[0], dst[1], dflag[0], dflag[1], H.nRecv[0], H.nRecv[1], H.recvIdx.p, src[0], src[1], sflag[0], sflag[1],
-                                 seq, v, scal.p, S != nullptr, &scal.p->ticket[4 + kind]);
+        k_halo_exchange_peer(st, H.nSend[0], H.nSend[1], H.sendIdx.p, dst[0], dst[1], dflag[0], dflag[1], H.nRecv[0], H.nRecv[1], H.recvIdx.p, src[0], src[1], sflag[0], sflag[1],
+                             seq, v, scal.p, S != nullptr, &scal.p->ticket[4 + kind]);
         return;
     }
 #endif
@@ -1179,21 +1159,14 @@ static OpArgs make_op(const Solver& S) {
     A.uInv = S.uInv.p; A.valScale = S.g.invDx / 64.;
     A.rowsK = S.ownK; A.rowsP = S.ownP; A.rowsE = S.ownE;
     A.s1 = S.sr1; A.s2 = S.sr2; A.sched1 = S.sched1.p; A.sched2 = S.sched2.p; A.nSched1 = S.nSched1; A.nSched2 = S.nSched2;
-    A.sched1a = S.sched1a.p; A.sched1b = S.sched1b.p; A.nSched1a = S.nSched1a; A.nSched1b = S.nSched1b;
     return A;
 }
 OpArgs Solver::make_op_args() const { return make_op(*this); }
 
 // pass 1 of an operator apply including the reduced term: w = [dt Mc^-1 K x ; c_f . B^-1 J x]
-void Solver::pass1Apply(const OpArgs& A, const double* xin, const PcgScalars* S, bool reverse, const VecLink& V, bool withShared) {
-#ifndef PS_EMULATE
-    if (RG.count > 0 && !reverse && k_pass1_regions(st, A, xin, w.p, g.dt, S, g, RG, 1.0, V)) {}      // active rows and regions in one launch
-    else
-#endif
-    {
-        k_pass1(st, A, xin, w.p, g.dt, S, reverse, 0, V);       // V: wait for the neighbours' entries of x at the head (direct halo stores)
-        if (RG.count > 0) reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, S);          // moments -> B^-1 -> expand, one CTA per region
-    }
+void Solver::pass1Apply(const OpArgs& A, const double* xin, const PcgScalars* S, const VecLink& V, bool withShared) {
+    k_pass1(st, A, xin, w.p, g.dt, S, V);       // V: wait for the neighbours' entries of x at the head (direct halo stores)
+    if (RG.count > 0) reduced_apply(st, g, RG, w.p + C.nActiveVs, 1.0, S);          // moments -> B^-1 -> expand, one CTA per region
     if (withShared) sharedApply(w.p + C.nActiveVs, nullptr, 0.0, 1.0, 1.0, nullptr, S);
 }
 
@@ -1297,14 +1270,7 @@ int Solver::solve() {
     allreduce(scal.p->red + 3, 3);
     k_cg_begin(st, scal.p, reduceCtx(1, -1));
     bool cancelled = false;
-    // PS_DBG_SKIP (timing experiments only, the iterates are WRONG with it): bit 0 drops the halo exchanges, bit 1 the
-    // cross-rank reductions of the CG loop -- what is left is each rank iterating on its own slab (profiles/r01_dist_probe*.log)
-    const int dbgSkip = getenv("PS_DBG_SKIP") ? atoi(getenv("PS_DBG_SKIP")) : 0;
-    static const bool zigzag = getenv("PS_ZIGZAG") && atoi(getenv("PS_ZIGZAG")) != 0;      // A/B knob; off: measured 2 % slower on B200 (profiles/r02_probe_s3_256_v2*.log)
-    auto rctx = [&](int slotIn, int slotOut, int slotIn2 = -1) { return (dbgSkip & 2) ? PeerCtx() : reduceCtx(slotIn, slotOut, slotIn2); };
-    auto xchg = [&](Halo& H, double* v) { if (!(dbgSkip & 1)) exchange(H, v, scal.p); };
-    auto ared = [&](double* buf, int cnt) { if (!(dbgSkip & 2)) allreduce(buf, cnt); };
-    const bool fused = fusedHalo && peer.on && !dbgSkip && !zigzag;
+    const bool fused = fusedHalo && peer.on;
 #ifndef PS_EMULATE
     auto myFlag = [&](int kind, int side) -> const unsigned long long* {
         const int pr = side == 0 ? part.rank - 1 : part.rank + 1;
@@ -1327,31 +1293,26 @@ int Solver::solve() {
         for (int k = 0; k < batch; ++k) {
             const bool tr = (it + k == traceIter);
             mark(tr, "start");
-            // The three sweeps of an iteration alternate direction, and so do consecutive iterations: each kernel starts on the end of
-            // the vector its predecessor wrote last (w, Ap, p: 80 - 130 MB each, the L2 holds 126 MB), instead of on the part that
-            // has been evicted.  Results do not depend on the direction (every row is computed the same way; the dot products are
-            // summed per CTA, then over the CTAs in index order).
-            const bool rev = zigzag && ((it + k) & 1);
             // halos: with the peer transport the boundary entries are stored straight into the neighbours' vectors by a short push launch
             // and the consuming kernel waits at its head (VecLink); only the very first p of a solve goes by the exchange kernel
             VecLink l1, l2;
             if (fused) {
                 if (it + k > 0) { l1.wait[0] = myFlag(0, 0); l1.wait[1] = myFlag(0, 1); l1.waitSeq = peer.seqVec[0]; }
-                else xchg(haloX, p.p);
-            } else xchg(haloX, p.p);
+                else exchange(haloX, p.p, scal.p);
+            } else exchange(haloX, p.p, scal.p);
             mark(tr, "halo p");
-            pass1Apply(A, p.p, scal.p, rev, l1, false);         mark(tr, "pass1 + regions");          // w = [dt Mc^-1 K p ; c_f . B^-1 J p]
+            pass1Apply(A, p.p, scal.p, l1, false);              mark(tr, "pass1 + regions");          // w = [dt Mc^-1 K p ; c_f . B^-1 J p]
             if (RG.nShared > 0) { sharedApply(w.p + C.nActiveVs, nullptr, 0.0, 1.0, 1.0, nullptr, scal.p); mark(tr, "shared regions"); }
             if (fused) { l2 = pushDirect(haloW, 1, nullptr); l2.wait[0] = myFlag(1, 0); l2.wait[1] = myFlag(1, 1); l2.waitSeq = peer.seqVec[1]; }
-            else xchg(haloW, w.p);
+            else exchange(haloW, w.p, scal.p);
             mark(tr, "halo w");
-            k_pass2(st, A, w.p, p.p, Ap.p, 0.5, nullptr, dotPartial.p, rctx(-1, 0), scal.p, 3, r.p, zigzag && !rev, l2);   // + this rank's p.Ap, r.Ap, Ap.Ap to every rank
-            ared(scal.p->red, 3);                               mark(tr, "pass2 (+allreduce)");
-            const PeerCtx uc = rctx(0, 1, 1);                   // global p.Ap.. and the previous r.r, x.p, p.p in; new r.r, x.p, p.p out
+            k_pass2(st, A, w.p, p.p, Ap.p, 0.5, nullptr, dotPartial.p, reduceCtx(-1, 0), scal.p, 3, r.p, l2);   // + this rank's p.Ap, r.Ap, Ap.Ap to every rank
+            allreduce(scal.p->red, 3);                          mark(tr, "pass2 (+allreduce)");
+            const PeerCtx uc = reduceCtx(0, 1, 1);              // global p.Ap.. and the previous r.r, x.p, p.p in; new r.r, x.p, p.p out
             VecLink l3;
             if (fused) l3 = pushDirect(haloX, 0, &uc);          // the boundary entries of the p this update is about to form, on their way while it runs
-            k_cg_update(st, ownSys, x.p, r.p, p.p, Ap.p, dotPartial.p, scal.p, uc, rev, l3);
-            ared(scal.p->red + 3, 3);                           mark(tr, "update x,r,p (+allreduce)");
+            k_cg_update(st, ownSys, x.p, r.p, p.p, Ap.p, dotPartial.p, scal.p, uc, l3);
+            allreduce(scal.p->red + 3, 3);                      mark(tr, "update x,r,p (+allreduce)");
         }
         it += batch;
         copy_d2h(&h, scal.p, sizeof h, st);

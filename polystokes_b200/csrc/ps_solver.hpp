@@ -82,7 +82,6 @@ struct RegionData {
     int32_t maxRegionRows = 0;   // largest number of coupled reduced rows of one region (decides fused vs chunked reduced kernels)
     int32_t maxRegionAxisRows = 0;                    // largest row count of one (region, face axis) built here (read-only count)
     int32_t maxRegionCells = 0, minRegionCells = 0;   // REDUCED cells of the largest / smallest owned region (read-only counts)
-    DBuf<int32_t> regionOrder;   // [R] launch order of reduced_region_kernel: the owned regions by decreasing row count (longest CTA first)
     DBuf<double> partial;    // per-chunk partial sums
     DBuf<double> t, s;       // [R][26] per-apply moment / B^-1 t
     DBuf<unsigned int> regionTicket;   // [R] chunks of the region that have delivered their moments (self-resetting)
@@ -252,7 +251,7 @@ public:
 
     // operator y = A x on device vectors (Apply.h:102-179)
     void applyOperator(const double* x, double* y, double* pApPartial);
-    void pass1Apply(const OpArgs& A, const double* x, const PcgScalars* S, bool reverse = false, const VecLink& V = VecLink(), bool withShared = true);   // pass 1 + the reduced term
+    void pass1Apply(const OpArgs& A, const double* x, const PcgScalars* S, const VecLink& V = VecLink(), bool withShared = true);   // pass 1 + the reduced term
     // the reduced term of the shared regions: s_r = B_r^-1 (extraScale extra_r + tScale t_r), t_r summed over the ranks (collective
     // when tScale != 0), then w_f = scale c_f . s_r on this rank's shared rows (scale 0: no expansion); sOut (region-indexed) receives s_r
     void sharedApply(double* wRows, const double* extra, double extraScale, double tScale, double scale, double* sOut, const PcgScalars* S);
@@ -274,8 +273,8 @@ public:
     // matrices + vectors
     CompactOp Op;                 // K_ext and K_ext^T
     SchedRanges sr1, sr2;         // block schedules of pass 1 / pass 2 over the owned rows (merge_schedule)
-    DBuf<int32_t> sched1, sched2, sched1a, sched1b;
-    int nSched1 = 0, nSched2 = 0, nSched1a = 0, nSched1b = 0;
+    DBuf<int32_t> sched1, sched2;
+    int nSched1 = 0, nSched2 = 0;
     void buildSchedules();
     DBuf<double> mcInv, mc, rhsU, oldVs, uInv, uDiag, rhsPT, b;
     DBuf<double> x, r, p, Ap, w, velSol;
@@ -346,29 +345,23 @@ struct OpArgs {   // everything one operator apply touches
     int64_t nRowsExt, nActiveVs, nP, nT, nC, nE;
     SchedRanges s1, s2;           // pass 1: face rows x, y, z, coupled reduced rows; pass 2: cells, edges yz, xz, xy (edge numbering)
     const int32_t* sched1; const int32_t* sched2; int nSched1, nSched2;
-    const int32_t* sched1a; const int32_t* sched1b; int nSched1a, nSched1b;   // pass 1 split: coupled reduced rows | active rows (same merged order)
     RowSet rowsK, rowsP, rowsE;   // rows this rank computes (all rows on one GPU); the centre-stress rows follow rowsP
     const uint64_t* kcode; const int32_t* kcol; const uint8_t* kmc; const double* mcInvLut;
     const uint64_t* ccode; const int32_t* ccol; const uint32_t* ecode; const int32_t* ecol;
     const double* uInv;
     double valScale;              // invDx / 64
 };
-void k_pass1(cudaStream_t, const OpArgs&, const double* x, double* w, double activeScale, const PcgScalars* scal, bool reverse = false, int part = 0, const VecLink& V = VecLink());
-#ifndef PS_EMULATE
-// pass 1 and the reduced term of one apply in two launches: coupled reduced rows, then active rows interleaved with the regions.
-// false: not applicable (no tiled regions of this rank / PS_OVERLAP=0) -- nothing was launched, use k_pass1 + reduced_apply
-bool k_pass1_regions(cudaStream_t, const OpArgs&, const double* x, double* w, double activeScale, const PcgScalars* scal, const Geom&, const RegionData&, double scale, const VecLink& V = VecLink());
-#endif
+void k_pass1(cudaStream_t, const OpArgs&, const double* x, double* w, double activeScale, const PcgScalars* scal, const VecLink& V = VecLink());
 // mode bit 0: dot(x, y) (p.Ap) -> red[0]; bit 1: also dot(r2, y), dot(y, y) (r.Ap, Ap.Ap) -> red[1], red[2]
 void k_pass2(cudaStream_t, const OpArgs&, const double* w, const double* x, double* y, double muScale, const double* add, double* dotPartial, const PeerCtx& P, PcgScalars* scal, int mode,
-             const double* r2 = nullptr, bool reverse = false, const VecLink& V = VecLink());
+             const double* r2 = nullptr, const VecLink& V = VecLink());
 // moments of w_f per chunk; with `solve` the last chunk of every region also runs reduced_finish(nullptr, 0, 1) for it (one launch less)
 void reduced_moments(cudaStream_t, const Geom&, const RegionData&, const double* wRows, const PcgScalars* scal, bool solve = false);
 void reduced_finish(cudaStream_t, const Geom&, const RegionData&, const double* extraRhs, double extraScale, double tScale, const PcgScalars* scal);
 void reduced_expand(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
 // the reduced term of one apply: w_f <- scale * c_f . B^-1 (sum_f c_f w_f); one fused launch for tiled regions, moments + expand otherwise
 void reduced_apply(cudaStream_t, const Geom&, const RegionData&, double* wRows, double scale, const PcgScalars* scal);
-int region_path(const OpArgs&, const RegionData&);      // the kernels reduced_apply / pass1Apply choose (ps_pcg.cu)
+int region_path(const RegionData&);      // the kernels reduced_apply chooses (ps_pcg.cu)
 // shared regions (RegionData::nShared): moments of this rank's shared rows per chunk, their sum per slot in chunk order (shMoments,
 // then summed over the ranks by the caller), the small solve of the slots this rank takes part in, the expansion onto its shared rows
 void shared_moments(cudaStream_t, const Geom&, const RegionData&, const double* wRows, const PcgScalars* scal);
@@ -380,7 +373,7 @@ void shared_expand(cudaStream_t, const Geom&, const RegionData&, double* wRows, 
 void shared_exchange_peer(cudaStream_t, const RegionData&, const SharedPeer& P, const double* extra, double extraScale, double tScale, double* sOut,
                           const PcgScalars* scal, PcgScalars* err);
 #endif
-void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, bool reverse = false, const VecLink& V = VecLink());
+void k_cg_update(cudaStream_t, const RangeSet& own, double* x, double* r, double* p, const double* Ap, double* dotPartial, PcgScalars* scal, const PeerCtx& P, const VecLink& V = VecLink());
 void k_cg_init(cudaStream_t, const RangeSet& own, const double* b, double* x, double* r, double* p, double* dotPartial, PcgScalars* scal, double tol, int maxIter, const PeerCtx& P);
 void k_cg_begin(cudaStream_t, PcgScalars* scal, const PeerCtx& P);
 // BiCGSTAB fallback (pcg.h:134-200).  Dot products land rank-local in scal->bred[], the host enqueues the all-reduce
@@ -403,15 +396,11 @@ void k_eig_first_p(cudaStream_t, const RangeSet& own, const double* diag, const 
 void k_eig_update_xr(cudaStream_t, const RangeSet& own, const double* diag, double* x, double* r, const double* p, const double* Ap, double* dotPartial, PcgScalars* scal);
 void k_eig_update_p(cudaStream_t, const RangeSet& own, const double* diag, double* p, const double* r, const PcgScalars* scal);
 #ifndef PS_EMULATE
-void k_halo_push_peer(cudaStream_t, int64_t n0, int64_t n1, const int32_t* idx, const double* v, double* dst0, double* dst1, unsigned long long* flag0, unsigned long long* flag1,
-                      unsigned long long seq, PcgScalars* S, bool respectDone, unsigned int* ticket);
 void k_halo_push_direct(cudaStream_t, int64_t n0, int64_t n1, const int32_t* idx, const double* v, double* dst0, double* dst1, const PcgScalars* S);
 void k_halo_push_p(cudaStream_t, int64_t n0, int64_t n1, const int32_t* idx, const double* r, const double* p, const double* Ap, double* dst0, double* dst1, PcgScalars* S, const PeerCtx& P);
 void k_halo_exchange_peer(cudaStream_t, int64_t ns0, int64_t ns1, const int32_t* sendIdx, double* dst0, double* dst1, unsigned long long* dflag0, unsigned long long* dflag1,
                           int64_t nr0, int64_t nr1, const int32_t* recvIdx, const double* src0, const double* src1, const unsigned long long* sflag0, const unsigned long long* sflag1,
                           unsigned long long seq, double* v, PcgScalars* S, bool respectDone, unsigned int* ticket);
-void k_halo_unpack_peer(cudaStream_t, int64_t n0, int64_t n1, const int32_t* idx, const double* src0, const double* src1, const unsigned long long* flag0, const unsigned long long* flag1,
-                        unsigned long long seq, double* v, PcgScalars* S, bool respectDone);
 #endif
 void k_recover_active(cudaStream_t, const Geom&, const RowSet& rows, const double* wAct, const double* mcInv, const double* rhsU, double* velSol);
 // faces this rank writes: active faces with index in [aLo, aHi), reduced faces of regions [regLo, regHi), every face without a DOF;

@@ -1,5 +1,5 @@
 """Per-iteration timing of the slab-decomposed CG under torchrun (one process per GPU): cg_iteration / pass1 / pass2 /
-apply on this rank's slab of S3.  Run once per setting of PS_COMM / PS_DBG_SKIP / ... (the library reads them once)."""
+apply on this rank's slab of S3.  Run once per setting of PS_COMM (the library reads it once)."""
 import argparse, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -30,7 +30,7 @@ t = torch.tensor([res[k] for k in res], device="cuda", dtype=torch.float64)
 if world > 1:
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
 if rank == 0:
-    env = {k: os.environ.get(k) for k in ("PS_COMM", "PS_DBG_SKIP", "PS_PDL", "PS_HALO_SPLIT") if os.environ.get(k)}
+    env = {k: os.environ.get(k) for k in ("PS_COMM",) if os.environ.get(k)}
     print(f"[dist_probe {a.tag}] world={world} peer={s.count('peerTransport')} env={env} max over ranks, us: " +
           "  ".join(f"{k} {float(v)*1e3:.1f}" for k, v in zip(res, t.tolist())), flush=True)
 if world > 1:

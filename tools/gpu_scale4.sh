@@ -11,5 +11,4 @@ tail -3 gpurun_out/bench_err_n4.log
 N=4
 run() { timeout -k 10 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port $((29530 + RANDOM % 100)) tools/dist_probe.py --tag "$1" 2>&1 | grep "dist_probe" | tee -a gpurun_out/dist_probe_n$N.log; }
 run full
-PS_DBG_SKIP=3 run no_halo_no_reduce
 PS_COMM=nccl run nccl

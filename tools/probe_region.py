@@ -1,4 +1,4 @@
-"""A/B probe of the reduced term on the GPU box: one setup of S3, then the region kernel alone, pass 1 + regions and a CG iteration."""
+"""Probe of the reduced term on the GPU box: one setup of S3, then the region kernel alone, pass 1 + regions and a CG iteration."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -8,5 +8,5 @@ sc = scenes.scene_s3(n)
 d = lambda x: torch.from_numpy(np.ascontiguousarray(x)).cuda()
 s = PolyStokesSolver.from_scene(sc)
 s.setup(d(sc.surface), d(sc.collision), d(sc.viscosity), [d(v) for v in sc.vel], [d(v) for v in sc.colvel])
-tag = f"LPT={os.environ.get('PS_REGION_LPT', '0')} VARIANT={os.environ.get('PS_REGION_VARIANT', '-')}"
+tag = f"regionPath={s.count('regionPath')}"
 print(tag, " ".join(f"{k} {s.time_kernel(k, 40) * 1e3:.1f} us" for k in ("reduced", "pass1", "cg_iteration")), flush=True)

@@ -1,11 +1,10 @@
-# round 2, 2 GPUs: single-GPU probe (region kernel variants, vectorised update), distributed parity (slab-local + replicated, peer + nccl),
+# round 2, 2 GPUs: single-GPU probe (vectorised update), distributed parity (slab-local + replicated, peer + nccl),
 # the ps_create_multi handle, bench at N = 2 (process per GPU) and through the multi handle
 set -x
 cd $GRAFT_REPO_ROOT
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=index,name --format=csv
 CUDA_VISIBLE_DEVICES=0 timeout -k 10 600 python tools/probe.py --scene S3 --n 256 --steps 2 2>&1 | tail -12 | tee gpurun_out/r02_probe_s3_256_v5.log
-for v in 0 1 2 4; do PS_REGION_VARIANT=$v CUDA_VISIBLE_DEVICES=0 timeout -k 10 600 python tools/probe.py --scene S3 --n 256 --steps 1 --reps 30 2>&1 | grep -E "^reduced|^cg_iteration" | sed "s/^/variant $v: /" | tee -a gpurun_out/r02_sweep_region_v5.log; done
 timeout -k 10 1500 python -m pytest tests/test_gpu_distributed.py tests/test_gpu_multi.py -q -x -m gpu 2>&1 | tail -12 | tee gpurun_out/r02_pytest_gpu_dist_n2_v5.log
 timeout -k 10 900 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 bench.py --gpus 2 --steps 10 --warmup 3 2> gpurun_out/r02_bench_err_n2_v5.log | tee gpurun_out/r02_bench_n2_v5.json
 tail -3 gpurun_out/r02_bench_err_n2_v5.log
