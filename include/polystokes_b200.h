@@ -144,7 +144,9 @@ const char* ps_last_error(void);
  * tilePadding 0) are solved with a cross-rank reduction: each rank forms the moments of the region's rows in its slab, one
  * all-reduce per operator apply sums them, and every rank solves the region's small system; the setup stays replicated for
  * these configurations (ps_get_count "sharedRegions" counts such regions).  ps_set_params may switch doTile between steps: the
- * cuts follow (multiples of 16 without tiles, of lcm(16, tileSize) with them).
+ * cuts follow (multiples of 16 without tiles, of lcm(16, tileSize) with them).  The cuts are even in layers unless the caller sets
+ * them (ps_set_partition, ps_rebalance); caller-set cuts are kept by ps_set_params while they remain multiples of the unit, and
+ * replaced by the even cuts when a new tileSize makes them illegal.
  * cancel_cb must answer identically on all ranks. */
 /* ---- several GPUs behind ONE handle (SURVEY.md section 8b; the caller is one cook thread, exec/HDK_PolyStokes.C:222-345) ----
  * ps_create_multi builds the same slab decomposition inside one process: one rank per device devs[0..ndev) (NULL: devices
@@ -159,6 +161,19 @@ int ps_comm_unique_id(void* id128);
 int ps_comm_init(ps_handle h, int rank, int nranks, const void* id128);
 /* z cuts of all ranks: zCut[nranks+1] (may be NULL); returns nranks, this rank's slab in *zLo, *zHi */
 int ps_get_partition(ps_handle h, int32_t* rank, int32_t* zLo, int32_t* zHi, int32_t* zCut);
+/* Collective on a decomposed handle.  zCut[nranks+1]: 0 = zCut[0] < ... < zCut[nranks] = nz, interior cuts multiples of the unit
+ * (lcm(16, tileSize) layers with tiles, 16 without); NULL = the even cuts.  PS_INVALID (the same on every rank, agreed by one
+ * all-reduce) for cuts that break a rule or differ between ranks; the handle keeps its cuts then.  Takes effect at the next ps_setup /
+ * ps_step.  On one GPU only NULL and {0, nz} are accepted (and change nothing). */
+int ps_set_partition(ps_handle h, const int32_t* zCut);
+/* Collective; needs a prior setup.  Every setup measures the work of each z-unit: the algorithmic bytes of one CG iteration
+ * (ps_kernel_bytes "cg_iteration") of the rows the unit holds -- ps_get_vector "unitLoad", the same on every rank and independent of
+ * the cuts; "unitCounts" is the table behind it, [unit][9]: active voxels of the 7 sample slots, coupled reduced rows (by the z of
+ * their face), regions (by the z of their first cell).  ps_rebalance takes the cuts that minimise the largest slab's load (the
+ * lexicographically smallest such cuts, every slab at least one unit) and applies them only if they lower that maximum:
+ * PS_SUCCESS (applied; effective at the next ps_setup / ps_step), PS_NOCHANGE (kept; always on one GPU), PS_INVALID (no setup yet,
+ * or the tiling changed since).  zCut (may be NULL) receives the cuts the handle holds afterwards. */
+int ps_rebalance(ps_handle h, int32_t* zCut);
 
 /* ---- introspection for parity tests (read-only views of the solver state, copied to HOST memory) ---- */
 /* counters by name: nCenter nFaceX nFaceY nFaceZ nEdgeYZ nEdgeXZ nEdgeXY nActiveVs nReducedVs nPressures
@@ -176,7 +191,7 @@ int64_t ps_get_weight_field(ps_handle h, int liquid, int slot, float* out);
  * blocks are dense, so it only fits for small / medium grids -- PS_FAILED beyond 2^31-1 entries or device memory). */
 int ps_get_csr(ps_handle h, const char* name, int64_t* rows, int64_t* cols, int64_t* nnz, int64_t* rowptr, int32_t* colidx, double* vals);
 /* dense vectors by name (activeRHS reducedRHS pressureRHS stressRHS b guess diagA solution velSolution com bestFit
- * MrDense ViscDense BinvDense); returns the length.  diagA = diag(A) formed from the factors (one GPU).  On a rank of a job with one
+ * MrDense ViscDense BinvDense unitLoad unitCounts); returns the length.  diagA = diag(A) formed from the factors (one GPU).  On a rank of a job with one
  * process per GPU, b / solution / guess / region data are zero outside the calling rank's share, so the sum over ranks is the global
  * vector; a ps_create_multi handle returns the global vector. */
 int64_t ps_get_vector(ps_handle h, const char* name, double* out);

@@ -56,7 +56,8 @@ class ps_stats(C.Structure):
 # every symbol include/polystokes_b200.h declares
 SYMBOLS = ["ps_create", "ps_destroy", "ps_step", "ps_setup", "ps_solve", "ps_export", "ps_last_error", "ps_get_count", "ps_get_real",
            "ps_get_index_field", "ps_get_weight_field", "ps_get_csr", "ps_get_vector", "ps_apply", "ps_time_kernel", "ps_kernel_bytes", "ps_timer",
-           "ps_comm_unique_id", "ps_comm_init", "ps_get_partition", "ps_create_multi", "ps_set_params", "ps_alloc_pinned", "ps_free_pinned"]
+           "ps_comm_unique_id", "ps_comm_init", "ps_get_partition", "ps_create_multi", "ps_set_params", "ps_alloc_pinned", "ps_free_pinned",
+           "ps_set_partition", "ps_rebalance"]
 
 _cache = {}
 
@@ -95,5 +96,7 @@ def load(path=None):
     L.ps_comm_unique_id.argtypes = [C.c_void_p]; L.ps_comm_unique_id.restype = C.c_int
     L.ps_comm_init.argtypes = [H, C.c_int, C.c_int, C.c_void_p]; L.ps_comm_init.restype = C.c_int
     L.ps_get_partition.argtypes = [H] + [C.POINTER(C.c_int32)] * 4; L.ps_get_partition.restype = C.c_int
+    L.ps_set_partition.argtypes = [H, C.c_void_p]; L.ps_set_partition.restype = C.c_int
+    L.ps_rebalance.argtypes = [H, C.c_void_p]; L.ps_rebalance.restype = C.c_int
     _cache[path] = L
     return L

@@ -394,6 +394,9 @@ std::vector<double> view(Solver& S, Piece&& p, bool global) {
 }
 
 bool get_vector(Solver& S, const std::string& n, std::vector<double>& out, bool global) {
+    // replicated on every rank: the same answer from any rank, no collective
+    if (n == "unitLoad") { out = S.unitLoad; return true; }
+    if (n == "unitCounts") { out.assign(S.unitCounts.begin(), S.unitCounts.end()); return true; }
     if (n == "diagA") { if (S.part.multi()) return false; S.computeDiagonal(); out = S.diagA.to_host(S.st, (size_t)S.C.nSystemSize); return true; }
     if (n == "guess" && global && S.part.multi()) S.constructGuessVectors();      // several ranks: formed where it is read (collective)
     Piece p;
@@ -576,6 +579,17 @@ int ps_get_partition(ps_handle h, int32_t* rank, int32_t* zLo, int32_t* zHi, int
     if (zHi) *zHi = p.zCut[p.rank + 1];
     if (zCut) for (int k = 0; k <= p.nranks; ++k) zCut[k] = p.zCut[k];
     return p.nranks;
+}
+
+int ps_set_partition(ps_handle h, const int32_t* zCut) {
+    if (!h) { g_lastError = "ps_set_partition: null handle"; return PS_INVALID; }
+    if (h->multi) { MultiGroup* G = h->multi; return G->run([&](int k) { return ps_set_partition(G->kids[(size_t)k], zCut); }); }
+    return guarded(h, [&] { return h->S->setPartition(zCut); });
+}
+int ps_rebalance(ps_handle h, int32_t* zCut) {
+    if (!h) { g_lastError = "ps_rebalance: null handle"; return PS_INVALID; }
+    if (h->multi) { MultiGroup* G = h->multi; return G->run([&](int k) { return ps_rebalance(G->kids[(size_t)k], k == 0 ? zCut : nullptr); }); }
+    return guarded(h, [&] { return h->S->rebalance(zCut); });
 }
 
 int ps_set_params(ps_handle h, const ps_params* params) {
@@ -762,33 +776,21 @@ int ps_apply(ps_handle h, const double* x, double* y) {
 double ps_kernel_bytes(ps_handle h, const char* name) {
     if (!h || !name) return 0;
     const Solver& S = *h->S; const Counts& C = S.C; const std::string nm(name);
-    // DESIGN.md section 5.  Compact operator: 8 B of codes + 6 x 4 B columns per face row (+ 1 B mass code on active rows),
-    // 8 + 24 B per cell (serves the pressure row and the 3 centre-stress rows), 4 + 16 B per edge; every vector is read /
-    // written once.  "csr_*" = the same passes priced as the CSR SpMV of SURVEY.md 8d (12 B per stored non-zero).
-    const double nE = (double)(C.nEdge[0] + C.nEdge[1] + C.nEdge[2]);
-    const double n = (double)C.nSystemSize;
-    const double nRed = (double)S.RG.nRows;
-    // pass 1 = the sweep over the compact rows of K_ext (x once, w once) + the region kernel (below)
-    const double pass1Sweep = 32.0 * C.nRowsExt + 1.0 * C.nActiveVs /*matrix*/ + 8.0 * n /*x*/ + 8.0 * C.nRowsExt /*w write*/;
-    const double pass2 = 32.0 * C.nCenter + 20.0 * nE /*matrix*/ + 8.0 * C.nRowsExt /*w read*/ + 8.0 * (C.nCenter + nE) /*mu^-1: once per cell / edge*/
-                       + 8.0 * n /*x (stress part: the mu term; pressure part: the fused dot)*/ + 8.0 * n /*y*/;
-    const double pass2Dots = pass2 + 8.0 * n /*r for the fused r.Ap*/;
-    const double csrPass1 = 12.0 * 8.0 * C.nRowsExt + 8.0 * n + 8.0 * C.nActiveVs + 8.0 * C.nRowsExt;
-    const double csrPass2 = 12.0 * (6.0 * C.nPressures + 2.0 * 3 * C.nCenter + 4.0 * nE) + 8.0 * C.nRowsExt + 8.0 * C.nStresses + 8.0 * C.nStresses + 8.0 * n;
-    if (nm == "csr_pass1") return csrPass1;
-    if (nm == "csr_pass2") return csrPass2;
-    if (nm == "csr_apply") return csrPass1 + csrPass2 + nRed * 24.0 + (double)S.RG.count * (RDOF * RDOF + 2 * RDOF + 30) * 8.0;
-    // reduced rows: w read + packed coordinates (moments), packed coordinates + w write (expand), B^-1 + t,s,sigma per region
-    const double reduced = nRed * (8.0 + 4.0) + nRed * (4.0 + 8.0) + (double)S.RG.count * (RDOF * RDOF + 2 * RDOF + 30) * 8.0;
-    const double pass1 = pass1Sweep + reduced;
-    if (nm == "pass1") return pass1;
-    if (nm == "pass1_sweep") return pass1Sweep;
-    if (nm == "pass2") return pass2;
-    if (nm == "pass2_dots") return pass2Dots;
-    if (nm == "reduced") return reduced;
-    if (nm == "apply") return pass1 + pass2;
-    if (nm == "cg_update") return 56.0 * n;
-    if (nm == "cg_iteration") return pass1 + pass2Dots + 56.0 * n /*x, r, p update: x, r, p, Ap in; x, r, p out*/;
+    // DESIGN.md section 5; the byte model itself is OpBytes (ps_solver.hpp), also behind the unit loads of ps_rebalance
+    OpCounts c;
+    c.nCenter = C.nCenter; c.nActiveVs = C.nActiveVs; c.nEdges = C.nEdge[0] + C.nEdge[1] + C.nEdge[2]; c.nRedRows = S.RG.nRows; c.nRegions = S.RG.count;
+    const OpBytes b(c);
+    if (nm == "csr_pass1") return b.csrPass1;
+    if (nm == "csr_pass2") return b.csrPass2;
+    if (nm == "csr_apply") return b.csrApply;
+    if (nm == "pass1") return b.pass1;
+    if (nm == "pass1_sweep") return b.pass1Sweep;
+    if (nm == "pass2") return b.pass2;
+    if (nm == "pass2_dots") return b.pass2Dots;
+    if (nm == "reduced") return b.reduced;
+    if (nm == "apply") return b.pass1 + b.pass2;
+    if (nm == "cg_update") return b.cgUpdate;
+    if (nm == "cg_iteration") return b.cgIteration;
     return 0;
 }
 

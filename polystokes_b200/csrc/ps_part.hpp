@@ -8,6 +8,7 @@
 // single-GPU result -- while the per-region Gram builds, the operator rows and all CG vector work are
 // restricted to the owned ranges.  Per CG iteration: one halo exchange of p, one of w, two scalar all-reduces.
 #pragma once
+#include <limits>
 #include "ps_grid.hpp"
 
 namespace ps {
@@ -84,5 +85,46 @@ struct Partition {
     // every operator apply sums its moments over the ranks (Solver::sharedApply).
     bool spanning = false;
 };
+
+// Cuts: 0 = zCut[0] < ... < zCut[nranks] = nz, the interior ones multiples of the unit lcm(16, tileSize) (16 without tiles).
+inline bool valid_cuts(const std::vector<int>& zCut, int nranks, int nz, int unit) {
+    if ((int)zCut.size() != nranks + 1 || zCut[0] != 0 || zCut[nranks] != nz) return false;
+    for (int k = 0; k < nranks; ++k) if (zCut[k + 1] <= zCut[k] || (k > 0 && zCut[k] % unit != 0)) return false;
+    return true;
+}
+// largest slab load of cuts given in units (cut[k] = first unit of slab k, cut[nranks] = number of units)
+inline double max_slab_load(const std::vector<double>& load, const std::vector<int>& cut) {
+    double worst = 0.;
+    for (size_t k = 0; k + 1 < cut.size(); ++k) {
+        double s = 0.;
+        for (int u = cut[k]; u < cut[k + 1]; ++u) s += load[(size_t)u];
+        worst = std::max(worst, s);
+    }
+    return worst;
+}
+// Work-balanced cuts, in units: among the cut vectors that give every slab at least one unit, those that minimise the largest slab
+// load, and among those the lexicographically smallest.  A DP gives the least achievable maximum of every suffix split; the cuts are
+// then taken greedily, each as low as the rest still allows.  The loads are integers below 2^53, so every sum and comparison is exact.
+inline std::vector<int> balanced_cuts(const std::vector<double>& load, int nranks) {
+    const int n = (int)load.size();
+    std::vector<double> pre((size_t)n + 1, 0.);
+    for (int u = 0; u < n; ++u) pre[u + 1] = pre[u] + load[(size_t)u];
+    const double inf = std::numeric_limits<double>::infinity();
+    // best[k][i]: least largest load when units [i, n) are split into k non-empty slabs
+    std::vector<std::vector<double>> best((size_t)nranks + 1, std::vector<double>((size_t)n + 1, inf));
+    for (int i = 0; i < n; ++i) best[1][i] = pre[n] - pre[i];
+    for (int k = 2; k <= nranks; ++k)
+        for (int i = 0; i + k <= n; ++i)
+            for (int j = i + 1; j + k - 1 <= n; ++j) best[k][i] = std::min(best[k][i], std::max(pre[j] - pre[i], best[k - 1][j]));
+    const double target = best[nranks][0];
+    std::vector<int> cut((size_t)nranks + 1, 0);
+    cut[nranks] = n;
+    for (int k = 1; k < nranks; ++k) {
+        int j = cut[k - 1] + 1;
+        while (pre[j] - pre[cut[k - 1]] > target || best[nranks - k][j] > target) ++j;
+        cut[k] = j;
+    }
+    return cut;
+}
 
 }  // namespace ps

@@ -139,7 +139,7 @@ int64_t tile_order_scan(cudaStream_t st, const Geom& g, int slot, const uint8_t*
         cuts->assign((size_t)nc, 0);
         for (int k = 0; k < nc; ++k) {
             const int z = (*zCut)[k];
-            const int64_t tile = (int64_t)(z >> 4) * t.tx * t.ty;
+            const int64_t tile = (int64_t)std::max(0, (z >> 4) - tzA) * t.tx * t.ty;
             (*cuts)[k] = (k == nc - 1 || tile >= nTiles) ? off[nTiles] : off[tile];
         }
         (*cuts)[0] = 0;
@@ -148,6 +148,41 @@ int64_t tile_order_scan(cudaStream_t st, const Geom& g, int slot, const uint8_t*
     int32_t total = 0;
     copy_d2h(&total, tileCounts.p + nTiles, sizeof(int32_t), st);
     return total;
+}
+
+// Per-CTA histogram in shared memory: the lanes of a warp that hit the same bin add once (rows of one region share their z), and every CTA
+// adds its bins to the global counters once.
+__global__ void __launch_bounds__(256) unit_counts_kernel(Geom g, int unit, int nUnits, const uint32_t* __restrict__ rowXYZ, int64_t rLo, int64_t nRows,
+                                                          const int32_t* __restrict__ cellList, const int32_t* __restrict__ cellStart, int32_t regLo,
+                                                          int64_t n, int* counts) {
+    __shared__ int h[2 * MAX_UNITS];
+    for (int i = threadIdx.x; i < 2 * nUnits; i += blockDim.x) h[i] = 0;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    for (int64_t base = (int64_t)blockIdx.x * blockDim.x; base < n; base += (int64_t)gridDim.x * blockDim.x) {      // uniform per warp
+        const int64_t i = base + threadIdx.x;
+        int bin = -1;
+        if (i < nRows) bin = 2 * min((int)((rowXYZ[rLo + i] >> 20) & 1023u) / unit, nUnits - 1);
+        else if (i < n) {
+            const int32_t r = regLo + (int32_t)(i - nRows);
+            if (cellStart[r + 1] > cellStart[r]) bin = 2 * min(delin(g, SL_CENTER, cellList[cellStart[r]]).z / unit, nUnits - 1) + 1;
+        }
+        const unsigned same = __match_any_sync(0xffffffffu, bin);
+        if (bin >= 0 && lane == __ffs(same) - 1) atomicAdd(&h[bin], __popc(same));
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < 2 * nUnits; i += blockDim.x) if (h[i]) atomicAdd(&counts[i], h[i]);
+}
+
+void k_unit_counts(cudaStream_t st, const Geom& g, int unit, int nUnits, const uint32_t* rowXYZ, int64_t rLo, int64_t rHi,
+                   const int32_t* cellList, const int32_t* cellStart, int32_t regLo, int32_t regHi, int* counts) {
+    if (nUnits > MAX_UNITS) throw Error("k_unit_counts: more z-units than MAX_UNITS");
+    const int64_t n = (rHi - rLo) + (regHi - regLo);
+    if (n <= 0) return;
+    const int64_t blocks = std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 4);
+    unit_counts_kernel<<<(unsigned)blocks, 256, 0, st>>>(g, unit, nUnits, rowXYZ, rLo, rHi - rLo, cellList, cellStart, regLo, n, counts);
+    PS_COUNT_LAUNCH(1);
+    PS_CUDA(cudaGetLastError());
 }
 
 // ascending list of the indices i < n with flag[i] != 0, written to out[outOffset...]; returns the count
@@ -213,8 +248,8 @@ int64_t tile_order_scan(cudaStream_t, const Geom& g, int slot, const uint8_t* fl
                         const std::vector<int>* zCut, std::vector<int64_t>* cuts, const int* tileZ) {
     const int rx = g.r[slot][0], ry = g.r[slot][1], rz = g.r[slot][2];
     int32_t n = 0;
-    if (zCut && cuts) cuts->assign(zCut->size(), -1);
     const int zA = tileZ ? std::max(0, tileZ[0] * 16) : 0, zB = tileZ ? std::min(rz, tileZ[1] * 16) : rz;
+    if (zCut && cuts) { cuts->assign(zCut->size(), -1); for (size_t k = 0; k < zCut->size(); ++k) if ((*zCut)[k] < zA) (*cuts)[k] = 0; }
     for (int tk = zA; tk < zB; tk += 16) for (int tj = 0; tj < ry; tj += 16) for (int ti = 0; ti < rx; ti += 16) {
         if (zCut && cuts && tj == 0 && ti == 0) for (size_t k = 0; k < zCut->size(); ++k) if ((*zCut)[k] == tk) (*cuts)[k] = n;
         for (int k = tk; k < std::min(tk + 16, rz); ++k) for (int j = tj; j < std::min(tj + 16, ry); ++j) for (int i = ti; i < std::min(ti + 16, rx); ++i) {
@@ -224,6 +259,14 @@ int64_t tile_order_scan(cudaStream_t, const Geom& g, int slot, const uint8_t* fl
     }
     if (zCut && cuts) { for (size_t k = 0; k < cuts->size(); ++k) if ((*cuts)[k] < 0 || k + 1 == cuts->size()) (*cuts)[k] = n; (*cuts)[0] = 0; }
     return n;
+}
+
+void k_unit_counts(cudaStream_t, const Geom& g, int unit, int nUnits, const uint32_t* rowXYZ, int64_t rLo, int64_t rHi,
+                   const int32_t* cellList, const int32_t* cellStart, int32_t regLo, int32_t regHi, int* counts) {
+    if (nUnits > MAX_UNITS) throw Error("k_unit_counts: more z-units than MAX_UNITS");
+    for (int64_t i = rLo; i < rHi; ++i) ++counts[2 * std::min((int)((rowXYZ[i] >> 20) & 1023u) / unit, nUnits - 1)];
+    for (int32_t r = regLo; r < regHi; ++r)
+        if (cellStart[r + 1] > cellStart[r]) ++counts[2 * std::min(delin(g, SL_CENTER, cellList[cellStart[r]]).z / unit, nUnits - 1) + 1];
 }
 
 int64_t select_flagged(cudaStream_t, int64_t n, const uint8_t* flag, DBuf<int32_t>& out, int64_t outOffset) {

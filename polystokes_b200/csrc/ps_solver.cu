@@ -106,7 +106,7 @@ Solver::Solver(const ps_params& p) : P(p) {
 
 static int gcd_i(int a, int b) { while (b) { const int t = a % b; a = b; b = t; } return a; }
 
-// z cuts at multiples of lcm(16, tileSize), as even as the unit allows (ps_part.hpp)
+// z cuts at multiples of lcm(16, tileSize): the caller's (ps_set_partition, ps_rebalance) or as even as the unit allows (ps_part.hpp)
 void Solver::initComm(Comm* c) {
     std::unique_ptr<Comm> guard(c);
     if (c->nranks < 1 || c->rank < 0 || c->rank >= c->nranks) throw Error("ps_comm_init: bad rank / nranks");
@@ -115,18 +115,30 @@ void Solver::initComm(Comm* c) {
     comm = guard.release();
     haveSetup = false;
 }
-// the slab decomposition as a function of the grid and the tiling / layer parameters (ps_comm_init, ps_set_params)
+int Solver::cutUnit() const { return (P.doReducedRegions && P.doTile && P.tileSize >= 1) ? 16 / gcd_i(16, P.tileSize) * P.tileSize : 16; }
+std::vector<int> Solver::unitBounds() const {
+    const int unit = cutUnit(), nUnits = (g.nz + unit - 1) / unit;
+    std::vector<int> b((size_t)nUnits + 1, g.nz);
+    for (int u = 0; u < nUnits; ++u) b[u] = u * unit;
+    return b;
+}
+// the slab decomposition as a function of the grid, the tiling / layer parameters and the caller's cuts (ps_comm_init, ps_set_params,
+// ps_set_partition, ps_rebalance)
 void Solver::computePartition(int rank, int nranks) {
-    int unit = 16;
-    if (P.doReducedRegions && P.doTile && P.tileSize >= 1) unit = 16 / gcd_i(16, P.tileSize) * P.tileSize;
+    const int unit = cutUnit();
     // untiled regions, or tiles without padding, may reach across a cut: shared regions (ps_part.hpp), replicated setup
     part.spanning = nranks > 1 && P.doReducedRegions && (!P.doTile || P.tilePadding < 1 || P.tileSize < 1);
     const int nUnits = (g.nz + unit - 1) / unit;
     if (nranks > nUnits) throw Error("ps_comm_init: more ranks than z-slabs of lcm(16, tileSize) cells");
     part.rank = rank; part.nranks = nranks;
-    part.zCut.assign((size_t)nranks + 1, 0);
-    for (int k = 0; k <= nranks; ++k) part.zCut[k] = std::min(g.nz, (int)(((int64_t)k * nUnits + nranks / 2) / nranks) * unit);
-    part.zCut[0] = 0; part.zCut[nranks] = g.nz;
+    // the caller's cuts while they are multiples of the unit (ps_set_params may change it), the even cuts otherwise
+    if (!userCut.empty() && !valid_cuts(userCut, nranks, g.nz, unit)) userCut.clear();
+    if (!userCut.empty()) part.zCut = userCut;
+    else {
+        part.zCut.assign((size_t)nranks + 1, 0);
+        for (int k = 0; k <= nranks; ++k) part.zCut[k] = std::min(g.nz, (int)(((int64_t)k * nUnits + nranks / 2) / nranks) * unit);
+        part.zCut[0] = 0; part.zCut[nranks] = g.nz;
+    }
     for (int k = 0; k < nranks; ++k) if (part.zCut[k + 1] <= part.zCut[k]) throw Error("ps_comm_init: empty z-slab");
     g.zLo = part.zCut[rank]; g.zHi = part.zCut[rank + 1];
     // slab-local setup where regions cannot interact across a cut (ps_part.hpp); PS_SETUP_REPLICATED=1 forces the round-1 behaviour
@@ -598,6 +610,15 @@ void Solver::constructEdgesReducedIndices() { k_edges_reduced(st, g, F); }
 void Solver::constructActiveIndices() {
     uint8_t* flag = scratch8[0].p;
     int64_t cnt[N_SLOTS];
+    // every scan also tells where each z-unit starts in the numbering: the active counts of the own units (unitLoad); the slab cuts
+    // are unit boundaries
+    const std::vector<int> ub = unitBounds();
+    const int unit = cutUnit(), nUnits = (int)ub.size() - 1, uLo = g.zLo / unit, uHi = (g.zHi + unit - 1) / unit;
+    std::vector<int64_t> uc;
+    auto ownUnits = [&](int s) {
+        unitActive[s].assign((size_t)nUnits, 0);
+        for (int u = uLo; u < uHi; ++u) unitActive[s][u] = uc[u + 1] - uc[u];
+    };
     if (part.local) {
         // every slab numbers its own voxels from 0 (the scan visits its tile layers only); the global index adds the counts of the
         // slabs below -- exactly the reference's running counter, because tile order is z-slowest
@@ -606,7 +627,8 @@ void Solver::constructActiveIndices() {
             int tz[2];
             ownTileZ(s, tz);
             k_generic_to_active_flags(st, g, s, F.label[s], flag);
-            mine[s] = (double)tile_order_scan(st, g, s, flag, F.aidx[s], tileCounts, nullptr, nullptr, tz);
+            mine[s] = (double)tile_order_scan(st, g, s, flag, F.aidx[s], tileCounts, &ub, &uc, tz);
+            ownUnits(s);
         }
         const std::vector<double> all = hostAllgather(mine);
         for (int s = 0; s < N_SLOTS; ++s) {
@@ -619,8 +641,10 @@ void Solver::constructActiveIndices() {
     } else
     for (int s = 0; s < N_SLOTS; ++s) {
         k_generic_to_active_flags(st, g, s, F.label[s], flag);
-        if (part.multi()) cnt[s] = tile_order_scan(st, g, s, flag, F.aidx[s], tileCounts, &part.zCut, &part.slotCut[s]);
-        else { cnt[s] = tile_order_scan(st, g, s, flag, F.aidx[s], tileCounts); part.slotCut[s] = {0, cnt[s]}; }
+        cnt[s] = tile_order_scan(st, g, s, flag, F.aidx[s], tileCounts, &ub, &uc);
+        ownUnits(s);
+        part.slotCut[s].assign((size_t)part.nranks + 1, cnt[s]);
+        for (int k = 0; k < part.nranks; ++k) part.slotCut[s][k] = uc[part.zCut[k] / unit];
     }
     C = Counts();
     C.nCenter = cnt[SL_CENTER];
@@ -1568,6 +1592,7 @@ void Solver::applySolutionToVelocity(const ps_fields_out& out) {
 }
 
 void Solver::setup() {
+    unitLoad.clear(); unitCounts.clear();
     PS_WHERE("setup: peerResync");
     peerResync();
     // every rank must take part in the cancel all-reduce if any rank has a callback: agree on that once per setup
@@ -1598,7 +1623,7 @@ void Solver::setup() {
     PS_WHERE("setup: region matrices");
     { StageTimer T(st, &stageMs[PS_STAGE_REGION_MATRICES]); if (P.doReducedRegions) computeReducedRegionMatrices(); }
     PS_WHERE("setup: matrix blocks");
-    { StageTimer T(st, &stageMs[PS_STAGE_MATRIX_BLOCKS]); constructMatrixBlocks(); }
+    { StageTimer T(st, &stageMs[PS_STAGE_MATRIX_BLOCKS]); constructMatrixBlocks(); computeUnitLoads(); }
     PS_WHERE("setup: assemble");
     haveDiag = false; haveA = false;
     {
@@ -1609,6 +1634,85 @@ void Solver::setup() {
     }
     haveSetup = true;
     result = R_INCOMPLETE;
+}
+
+// The work table of the setup (Solver::unitLoad): the active counts of the own units from the scans, the coupled reduced rows and the
+// regions this rank owns counted by one kernel, all of it summed over the ranks by one all-gather (integers far below 2^53).
+void Solver::computeUnitLoads() {
+    PS_WHERE("setup: unit loads");
+    const int unit = cutUnit(), nU = (int)unitActive[0].size();
+    std::vector<double> mine((size_t)nU * UC_N, 0.);
+    for (int s = 0; s < N_SLOTS; ++s) for (int u = 0; u < nU; ++u) mine[(size_t)u * UC_N + s] = (double)unitActive[s][u];
+    const int64_t rLo = part.redRowCut[part.rank], rHi = part.redRowCut[part.rank + 1];
+    if (RG.count > 0 && (rHi > rLo || RG.regHi > RG.regLo)) {
+        DBuf<int>& cnt = scratch().rc;
+        cnt.alloc((size_t)2 * nU); cnt.zero(st, (size_t)2 * nU);
+        k_unit_counts(st, g, unit, nU, RG.rowXYZ.p, rLo, rHi, RG.cellList.p, RG.cellStart.p, RG.regLo, RG.regHi, cnt.p);
+        const std::vector<int> h = cnt.to_host(st, (size_t)2 * nU);
+        for (int u = 0; u < nU; ++u) { mine[(size_t)u * UC_N + UC_ROWS] = h[2 * u]; mine[(size_t)u * UC_N + UC_REGIONS] = h[2 * u + 1]; }
+    }
+    const std::vector<double> all = hostAllgather(mine);
+    unitCounts.assign(mine.size(), 0);
+    for (int k = 0; k < part.nranks; ++k) for (size_t i = 0; i < mine.size(); ++i) unitCounts[i] += std::llround(all[(size_t)k * mine.size() + i]);
+    unitLoad.assign((size_t)nU, 0.);
+    for (int u = 0; u < nU; ++u) {
+        const int64_t* t = unitCounts.data() + (size_t)u * UC_N;
+        OpCounts c;
+        c.nCenter = t[SL_CENTER]; c.nActiveVs = t[SL_FACE] + t[SL_FACE + 1] + t[SL_FACE + 2]; c.nEdges = t[SL_EDGE] + t[SL_EDGE + 1] + t[SL_EDGE + 2];
+        c.nRedRows = t[UC_ROWS]; c.nRegions = t[UC_REGIONS];
+        unitLoad[u] = OpBytes(c).cgIteration;
+    }
+    loadUnit = unit;
+}
+
+// ps_set_partition: the cuts must be legal and the same on every rank; one all-gather of every rank's verdict and cuts decides for all
+int Solver::setPartition(const int32_t* zCut) {
+    const int N = part.nranks;
+    std::vector<int> want;
+    if (zCut) want.assign(zCut, zCut + N + 1);
+    const bool ok = !zCut || valid_cuts(want, N, g.nz, cutUnit());
+    std::vector<double> mine((size_t)N + 3, 0.);
+    mine[0] = ok ? 1. : 0.; mine[1] = zCut ? 1. : 0.;
+    for (int k = 0; zCut && k <= N; ++k) mine[2 + k] = want[k];
+    const std::vector<double> all = hostAllgather(mine);
+    bool agree = true;
+    for (int r = 0; r < N; ++r) {
+        if (all[(size_t)r * mine.size()] != 1.) agree = false;
+        for (size_t i = 1; i < mine.size(); ++i) if (all[(size_t)r * mine.size() + i] != all[i]) agree = false;
+    }
+    if (!agree) {
+        g_lastError = "ps_set_partition: the cuts must run 0 = zCut[0] < ... < zCut[nranks] = nz with interior cuts at multiples of " +
+                      std::to_string(cutUnit()) + " layers, the same on every rank";
+        return PS_INVALID;
+    }
+    userCut = want;
+    if (comm) {
+        const std::vector<int> old = part.zCut;
+        computePartition(part.rank, N);
+        if (part.zCut != old) haveSetup = false;
+    }
+    return PS_SUCCESS;
+}
+
+// ps_rebalance: the same deterministic choice on every rank (the unit loads are replicated), no communication
+int Solver::rebalance(int32_t* zCut) {
+    int rc = PS_NOCHANGE;
+    if (unitLoad.empty() || loadUnit != cutUnit()) { g_lastError = "ps_rebalance: no unit loads of this tiling yet (call ps_setup or ps_step first)"; rc = PS_INVALID; }
+    else if (part.multi() && comm) {
+        const int N = part.nranks;
+        std::vector<int> cur((size_t)N + 1);
+        for (int k = 0; k <= N; ++k) cur[k] = (part.zCut[k] + loadUnit - 1) / loadUnit;
+        const std::vector<int> best = balanced_cuts(unitLoad, N);
+        if (max_slab_load(unitLoad, best) < max_slab_load(unitLoad, cur)) {
+            userCut.assign((size_t)N + 1, g.nz);
+            for (int k = 0; k < N; ++k) userCut[k] = best[k] * loadUnit;
+            computePartition(part.rank, N);
+            haveSetup = false;
+            rc = PS_SUCCESS;
+        }
+    }
+    if (zCut) std::copy(part.zCut.begin(), part.zCut.end(), zCut);
+    return rc;
 }
 
 // inputs + setup; a slab-local attempt that meets work for the boundary fix-up is repeated with the setup replicated (collective: the

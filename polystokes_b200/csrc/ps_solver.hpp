@@ -122,6 +122,36 @@ struct Counts {
     int64_t nRowsExt = 0;               // nActiveVs + coupled reduced rows
 };
 
+// Algorithmic bytes of the hot passes (DESIGN.md section 5) as a function of the counts they sweep: cells, active face rows, edges,
+// coupled reduced rows and regions.  Compact operator: 8 B of codes + 6 x 4 B columns per face row (+ 1 B mass code on active rows),
+// 8 + 24 B per cell (serves the pressure row and the 3 centre-stress rows), 4 + 16 B per edge; every vector is read / written once.
+// "csr*" = the same passes priced as the CSR SpMV of SURVEY.md 8d (12 B per stored non-zero).  Linear in the counts, so the bytes
+// of the parts of a grid (the z-units of Solver::unitLoad) sum to those of the whole grid.
+struct OpCounts { int64_t nCenter = 0, nActiveVs = 0, nEdges = 0, nRedRows = 0, nRegions = 0; };
+struct OpBytes {
+    double pass1Sweep, reduced, pass1, pass2, pass2Dots, csrPass1, csrPass2, csrApply, cgUpdate, cgIteration;
+    explicit OpBytes(const OpCounts& c) {
+        const double nE = (double)c.nEdges;
+        const double n = (double)(4 * c.nCenter + c.nEdges);                  // nSystemSize
+        const int64_t nRowsExt = c.nActiveVs + c.nRedRows, nStresses = 3 * c.nCenter + c.nEdges;
+        const double nRed = (double)c.nRedRows;
+        // pass 1 = the sweep over the compact rows of K_ext (x once, w once) + the region kernel (below)
+        pass1Sweep = 32.0 * nRowsExt + 1.0 * c.nActiveVs /*matrix*/ + 8.0 * n /*x*/ + 8.0 * nRowsExt /*w write*/;
+        pass2 = 32.0 * c.nCenter + 20.0 * nE /*matrix*/ + 8.0 * nRowsExt /*w read*/ + 8.0 * (c.nCenter + nE) /*mu^-1: once per cell / edge*/
+              + 8.0 * n /*x (stress part: the mu term; pressure part: the fused dot)*/ + 8.0 * n /*y*/;
+        pass2Dots = pass2 + 8.0 * n /*r for the fused r.Ap*/;
+        csrPass1 = 12.0 * 8.0 * nRowsExt + 8.0 * n + 8.0 * c.nActiveVs + 8.0 * nRowsExt;
+        csrPass2 = 12.0 * (6.0 * c.nCenter + 2.0 * 3 * c.nCenter + 4.0 * nE) + 8.0 * nRowsExt + 8.0 * nStresses + 8.0 * nStresses + 8.0 * n;
+        const double perRegion = (double)c.nRegions * (RDOF * RDOF + 2 * RDOF + 30) * 8.0;     // B^-1 + t, s, sigma
+        csrApply = csrPass1 + csrPass2 + nRed * 24.0 + perRegion;
+        // reduced rows: w read + packed coordinates (moments), packed coordinates + w write (expand)
+        reduced = nRed * (8.0 + 4.0) + nRed * (4.0 + 8.0) + perRegion;
+        pass1 = pass1Sweep + reduced;
+        cgUpdate = 56.0 * n;
+        cgIteration = pass1 + pass2Dots + 56.0 * n /*x, r, p update: x, r, p, Ap in; x, r, p out*/;
+    }
+};
+
 struct PcgScalars {   // device-resident CG state: no host round trip inside an iteration
     double rsold, pAp, alpha, beta, rsnew, xmag, rre;
     int iter, done, maxIter, pad;
@@ -206,6 +236,21 @@ public:
     Comm* comm = nullptr;
     void initComm(Comm* c);             // takes ownership; computes the z cuts
     void computePartition(int rank, int nranks);
+    int cutUnit() const;                // lcm(16, tileSize) layers with tiles, 16 without: the granularity of the cuts
+    // Caller-set cuts (ps_set_partition, ps_rebalance); empty = the even cuts.  computePartition takes them while they suit the unit.
+    std::vector<int> userCut;
+    int setPartition(const int32_t* zCut);     // collective; PS_SUCCESS or PS_INVALID (agreed by every rank)
+    int rebalance(int32_t* zCut);              // PS_SUCCESS (cuts moved), PS_NOCHANGE, PS_INVALID (no unit loads)
+    // Work per z-unit of the last setup: unitCounts[u][UC_N] = active voxels of the 7 sample slots, coupled reduced rows (by the z of
+    // their face) and regions (by the z of their first cell) in unit u, the last unit with the slots' top layer; unitLoad[u] = the
+    // CG-iteration bytes of those counts (OpBytes).  Independent of the cuts, replicated on every rank.
+    enum { UC_ROWS = N_SLOTS, UC_REGIONS, UC_N };
+    std::vector<int64_t> unitActive[N_SLOTS];   // this rank's own units (constructActiveIndices)
+    std::vector<int64_t> unitCounts;
+    std::vector<double> unitLoad;
+    int loadUnit = 0;                           // the unit the table was formed with
+    void computeUnitLoads();
+    std::vector<int> unitBounds() const;        // z of the first layer of every unit, then nz
     // Slab-local setup assumes that the boundary fix-up (S_Cls:1073-1172, a serial sweep) has nothing to do.  A step that finds a
     // candidate cell -- all ranks learn it from one all-reduce -- is restarted with the setup replicated (the round-1 form); the
     // handle stays there until the tiling / layer parameters change.
@@ -320,10 +365,16 @@ void k_valid_faces(cudaStream_t, const Geom&, const Fields&, float* const valid[
 
 // tile-order exclusive scan of a dense 0/1 flag field: out[q] = rank among flagged voxels in the
 // reference's voxel iteration order, -1 where the flag is 0.  Returns the total (host sync).
-// If `zCut` is given, cuts[k] receives the rank of the first flagged voxel with z >= zCut[k] (cuts multiple of 16).
+// If `zCut` is given, cuts[k] receives the rank of the first flagged voxel with z >= zCut[k] (cuts multiple of 16; the last entry
+// receives the total, 0 for a z below the scanned layers).
 // With `tileZ` only the tile layers [tileZ[0], tileZ[1]) are scanned (ranks start at 0 on the first of them; `out` is written there only).
 int64_t tile_order_scan(cudaStream_t, const Geom&, int slot, const uint8_t* flag, int32_t* out, DBuf<int32_t>& tileCounts,
                         const std::vector<int>* zCut = nullptr, std::vector<int64_t>* cuts = nullptr, const int* tileZ = nullptr);
+// counts[2u] += coupled reduced rows [rLo, rHi) whose face lies in z-unit u (the top face plane in the last unit), counts[2u+1] +=
+// regions [regLo, regHi) whose first cell in tile order lies in it (nUnits <= MAX_UNITS).  Integer counters: exact in any launch order.
+constexpr int MAX_UNITS = 64;         // nz <= 1022 (10-bit packed row coordinates), units >= 16 layers
+void k_unit_counts(cudaStream_t, const Geom&, int unit, int nUnits, const uint32_t* rowXYZ, int64_t rLo, int64_t rHi,
+                   const int32_t* cellList, const int32_t* cellStart, int32_t regLo, int32_t regHi, int* counts);
 // out[k] = in[0] + ... + in[k-1] for k < n; returns the total (host sync)
 int64_t exclusive_scan_i64(cudaStream_t, int64_t n, const int64_t* in, int64_t* out);
 // stable sort of (key, value) pairs by key (keys < 2^keyBits)

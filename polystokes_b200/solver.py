@@ -138,6 +138,25 @@ class PolyStokesSolver:
         self.lib.ps_get_partition(self.h, C.byref(r), C.byref(lo), C.byref(hi), cuts)
         return r.value, n, lo.value, hi.value, list(cuts)
 
+    def set_partition(self, cuts=None):
+        """Collective: z cuts [nranks+1] for the next setup / step (None = the even cuts).  Returns PS_SUCCESS, or PS_INVALID on every
+        rank when the cuts break a rule or differ between ranks (the handle keeps its cuts)."""
+        arr = None if cuts is None else (C.c_int32 * len(cuts))(*[int(c) for c in cuts])
+        rc = self.lib.ps_set_partition(self.h, arr)
+        if rc == PS_FAILED:
+            raise PolyStokesError(f"ps_set_partition failed: {self.last_error()}")
+        return rc
+
+    def rebalance(self):
+        """Collective: cuts that balance the CG-iteration bytes of the last setup over the slabs (vector "unitLoad").  Returns
+        (rc, cuts): PS_SUCCESS when the cuts moved (effective at the next setup / step), PS_NOCHANGE, or PS_INVALID before a setup."""
+        n = self.partition()[1]
+        cuts = (C.c_int32 * (n + 1))()
+        rc = self.lib.ps_rebalance(self.h, cuts)
+        if rc == PS_FAILED:
+            raise PolyStokesError(f"ps_rebalance failed: {self.last_error()}")
+        return rc, list(cuts)
+
     def last_error(self):
         e = self.lib.ps_last_error()
         return e.decode() if e else ""
