@@ -153,20 +153,6 @@ static void build_region_tables(double* T) {
         }
 }
 
-// v^e for e in 0..4 without divergent control flow
-PS_HD double pow_small(double v, int e) {
-    const double v2 = v * v;
-    double r = (e & 1) ? v : 1.;
-    if (e & 2) r *= v2;
-    if (e & 4) r *= v2 * v2;
-    return r;
-}
-// exponents (ex, ey, ez) of monomial k of {1,x,y,z,xx,xy,xz,yy,yz,zz}, packed 4 bits each
-PS_HD int monomial_exps(int k) {
-    const int t[10] = {0x000, 0x001, 0x010, 0x100, 0x002, 0x011, 0x101, 0x020, 0x110, 0x200};
-    return t[k];
-}
-
 // phase 1: everything the moments need from one REDUCED cell, staged as stage[field * GRAM_CELLS + slot]:
 // fields 0-2 the cell-centre offset from the region's COM, 3-8 wM, 9-14 wN, 15-20 wN*u of the 6 faces, 21 mu, 22-33 mu of
 // the owned REDUCED edges
@@ -206,72 +192,8 @@ PS_D void stage_cell(const Geom& g, const Fields& F, const double* com, int64_t 
         }
     }
 }
-// phase 2: moment `item` (0..234 work items, see the layout constants) over the staged cells, in cell order.
-// A face of axis a sits at the cell-centre offset -+ dx/2 on axis a; an edge of axis e at -+ dx/2 on the two other axes.
-PS_D void accumulate_item(const Geom& g, const double* stage, int nCells, int item, double* out) {
-    const double h = 0.5 * g.dx;
-    if (item < 195) {
-        const bool rhs = item >= 165;
-        const int a = rhs ? (item - 165) / 10 : item / 55;
-        int ex;
-        if (rhs) ex = monomial_exps((item - 165) % 10);
-        else { int k, l; sym_pair(10, item % 55, k, l); ex = monomial_exps(k) + monomial_exps(l); }
-        const int e[3] = {ex & 15, (ex >> 4) & 15, (ex >> 8) & 15};
-        const int b = (a + 1) % 3, c = (a + 2) % 3;
-        const double* pa = stage + a * GRAM_CELLS; const double* pb = stage + b * GRAM_CELLS; const double* pc = stage + c * GRAM_CELLS;
-        const double* w0 = stage + ((rhs ? 15 : 3) + 2 * a) * GRAM_CELLS;    // wM (or wN*u) of the two faces of axis a
-        const double* w1 = stage + (9 + 2 * a) * GRAM_CELLS;                  // wN
-        double acc0 = 0., acc1 = 0.;
-        for (int s = 0; s < nCells; ++s) {
-            const double base = pow_small(pb[s], e[b]) * pow_small(pc[s], e[c]);
-            for (int dir = 0; dir < 2; ++dir) {
-                const double wa = w0[dir * GRAM_CELLS + s], wb = rhs ? 0. : w1[dir * GRAM_CELLS + s];
-                if (wa == 0. && wb == 0.) continue;
-                const double pr = base * pow_small(dir ? pa[s] + h : pa[s] - h, e[a]);
-                acc0 += wa * pr; acc1 += wb * pr;
-            }
-        }
-        if (rhs) out[MOM_RHS + (item - 165)] = acc0;
-        else { out[MOM_QM + item] = acc0; out[MOM_QN + item] = acc1; }
-    } else if (item < 205) {                             // T^c: cell-centred stresses, sum mu (1,x,y,z)(1,x,y,z)^T
-        int k, l; sym_pair(4, item - 195, k, l);
-        const int ex = monomial_exps(k) + monomial_exps(l);
-        const double* mu = stage + 21 * GRAM_CELLS;
-        double acc = 0.;
-        for (int s = 0; s < nCells; ++s)
-            acc += mu[s] * (pow_small(stage[s], ex & 15) * pow_small(stage[GRAM_CELLS + s], (ex >> 4) & 15) * pow_small(stage[2 * GRAM_CELLS + s], (ex >> 8) & 15));
-        out[MOM_TC + (item - 195)] = acc;
-    } else {                                             // T^e: edge-centred stresses of edge axis e
-        const int e = (item - 205) / 10; int k, l; sym_pair(4, (item - 205) % 10, k, l);
-        const int ex = monomial_exps(k) + monomial_exps(l);
-        const int ee[3] = {ex & 15, (ex >> 4) & 15, (ex >> 8) & 15};
-        const int a = e == 0 ? 1 : 0, b = e == 2 ? 1 : 2;
-        const double* pe = stage + e * GRAM_CELLS; const double* pa = stage + a * GRAM_CELLS; const double* pb = stage + b * GRAM_CELLS;
-        double acc = 0.;
-        for (int s = 0; s < nCells; ++s) {
-            const double along = pow_small(pe[s], ee[e]);
-            for (int db = 0; db < 2; ++db) for (int da = 0; da < 2; ++da) {
-                const double mu = stage[(22 + e * 4 + db * 2 + da) * GRAM_CELLS + s];
-                if (mu == 0.) continue;
-                acc += mu * (along * pow_small(da ? pa[s] + h : pa[s] - h, ee[a]) * pow_small(db ? pb[s] + h : pb[s] - h, ee[b]));
-            }
-        }
-        out[MOM_TE + (item - 205)] = acc;
-    }
-}
-constexpr int MOM_ITEMS = 235;
 
 #ifndef PS_EMULATE
-__global__ void __launch_bounds__(GRAM_CELLS) gram_moments_kernel(Geom g, Fields F, const double* __restrict__ com, const int32_t* __restrict__ cellList,
-                                                                 const int32_t* __restrict__ chunk, double* __restrict__ partial, int chunk0) {
-    extern __shared__ double stage[];              // [STAGE_DOUBLES][GRAM_CELLS]
-    const int ch = chunk0 + blockIdx.x;
-    const int region = chunk[3 * ch + 0], begin = chunk[3 * ch + 1], end = chunk[3 * ch + 2];
-    const int nCells = end - begin;
-    if ((int)threadIdx.x < nCells) stage_cell(g, F, com + 3 * region, cellList[begin + threadIdx.x], threadIdx.x, stage);
-    __syncthreads();
-    if (threadIdx.x < MOM_ITEMS) accumulate_item(g, stage, nCells, threadIdx.x, partial + (size_t)ch * MOM_COUNT);
-}
 // ---- the same moments on the FP64 tensor cores (DMMA.8x8x4) ------------------------------------------------------------------
 // Per face axis a the moments are one dense contraction over the 2 x 256 face samples of the chunk,
 //     Phi_a^T [ W_M Phi_a | W_N Phi_a | W_N u ]        Phi_a : 512 x 10 (monomials of the face offsets),   10 x 21 outputs,
@@ -400,24 +322,82 @@ __global__ void __launch_bounds__(GRAM_CELLS, 2) gram_moments_dmma_kernel(Geom g
 }
 void region_gram_partials(cudaStream_t st, const Geom& g, const Fields& F, const RegionData& RG, double* partial) {
     if (RG.cellChunkHi <= RG.cellChunkLo) return;
-    const size_t smem = (size_t)STAGE_DOUBLES * GRAM_CELLS * sizeof(double);
-    // PS_GRAM_DMMA=0: the scalar kernel (one work item per moment), kept for A/B timing and as the summation-order reference
-    static const bool dmma = !(getenv("PS_GRAM_DMMA") && atoi(getenv("PS_GRAM_DMMA")) == 0);
-    if (dmma) {
-        const size_t smem2 = smem + (size_t)PHI_DOUBLES * sizeof(double);
-        PS_CUDA(cudaFuncSetAttribute(gram_moments_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));      // a per-DEVICE attribute: set on every call
-        gram_moments_dmma_kernel<<<RG.cellChunkHi - RG.cellChunkLo, GRAM_CELLS, smem2, st>>>(g, F, RG.com.p, RG.cellList.p, RG.cellChunk.p, partial, RG.cellChunkLo);
-        PS_COUNT_LAUNCH(1);
-        PS_CUDA(cudaGetLastError());
-        return;
-    }
+    const size_t smem = (size_t)(STAGE_DOUBLES * GRAM_CELLS + PHI_DOUBLES) * sizeof(double);
     // a per-DEVICE attribute: set on every call (a process-wide "done" flag left the second GPU of a multi-device handle without it)
-    PS_CUDA(cudaFuncSetAttribute(gram_moments_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gram_moments_kernel<<<RG.cellChunkHi - RG.cellChunkLo, GRAM_CELLS, smem, st>>>(g, F, RG.com.p, RG.cellList.p, RG.cellChunk.p, partial, RG.cellChunkLo);
+    PS_CUDA(cudaFuncSetAttribute(gram_moments_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gram_moments_dmma_kernel<<<RG.cellChunkHi - RG.cellChunkLo, GRAM_CELLS, smem, st>>>(g, F, RG.com.p, RG.cellList.p, RG.cellChunk.p, partial, RG.cellChunkLo);
     PS_COUNT_LAUNCH(1);
     PS_CUDA(cudaGetLastError());
 }
 #else
+// the emulation twin: the moments one at a time (phase 2 below), each a serial sum in cell order
+// v^e for e in 0..4 without divergent control flow
+PS_HD double pow_small(double v, int e) {
+    const double v2 = v * v;
+    double r = (e & 1) ? v : 1.;
+    if (e & 2) r *= v2;
+    if (e & 4) r *= v2 * v2;
+    return r;
+}
+// exponents (ex, ey, ez) of monomial k of {1,x,y,z,xx,xy,xz,yy,yz,zz}, packed 4 bits each
+PS_HD int monomial_exps(int k) {
+    const int t[10] = {0x000, 0x001, 0x010, 0x100, 0x002, 0x011, 0x101, 0x020, 0x110, 0x200};
+    return t[k];
+}
+// phase 2: moment `item` (0..234 work items, see the layout constants) over the staged cells, in cell order.
+// A face of axis a sits at the cell-centre offset -+ dx/2 on axis a; an edge of axis e at -+ dx/2 on the two other axes.
+PS_D void accumulate_item(const Geom& g, const double* stage, int nCells, int item, double* out) {
+    const double h = 0.5 * g.dx;
+    if (item < 195) {
+        const bool rhs = item >= 165;
+        const int a = rhs ? (item - 165) / 10 : item / 55;
+        int ex;
+        if (rhs) ex = monomial_exps((item - 165) % 10);
+        else { int k, l; sym_pair(10, item % 55, k, l); ex = monomial_exps(k) + monomial_exps(l); }
+        const int e[3] = {ex & 15, (ex >> 4) & 15, (ex >> 8) & 15};
+        const int b = (a + 1) % 3, c = (a + 2) % 3;
+        const double* pa = stage + a * GRAM_CELLS; const double* pb = stage + b * GRAM_CELLS; const double* pc = stage + c * GRAM_CELLS;
+        const double* w0 = stage + ((rhs ? 15 : 3) + 2 * a) * GRAM_CELLS;    // wM (or wN*u) of the two faces of axis a
+        const double* w1 = stage + (9 + 2 * a) * GRAM_CELLS;                  // wN
+        double acc0 = 0., acc1 = 0.;
+        for (int s = 0; s < nCells; ++s) {
+            const double base = pow_small(pb[s], e[b]) * pow_small(pc[s], e[c]);
+            for (int dir = 0; dir < 2; ++dir) {
+                const double wa = w0[dir * GRAM_CELLS + s], wb = rhs ? 0. : w1[dir * GRAM_CELLS + s];
+                if (wa == 0. && wb == 0.) continue;
+                const double pr = base * pow_small(dir ? pa[s] + h : pa[s] - h, e[a]);
+                acc0 += wa * pr; acc1 += wb * pr;
+            }
+        }
+        if (rhs) out[MOM_RHS + (item - 165)] = acc0;
+        else { out[MOM_QM + item] = acc0; out[MOM_QN + item] = acc1; }
+    } else if (item < 205) {                             // T^c: cell-centred stresses, sum mu (1,x,y,z)(1,x,y,z)^T
+        int k, l; sym_pair(4, item - 195, k, l);
+        const int ex = monomial_exps(k) + monomial_exps(l);
+        const double* mu = stage + 21 * GRAM_CELLS;
+        double acc = 0.;
+        for (int s = 0; s < nCells; ++s)
+            acc += mu[s] * (pow_small(stage[s], ex & 15) * pow_small(stage[GRAM_CELLS + s], (ex >> 4) & 15) * pow_small(stage[2 * GRAM_CELLS + s], (ex >> 8) & 15));
+        out[MOM_TC + (item - 195)] = acc;
+    } else {                                             // T^e: edge-centred stresses of edge axis e
+        const int e = (item - 205) / 10; int k, l; sym_pair(4, (item - 205) % 10, k, l);
+        const int ex = monomial_exps(k) + monomial_exps(l);
+        const int ee[3] = {ex & 15, (ex >> 4) & 15, (ex >> 8) & 15};
+        const int a = e == 0 ? 1 : 0, b = e == 2 ? 1 : 2;
+        const double* pe = stage + e * GRAM_CELLS; const double* pa = stage + a * GRAM_CELLS; const double* pb = stage + b * GRAM_CELLS;
+        double acc = 0.;
+        for (int s = 0; s < nCells; ++s) {
+            const double along = pow_small(pe[s], ee[e]);
+            for (int db = 0; db < 2; ++db) for (int da = 0; da < 2; ++da) {
+                const double mu = stage[(22 + e * 4 + db * 2 + da) * GRAM_CELLS + s];
+                if (mu == 0.) continue;
+                acc += mu * (along * pow_small(da ? pa[s] + h : pa[s] - h, ee[a]) * pow_small(db ? pb[s] + h : pb[s] - h, ee[b]));
+            }
+        }
+        out[MOM_TE + (item - 205)] = acc;
+    }
+}
+constexpr int MOM_ITEMS = 235;
 void region_gram_partials(cudaStream_t, const Geom& g, const Fields& F, const RegionData& RG, double* partial) {
     std::vector<double> stage((size_t)STAGE_DOUBLES * GRAM_CELLS);
     for (int ch = RG.cellChunkLo; ch < RG.cellChunkHi; ++ch) {

@@ -141,9 +141,9 @@ void Solver::computePartition(int rank, int nranks) {
     }
     for (int k = 0; k < nranks; ++k) if (part.zCut[k + 1] <= part.zCut[k]) throw Error("ps_comm_init: empty z-slab");
     g.zLo = part.zCut[rank]; g.zHi = part.zCut[rank + 1];
-    // slab-local setup where regions cannot interact across a cut (ps_part.hpp); PS_SETUP_REPLICATED=1 forces the round-1 behaviour
-    const bool forceRep = getenv("PS_SETUP_REPLICATED") && atoi(getenv("PS_SETUP_REPLICATED"));
-    part.local = nranks > 1 && !forceRep && !replicatedSetup && (!P.doReducedRegions || (P.doTile && P.tilePadding >= 2));
+    // slab-local setup where regions cannot interact across a cut (ps_part.hpp), unless a step with these tiling / layer
+    // parameters has fallen back to the replicated setup (NeedReplicatedSetup)
+    part.local = nranks > 1 && !replicatedSetup && (!P.doReducedRegions || (P.doTile && P.tilePadding >= 2));
     part.halo = std::min(16, std::max(4, P.activeLiquidBoundaryLayerSize + P.activeSolidBoundaryLayerSize + 3));
     if (part.local && P.activeLiquidBoundaryLayerSize + P.activeSolidBoundaryLayerSize + 3 > 16) part.local = false;      // the floods reach further than one tile layer
     g.wzLo = part.local ? std::max(0, g.zLo - part.halo) : 0;

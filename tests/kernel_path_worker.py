@@ -1,6 +1,6 @@
 """Child process of tests/test_gpu_kernel_paths.py: runs the library on a few scenes under ONE setting of the region-kernel
-knobs (PS_REGION_FUSE_MAX, PS_GRAM_DMMA).  The library reads each knob once per process, so every setting needs a process of its
-own; the knob comes in through the environment.
+knob (PS_REGION_FUSE_MAX).  The library reads the knob once per process, so every setting needs a process of its own; the knob
+comes in through the environment.
 
 usage: python kernel_path_worker.py [--lib PATH] [--tight] [--no-step] <out_dir> <scene>...
 

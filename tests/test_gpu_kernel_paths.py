@@ -2,7 +2,7 @@
 
 Which kernels carry the reduced term of an apply depends on the scene (<= 900 owned regions: reduced_region_kernel with 128 lanes per
 axis; more: 64 lanes; a region of more than 16384 coupled rows: the chunked reduced_moments_kernel with per-region tickets, then
-reduced_expand_kernel) and on knobs read once per process (PS_REGION_FUSE_MAX, PS_GRAM_DMMA).  Each setting runs in a child process
+reduced_expand_kernel) and on a knob read once per process (PS_REGION_FUSE_MAX).  Each setting runs in a child process
 (tests/kernel_path_worker.py) under a time-out; the library's `regionPath` count says which kernels ran, and each test asserts it, so a
 moved threshold fails here instead of silently covering another path.
 
@@ -33,7 +33,6 @@ ALL = TILED + ["blob64_notile"]
 SETTINGS = {
     "default": ({}, ALL),
     "fuse_max0": ({"PS_REGION_FUSE_MAX": "0"}, TILED),          # the chunked kernels on tiled regions: one chunk per (region, axis)
-    "gram_scalar": ({"PS_GRAM_DMMA": "0"}, ALL),
 }
 
 
@@ -189,17 +188,6 @@ def test_gpu_kernel_path_scenes_cover_the_edges(built, tmp_path_factory):
     assert any(c > 2 * 256 for c in cells) and any(c % 256 for c in cells)
     assert min(int(r["count_minRegionCells"]) for r in res.values()) < 32
     assert int(res["box96_tile8"]["count_regionCount"]) > 900
-
-
-@pytest.mark.gpu
-def test_gpu_gram_scalar_and_dmma_agree(built, tmp_path_factory):
-    """The scalar Gram kernel and the DMMA one sum in different orders: they agree per entry within the region gates.  (Each is
-    bit-identical to itself on a second handle: check_scene.)"""
-    d, s = run_worker("default", tmp_path_factory.getbasetemp()), run_worker("gram_scalar", tmp_path_factory.getbasetemp())
-    for name in d:
-        blocks = parity.region_block_errors(d[name].get, s[name].get, int(d[name]["count_regionCount"]))
-        for v, gate in parity.REGION_GATES.items():
-            assert blocks[v] <= gate, f"{name}: DMMA vs scalar Gram {v} {blocks[v]:.2e} > {gate:.0e}"
 
 
 def test_emulated_kernel_path_worker(built, tmp_path_factory):

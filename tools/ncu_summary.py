@@ -1,7 +1,10 @@
 """Summarise ncu output into tracked text files under profiles/.
 
-  python tools/ncu_summary.py launches gpurun_out/launches_step.csv profiles/r01_launch_shares.txt
-  python tools/ncu_summary.py full gpurun_out/prof_hot.ncu-rep profiles/r01_ncu_hot.txt [profiles/ncu_traffic.json]
+  python tools/ncu_summary.py launches launches_step.csv profiles/r01_launch_shares.txt
+  python tools/ncu_summary.py full prof_hot.ncu-rep profiles/r01_ncu_hot.txt [profiles/ncu_traffic.json]
+
+launches_step.csv is ncu's --csv log of gpu__time_duration.sum per launch, prof_hot.ncu-rep a --set full report, both of a run
+of tools/probe.py.
 """
 import collections, csv, json, re, subprocess, sys
 
